@@ -16,6 +16,8 @@ With N GPUs the z axis is sharded (nz/N redshifts per rank, total work fixed -> 
           out, every host<->device copy inside the timed region
   --impl reference : the reference's own CPU implementation on the host cores: the unmodified simonsobs/hmvec installed
           under oracle/_ref (oracle/build_ref.sh) when present, else the oracle port; one z-slab per worker process
+  --dump-outputs DIR : the outputs of the last timed step as .npy files.  The inputs depend only on the arguments, so
+          two builds of the project run with the same arguments can be compared array for array.
 """
 import argparse
 import contextlib
@@ -248,6 +250,29 @@ def summary_for_shard_check(P_local, cl, world, dist, dev):
     return {"cl": [np.asarray(c)[::100].tolist() for c in cl], "spectra_sums": sums.cpu().tolist()}
 
 
+DUMP_BUDGET = 60 * 10 ** 6     # bytes of array data --dump-outputs writes at most
+
+
+def sample_outputs(g, ks, nz_total, world, dist):
+    """What the caller of the timed launch sequence receives from its last step (GridSix.spectra()): P1h and P2h of
+    the seven spectra [nz, nk] and C_kk, C_kg, C_yy, all float64.  When the whole set exceeds DUMP_BUDGET the spectra
+    keep a fixed, seeded subset of their k columns, listed in `ks`.  With a sharded z axis the slabs are gathered."""
+    p1, p2, ckk, ckg = g.spectra()
+    tags, nk = tuple(p1), ks.size
+    ncol = min(nk, max(1, (DUMP_BUDGET - 8 * 3 * ckk.size) // (16 * len(tags) * nz_total + 8)))
+    cols = np.arange(nk) if ncol == nk else np.sort(np.random.default_rng(0).choice(nk, ncol, replace=False))
+    out = {}
+    for t in tags:
+        out["P1h_" + t] = p1[t][:, cols]
+        out["P2h_" + t] = p2[t][:, cols]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, out)          # rank order is z order
+        out = {n: np.concatenate([p[n] for p in parts]) for n in out}
+    out.update(C_kk=ckk, C_kg=ckg, C_yy=g.last_cyy, ks=ks[cols])
+    return out
+
+
 def run_b200(a):
     import torch
     import torch.distributed as dist
@@ -304,6 +329,7 @@ def run_b200(a):
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if sampler is not None else None
+    dump = sample_outputs(g, ks, a.nz, world, dist) if a.dump_outputs else None
 
     # ---- per-stage times: the same steps again with the stages strictly one after the other on one stream and an
     # event at every stage boundary (a kernel's own duration, for the roofline entries; their sum is `serial_ms`) ----
@@ -522,6 +548,12 @@ def run_b200(a):
                                           "Limber, single numpy thread, %s" % (
                                               a.cpu_nz, a.nz, a.nm, a.nk,
                                               "unmodified reference from oracle/_ref" if kind == "reference" else "oracle port")}
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
+        line["dump_outputs"] = {"dir": a.dump_outputs, "arrays": len(dump), "k_columns": int(dump["ks"].size),
+                                "bytes": int(sum(v.nbytes for v in dump.values()))}
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -548,7 +580,15 @@ def main():
                          "its cube to HBM and reading it back (hmv_uk_nfw + hmv_power_six, the faster default)")
     ap.add_argument("--write-shard-ref", action="store_true",
                     help="(1 GPU) write profiles/r02_shard_reference.json: the C_ell and spectra sums N>1 runs are checked against")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed (the seven P1h/P2h spectra, k-sampled "
+                         "to at most 60 MB, and C_kk, C_kg, C_yy) as DIR/<name>.npy, float64")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        # the reference arm times a sample of one-redshift slabs on a thinned mass axis, not the grid itself
+        ap.error("--dump-outputs applies to the B200 path (--impl b200)")
     if a.impl == "reference":
         run_reference(a)
     else:

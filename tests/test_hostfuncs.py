@@ -10,7 +10,7 @@ import pytest
 from conftest import load_golden, assert_close, ROOT
 
 # public def/class names of the reference's hmvec/hmvec.py (what `from .hmvec import *` in hmvec/__init__.py:1 exports
-# besides re-exported modules); regenerated from /root/reference when it is present (build container)
+# besides re-exported modules); checked against the installed reference (oracle/_ref) when it is present
 REFERENCE_NAMES = """HaloModel Fcon Mhalo_stellar Mhalo_stellar_core Mstellar_halo P_e P_e_generic P_e_generic_x R_from_M a2z avg_Nc
 avg_NcNs avg_Ns avg_NsNsm1 battaglia_gas_fit duffy_concentration hod_default_mfunc mdelta_from_mdelta
 mdelta_from_mdelta_unvectorized ngal_from_mthresh rho_gas rho_gas_generic rho_gas_generic_x rho_nfw rho_nfw_x
@@ -27,7 +27,7 @@ def hm():
 
 def test_export_surface(hm):
     names = set(REFERENCE_NAMES)
-    ref = "/root/reference/hmvec/hmvec.py"
+    ref = os.path.join(ROOT, "oracle", "_ref", "hmvec", "hmvec.py")
     if os.path.exists(ref):
         found = set(re.findall(r"^(?:def|class) (\w+)", open(ref).read(), re.M))
         assert found <= names, "REFERENCE_NAMES is stale: %s" % sorted(found - names)
