@@ -105,4 +105,69 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
                ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
+// ---- stage ring fed by bulk async copies -------------------------------------------------------------------------
+// Dynamic shared memory holds nst stages of stage_doubles, then full[nst] and empty[nst] mbarriers.  One producer lane
+// acquires a stage (waits until every consumer warp has released it), announces the bytes it will copy and issues the
+// copies on the stage's full barrier; each consumer warp waits on full and releases the stage with one arrive on empty.
+// Producer and every consumer walk the stages in the same order; a RingSlot names a stage and the parity of its lap.
+struct RingSlot {
+  int s = 0;           // stage
+  unsigned ph = 0;     // parity of the current lap
+};
+struct RingStage {
+  double* p;
+  unsigned long long* full;   // the barrier the stage's copies complete on
+};
+
+struct BulkRing {
+  double* base;
+  unsigned long long *full, *empty;
+  int nst, stage_doubles;
+
+  __host__ __device__ static constexpr size_t smem_bytes(int nst, int stage_doubles) {
+    return (size_t)nst * stage_doubles * sizeof(double) + 2 * (size_t)nst * sizeof(unsigned long long);
+  }
+  // carves the ring out of `smem`; thread 0 initialises the barriers, which the block may use after a __syncthreads()
+  __device__ __forceinline__ BulkRing(void* smem, int nst_, int stage_doubles_, unsigned consumer_warps)
+      : base(reinterpret_cast<double*>(smem)), nst(nst_), stage_doubles(stage_doubles_) {
+    full = reinterpret_cast<unsigned long long*>(base + (size_t)nst * stage_doubles);
+    empty = full + nst;
+    if (threadIdx.x == 0) {
+      for (int s = 0; s < nst; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, consumer_warps); }
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+  }
+  __device__ __forceinline__ double* stage(const RingSlot& c) const { return base + (size_t)c.s * stage_doubles; }
+  // Two ways to the same sequence of slots: slot(it) of the it-th fill, or a cursor stepped by advance().  With a
+  // compile-time nst the division is a multiply; which one a kernel uses is a register-allocation choice (ptxas spills).
+  __device__ __forceinline__ RingSlot slot(int it) const {
+    RingSlot c;
+    c.s = it % nst;
+    c.ph = (unsigned)(it / nst) & 1u;
+    return c;
+  }
+  __device__ __forceinline__ void advance(RingSlot& c) const {
+    if (++c.s == nst) { c.s = 0; c.ph ^= 1u; }
+  }
+  // producer: the empty barrier of a stage completes its phase ph ^ 1 before the first lap, so that lap passes at once.
+  // kSleep backs off between polls (mbar_wait_sleep) where the spinning lane would take the consumers' issue slots.
+  template <bool kSleep = false>
+  __device__ __forceinline__ RingStage acquire(const RingSlot& c, unsigned bytes) const {
+    if (kSleep) mbar_wait_sleep(empty + c.s, c.ph ^ 1u);
+    else mbar_wait(empty + c.s, c.ph ^ 1u);
+    mbar_expect_tx(full + c.s, bytes);
+    return {stage(c), full + c.s};
+  }
+  // consumer: wait until the stage's copies have landed
+  __device__ __forceinline__ const double* wait(const RingSlot& c) const {
+    mbar_wait(full + c.s, c.ph);
+    return stage(c);
+  }
+  // consumer warp: done with the stage
+  __device__ __forceinline__ void release(const RingSlot& c) const {
+    __syncwarp();
+    if ((threadIdx.x & 31) == 0) mbar_arrive(empty + c.s);
+  }
+};
+
 }  // namespace hmv

@@ -1,22 +1,34 @@
 // k_power.cu -- K5: fused 1-halo + 2-halo mass integrals (reference hmvec.py:469-572).
 //
-// HBM-bound streaming reductions over the mass axis of the u(z,M,k) cubes.  A CTA owns one redshift and a 512-wide
-// k tile and walks the whole mass axis: one producer lane issues 1-D bulk async copies (cp.async.bulk -> TMA unit) of
-// a few rows of every cube it needs plus the rows' 64-byte coefficient records into a shared-memory ring tracked by
-// mbarriers; eight consumer warps read the ring, each thread owning two adjacent k for ALL masses (no cross-thread
+// HBM-bound streaming reductions over the mass axis of the u(z,M,k) cubes.  A CTA owns one redshift and a k tile and
+// walks the whole mass axis: one producer lane issues 1-D bulk async copies (cp.async.bulk -> TMA unit) of a few rows of
+// every cube it needs plus the rows' 64-byte coefficient records into a shared-memory stage ring (BulkRing,
+// common.cuh); the consumer warps read the ring, each thread owning adjacent k for ALL masses (no cross-thread
 // reduction).  The trapezoid-in-linear-M weights, n(M,z), b(M,z) and the tracer amplitudes are folded into the
-// per-(z,M) records by a small prep kernel; the epilogue applies the 1-halo damping, the consistency terms and
-// P_lin.  Algorithmic traffic: 8*nm bytes per (z,k) per distinct cube read.
+// per-(z,M) records by a small prep kernel; the epilogue applies the 1-halo damping, the consistency terms and P_lin.
+// Algorithmic traffic: 8*nm bytes per (z,k) per distinct cube read.
+//   power_prep_kernel      coefficient records of a tracer pair (hmv_power, hmv_power_tab)
 //   power_pair_kernel      any tracer pair (matter / HOD / pressure), up to four distinct cubes
+//   power_one_kernel       a pair whose two legs read the same single cube and no central-profile cube
+//   power_six_prep_kernel  coefficient records of the six spectra (hmv_power_six, _six_tab, _six_nfw)
 //   power_six_kernel       {mm, ee, me, gg, gm, ge} in one pass over two cubes
-//   power_six_nfw_kernel   the same with the NFW profile evaluated in-kernel (spectra-only fusion)
+//   power_six_tab_kernel   the same with the electron profile interpolated from its bin tables
+//   power_one_tab_kernel   the auto spectrum of one profile given as bin tables (P_yy); nothing is streamed
+//   tile_range_kernel      {min, max} of ks, the range of power_six_nfw_kernel's polynomial records
+//   power_six_nfw_kernel   the six spectra with the NFW profile evaluated in-kernel (spectra-only fusion)
 #include <cstdlib>
+#include <initializer_list>
 #include "common.cuh"
 #include "nfw_device.cuh"
 #include "nfw_poly.cuh"
 
 namespace hmv {
 
+// 1-halo damping 1 - exp(-(k/kstar)^2) (hmvec.py:526)
+__device__ __forceinline__ double damp_1h(double k, double kstar) {
+  const double r = k / kstar;
+  return 1.0 - exp(-r * r);
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // prep: per-(z,M) coefficient rows + per-z offsets
@@ -83,7 +95,7 @@ __global__ void __launch_bounds__(256) power_prep_kernel(int nm, const double* _
   }
 }
 
-// Generic tracer pair on the same TMA ring as power_six_kernel: up to four distinct cubes (us_A, uc_A, us_B, uc_B,
+// Generic tracer pair on the same ring as power_six_kernel: up to four distinct cubes (us_A, uc_A, us_B, uc_B,
 // de-duplicated by pointer) are streamed once; a stage holds PR_R rows of every cube plus the rows' 64-byte records.
 constexpr int PR_K = 512, PR_R = 4, PR_CT = 256;
 
@@ -97,38 +109,34 @@ struct PairArgs {
   double *p1h, *p2h;
 };
 
+// P1h and P2h of one (z, k) of a tracer pair (hmvec.py:526, 572)
+__device__ __forceinline__ void pair_epilogue(const PairArgs& a, int z, int k, double p1, double iA, double iB) {
+  const long long o = (long long)z * a.nk + k;
+  if (a.p1h) a.p1h[o] = p1 * damp_1h(a.ks[k], a.kstar);
+  if (a.p2h) a.p2h[o] = a.Pzk[o] * (iA + a.zoff[2 * z]) * (iB + a.zoff[2 * z + 1]);
+}
+
 __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArgs a) {
   extern __shared__ __align__(128) unsigned char pair_smem[];
-  const int stage_doubles = a.ncube * PR_R * PR_K + PR_R * 8;
-  double* ring = reinterpret_cast<double*>(pair_smem);
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)a.nst * stage_doubles);
-  unsigned long long* empty = full + a.nst;
+  const BulkRing ring(pair_smem, a.nst, a.ncube * PR_R * PR_K + PR_R * 8, PR_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int z = blockIdx.y, k0 = blockIdx.x * PR_K;
   const int segk = min(PR_K, a.ldk - k0);
   const long long zrow = (long long)z * a.nm;
   const int nit = (a.nm + PR_R - 1) / PR_R;
-  if (tid == 0) {
-    for (int s = 0; s < a.nst; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, PR_CT / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   __syncthreads();
+  RingSlot slot;
 
   if (warp == PR_CT / 32) {            // ---- producer warp ----
     if (lane == 0) {
       const unsigned segb = (unsigned)segk * 8u;
-      int s = 0;
-      unsigned ph = 0;
-      for (int it = 0; it < nit; ++it) {
-        mbar_wait(empty + s, ph ^ 1u);
+      for (int it = 0; it < nit; ++it, ring.advance(slot)) {
         const int m0 = it * PR_R, rows = min(PR_R, a.nm - m0);
-        double* st = ring + (size_t)s * stage_doubles;
-        mbar_expect_tx(full + s, (unsigned)rows * ((unsigned)a.ncube * segb + 64u));
+        const RingStage st = ring.acquire(slot, (unsigned)rows * ((unsigned)a.ncube * segb + 64u));
         for (int c = 0; c < a.ncube; ++c)
           for (int r = 0; r < rows; ++r)
-            bulk_g2s(st + (c * PR_R + r) * PR_K, a.cube[c] + (zrow + m0 + r) * (long long)a.ldk + k0, segb, full + s);
-        bulk_g2s(st + a.ncube * PR_R * PR_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, full + s);
-        if (++s == a.nst) { s = 0; ph ^= 1u; }
+            bulk_g2s(st.p + (c * PR_R + r) * PR_K, a.cube[c] + (zrow + m0 + r) * (long long)a.ldk + k0, segb, st.full);
+        bulk_g2s(st.p + a.ncube * PR_R * PR_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
       }
     }
     return;
@@ -137,12 +145,9 @@ __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArg
   const bool active = 2 * tid < segk;
   double2 p1 = {0, 0}, iA = {0, 0}, iB = {0, 0};
   const double2 one = make_double2(1.0, 1.0);
-  int s = 0;
-  unsigned ph = 0;
-  for (int it = 0; it < nit; ++it) {
+  for (int it = 0; it < nit; ++it, ring.advance(slot)) {
     const int rows = min(PR_R, a.nm - it * PR_R);
-    const double* st = ring + (size_t)s * stage_doubles;
-    mbar_wait(full + s, ph);
+    const double* st = ring.wait(slot);
     if (active) {
 #pragma unroll
       for (int r = 0; r < PR_R; ++r) {
@@ -169,21 +174,14 @@ __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArg
         }
       }
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + s);
-    if (++s == a.nst) { s = 0; ph ^= 1u; }
+    ring.release(slot);
   }
   if (!active) return;
 #pragma unroll
   for (int e = 0; e < 2; ++e) {
     const int k = k0 + 2 * tid + e;
     if (k >= a.nk) break;
-    const long long o = (long long)z * a.nk + k;
-    if (a.p1h) {
-      const double r = a.ks[k] / a.kstar;
-      a.p1h[o] = (e ? p1.y : p1.x) * (1.0 - exp(-r * r));                                   // hmvec.py:526
-    }
-    if (a.p2h) a.p2h[o] = a.Pzk[o] * ((e ? iA.y : iA.x) + a.zoff[2 * z]) * ((e ? iB.y : iB.x) + a.zoff[2 * z + 1]);   // hmvec.py:572
+    pair_epilogue(a, z, k, e ? p1.y : p1.x, e ? iA.y : iA.x, e ? iB.y : iB.x);
   }
 }
 
@@ -194,37 +192,26 @@ __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArg
 // 5.9 TB/s); this one streams at the HBM rate.
 constexpr int ONE_K = 1024, ONE_R = 4, ONE_NST = 5, ONE_CT = 256;
 constexpr int ONE_STAGE_DOUBLES = ONE_R * ONE_K + ONE_R * 8;
-constexpr size_t ONE_SMEM = (size_t)ONE_NST * ONE_STAGE_DOUBLES * sizeof(double) + 2 * ONE_NST * sizeof(unsigned long long);
 
 __global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArgs a) {
   extern __shared__ __align__(128) unsigned char one_smem[];
-  double* ring = reinterpret_cast<double*>(one_smem);
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)ONE_NST * ONE_STAGE_DOUBLES);
-  unsigned long long* empty = full + ONE_NST;
+  const BulkRing ring(one_smem, ONE_NST, ONE_STAGE_DOUBLES, ONE_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int z = blockIdx.y, k0 = blockIdx.x * ONE_K;
   const int segk = min(ONE_K, a.ldk - k0);                 // doubles per row segment (multiple of 2)
   const long long zrow = (long long)z * a.nm;
   const int nit = (a.nm + ONE_R - 1) / ONE_R;
-  if (tid == 0) {
-    for (int s = 0; s < ONE_NST; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, ONE_CT / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   __syncthreads();
 
   if (warp == ONE_CT / 32) {            // ---- producer warp ----
     if (lane == 0) {
       const unsigned segb = (unsigned)segk * 8u;
       for (int it = 0; it < nit; ++it) {
-        const int s = it % ONE_NST;
-        const unsigned ph = (unsigned)(it / ONE_NST) & 1u;
-        mbar_wait(empty + s, ph ^ 1u);
         const int m0 = it * ONE_R, rows = min(ONE_R, a.nm - m0);
-        double* st = ring + (size_t)s * ONE_STAGE_DOUBLES;
-        mbar_expect_tx(full + s, (unsigned)rows * (segb + 64u));
+        const RingStage st = ring.acquire(ring.slot(it), (unsigned)rows * (segb + 64u));
         for (int r = 0; r < rows; ++r)
-          bulk_g2s(st + r * ONE_K, a.cube[0] + (zrow + m0 + r) * (long long)a.ldk + k0, segb, full + s);
-        bulk_g2s(st + ONE_R * ONE_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, full + s);
+          bulk_g2s(st.p + r * ONE_K, a.cube[0] + (zrow + m0 + r) * (long long)a.ldk + k0, segb, st.full);
+        bulk_g2s(st.p + ONE_R * ONE_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
       }
     }
     return;
@@ -234,11 +221,9 @@ __global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArg
   const bool act0 = 2 * tid < segk, act1 = 512 + 2 * tid < segk;
   double p1[4] = {0, 0, 0, 0}, iA[4] = {0, 0, 0, 0}, iB[4] = {0, 0, 0, 0};
   for (int it = 0; it < nit; ++it) {
-    const int s = it % ONE_NST;
-    const unsigned ph = (unsigned)(it / ONE_NST) & 1u;
+    const RingSlot slot = ring.slot(it);
     const int rows = min(ONE_R, a.nm - it * ONE_R);
-    const double* st = ring + (size_t)s * ONE_STAGE_DOUBLES;
-    mbar_wait(full + s, ph);
+    const double* st = ring.wait(slot);
     if (act0) {
 #pragma unroll
       for (int r = 0; r < ONE_R; ++r) {
@@ -259,19 +244,13 @@ __global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArg
         }
       }
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + s);
+    ring.release(slot);
   }
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
     const int k = k0 + (e >> 1) * 512 + 2 * tid + (e & 1);
     if (k >= a.nk || (e < 2 ? !act0 : !act1)) continue;
-    const long long o = (long long)z * a.nk + k;
-    if (a.p1h) {
-      const double r = a.ks[k] / a.kstar;
-      a.p1h[o] = p1[e] * (1.0 - exp(-r * r));                                                 // hmvec.py:526
-    }
-    if (a.p2h) a.p2h[o] = a.Pzk[o] * (iA[e] + a.zoff[2 * z]) * (iB[e] + a.zoff[2 * z + 1]);   // hmvec.py:572
+    pair_epilogue(a, z, k, p1[e], iA[e], iB[e]);
   }
 }
 
@@ -360,50 +339,84 @@ static int wave_tile(int nz, int ldk, int tile_max, int per_sm) {
 
 constexpr int SIX_K = 512, SIX_R = 4, SIX_NST = 6, SIX_CT = 256;   // k per CTA, rows per stage, stages, consumers
 constexpr int SIX_STAGE_DOUBLES = 2 * SIX_R * SIX_K + SIX_R * 8;
-constexpr size_t SIX_SMEM = (size_t)SIX_NST * SIX_STAGE_DOUBLES * sizeof(double) + 2 * SIX_NST * sizeof(unsigned long long);
 
-struct SixArgs {
-  int nz, nm, nk, ldk;
-  int tk;                  // k per CTA (multiple of 16, <= SIX_K): chosen per launch so that the grid fills whole waves
+// what the six-spectra epilogue reads besides the sums, and where it writes P1h / P2h of {mm, ee, me, gg, gm, ge}
+struct SixOut {
   long long spec_stride;   // doubles between consecutive spectra in p1h/p2h
-  const double *um, *ue, *coef;
   const double *zoff, *ks, *Pzk;
   double kstar;
   double *p1h, *p2h;
 };
 
+struct SixArgs {
+  int nm, nk, ldk;
+  int tk;                  // k per CTA (multiple of 16, <= SIX_K): chosen per launch so that the grid fills whole waves
+  const double *um, *ue, *coef;
+  SixOut out;
+};
+
+// the seven coefficients of a mass row's 64-byte record (power_six_prep_kernel)
+struct SixCoef { double A1, c1, c2, B1, B2, D1, D2; };
+
+__device__ __forceinline__ SixCoef six_coef(const double* rec) {
+  const double2* c = reinterpret_cast<const double2*>(rec);
+  const double2 c01 = c[0], c23 = c[1], c45 = c[2], c67 = c[3];
+  return {c01.x, c01.y, c23.x, c23.y, c45.x, c45.y, c67.x};
+}
+
+// one mass row at one wavenumber: 18 FMAs into the six 1-halo sums acc[0..6) and the 2-halo legs acc[6..9) (m, e, g)
+__device__ __forceinline__ void six_fma(double (&acc)[9], const SixCoef& c, double um, double ue) {
+  const double q1 = um * um, q2 = ue * ue, q3 = um * ue;
+  acc[0] = fma(c.A1, q1, acc[0]);
+  acc[1] = fma(c.A1, q2, acc[1]);
+  acc[2] = fma(c.A1, q3, acc[2]);
+  acc[3] = fma(c.c1, um, fma(c.c2, q1, acc[3]));
+  acc[4] = fma(c.B1, um, fma(c.B2, q1, acc[4]));
+  acc[5] = fma(c.B1, ue, fma(c.B2, q3, acc[5]));
+  acc[6] = fma(c.D1, um, acc[6]);
+  acc[7] = fma(c.D1, ue, acc[7]);
+  acc[8] = fma(c.D2, um, acc[8]);
+}
+
+// the six spectra of redshift z at wavenumber index k < nk (hmvec.py:526, 572)
+__device__ __forceinline__ void six_epilogue(const SixOut& a, int z, int nk, int k, const double (&acc)[9]) {
+  const long long S = a.spec_stride, o = (long long)z * nk + k;
+  const double zo0 = a.zoff[2 * z], zo1 = a.zoff[2 * z + 1];
+  if (a.p1h) {
+    const double damp = damp_1h(a.ks[k], a.kstar);
+#pragma unroll
+    for (int q = 0; q < 6; ++q) a.p1h[q * S + o] = acc[q] * damp;
+  }
+  if (a.p2h) {
+    const double P = a.Pzk[o];
+    const double Lm = acc[6] + zo0, Le = acc[7] + zo0, Lg = acc[8] + zo1;
+    a.p2h[0 * S + o] = P * Lm * Lm; a.p2h[1 * S + o] = P * Le * Le; a.p2h[2 * S + o] = P * Lm * Le;
+    a.p2h[3 * S + o] = P * Lg * Lg; a.p2h[4 * S + o] = P * Lg * Lm; a.p2h[5 * S + o] = P * Lg * Le;
+  }
+}
+
 __global__ void __launch_bounds__(SIX_CT + 32, 1) power_six_kernel(const SixArgs a) {
   extern __shared__ __align__(128) unsigned char six_smem[];
-  double* ring = reinterpret_cast<double*>(six_smem);
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)SIX_NST * SIX_STAGE_DOUBLES);
-  unsigned long long* empty = full + SIX_NST;
+  const BulkRing ring(six_smem, SIX_NST, SIX_STAGE_DOUBLES, SIX_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int z = blockIdx.y, k0 = blockIdx.x * a.tk;
   const int segk = min(a.tk, a.ldk - k0);                  // doubles per row segment (multiple of 2)
   const long long zrow = (long long)z * a.nm;
   const int nit = (a.nm + SIX_R - 1) / SIX_R;
-  if (tid == 0) {
-    for (int s = 0; s < SIX_NST; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, SIX_CT / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   __syncthreads();
 
   if (warp == SIX_CT / 32) {            // ---- producer warp: one elected lane drives the TMA unit ----
     if (lane == 0) {
       const unsigned segb = (unsigned)segk * 8u;
       for (int it = 0; it < nit; ++it) {
-        const int s = it % SIX_NST;
-        const unsigned ph = (unsigned)(it / SIX_NST) & 1u;
-        mbar_wait(empty + s, ph ^ 1u);                     // first lap passes immediately
         const int m0 = it * SIX_R, rows = min(SIX_R, a.nm - m0);
-        double* st = ring + (size_t)s * SIX_STAGE_DOUBLES;
-        mbar_expect_tx(full + s, (unsigned)rows * (2u * segb + 64u));
+        const RingStage st = ring.acquire(ring.slot(it), (unsigned)rows * (2u * segb + 64u));
         for (int r = 0; r < rows; ++r) {
           const long long off = (zrow + m0 + r) * (long long)a.ldk + k0;
-          bulk_g2s(st + r * SIX_K, a.um + off, segb, full + s);
-          bulk_g2s(st + (SIX_R + r) * SIX_K, a.ue + off, segb, full + s);
+          bulk_g2s(st.p + r * SIX_K, a.um + off, segb, st.full);
+          bulk_g2s(st.p + (SIX_R + r) * SIX_K, a.ue + off, segb, st.full);
         }
-        bulk_g2s(st + 2 * SIX_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, full + s);
+        bulk_g2s(st.p + 2 * SIX_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
       }
     }
     return;
@@ -411,91 +424,49 @@ __global__ void __launch_bounds__(SIX_CT + 32, 1) power_six_kernel(const SixArgs
 
   // ---- consumers: thread owns k = k0 + 2 tid, +1 over the whole mass axis ----
   const bool active = 2 * tid < segk;
-  double2 acc[9];
-#pragma unroll
-  for (int q = 0; q < 9; ++q) acc[q] = make_double2(0.0, 0.0);
+  double acc[2][9] = {};
   for (int it = 0; it < nit; ++it) {
-    const int s = it % SIX_NST;
-    const unsigned ph = (unsigned)(it / SIX_NST) & 1u;
+    const RingSlot slot = ring.slot(it);
     const int rows = min(SIX_R, a.nm - it * SIX_R);
-    const double* st = ring + (size_t)s * SIX_STAGE_DOUBLES;
-    mbar_wait(full + s, ph);
+    const double* st = ring.wait(slot);
     if (active) {
 #pragma unroll
       for (int r = 0; r < SIX_R; ++r) {
         if (r < rows) {
           const double2 um = *reinterpret_cast<const double2*>(st + r * SIX_K + 2 * tid);
           const double2 ue = *reinterpret_cast<const double2*>(st + (SIX_R + r) * SIX_K + 2 * tid);
-          const double2* c = reinterpret_cast<const double2*>(st + 2 * SIX_R * SIX_K + r * 8);
-          const double2 c01 = c[0], c23 = c[1], c45 = c[2], c67 = c[3];
-          const double A1 = c01.x, c1 = c01.y, c2 = c23.x, B1 = c23.y, B2 = c45.x, D1 = c45.y, D2 = c67.x;
-#define HMV_SIX(c)                                                          \
-  {                                                                         \
-    const double q1 = um.c * um.c, q2 = ue.c * ue.c, q3 = um.c * ue.c;      \
-    acc[0].c = fma(A1, q1, acc[0].c);                                       \
-    acc[1].c = fma(A1, q2, acc[1].c);                                       \
-    acc[2].c = fma(A1, q3, acc[2].c);                                       \
-    acc[3].c = fma(c1, um.c, fma(c2, q1, acc[3].c));                        \
-    acc[4].c = fma(B1, um.c, fma(B2, q1, acc[4].c));                        \
-    acc[5].c = fma(B1, ue.c, fma(B2, q3, acc[5].c));                        \
-    acc[6].c = fma(D1, um.c, acc[6].c);                                     \
-    acc[7].c = fma(D1, ue.c, acc[7].c);                                     \
-    acc[8].c = fma(D2, um.c, acc[8].c);                                     \
-  }
-          HMV_SIX(x)
-          HMV_SIX(y)
-#undef HMV_SIX
+          const SixCoef c = six_coef(st + 2 * SIX_R * SIX_K + r * 8);
+          six_fma(acc[0], c, um.x, ue.x);
+          six_fma(acc[1], c, um.y, ue.y);
         }
       }
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + s);                 // this warp is done with the stage
+    ring.release(slot);
   }
   if (!active) return;
-  const long long S = a.spec_stride;
-  const double zo0 = a.zoff[2 * z], zo1 = a.zoff[2 * z + 1];
 #pragma unroll
   for (int e = 0; e < 2; ++e) {
     const int k = k0 + 2 * tid + e;
     if (k >= a.nk) break;
-    double sv[9];
-#pragma unroll
-    for (int q = 0; q < 9; ++q) sv[q] = e ? acc[q].y : acc[q].x;
-    const long long o = (long long)z * a.nk + k;
-    if (a.p1h) {
-      const double r = a.ks[k] / a.kstar, damp = 1.0 - exp(-r * r);          // hmvec.py:526
-#pragma unroll
-      for (int q = 0; q < 6; ++q) a.p1h[q * S + o] = sv[q] * damp;
-    }
-    if (a.p2h) {                                                           // hmvec.py:572
-      const double P = a.Pzk[o];
-      const double Lm = sv[6] + zo0, Le = sv[7] + zo0, Lg = sv[8] + zo1;
-      a.p2h[0 * S + o] = P * Lm * Lm; a.p2h[1 * S + o] = P * Le * Le; a.p2h[2 * S + o] = P * Lm * Le;
-      a.p2h[3 * S + o] = P * Lg * Lg; a.p2h[4 * S + o] = P * Lg * Lm; a.p2h[5 * S + o] = P * Lg * Le;
-    }
+    six_epilogue(a.out, z, a.nk, k, acc[e]);
   }
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // The six spectra with the ELECTRON profile interpolated from its bin tables inside the reduction (hmv_profile_tables:
 // the transform's result before the expansion onto ks) instead of read from a cube: the 32 GB cube is neither written
-// nor re-read, the kernel streams the matter cube plus ~1 GB of table segments.  A CTA (z, 512-wide k tile) needs of
-// halo m only the bins between floor(kmin_tile * inv_m) and floor(kmax_tile * inv_m) + 1: the producer warp works
-// out those segments for up to four rows per stage (one lane per row), packs them behind the rows' matter segments
-// and coefficient records, and describes them in a small header; rows whose whole tile lies below the first bin
-// (u_e = u_1) or above the last one (u_e = 0) need no table data at all.  Consumers interpolate exactly as the
-// transform's own expansion does (np.interp semantics of fft.py:102-107).
+// nor re-read, the kernel streams the matter cube plus the rows' table parameters, and gathers the two bins around
+// each wavenumber from the tables (which the redshift's CTAs share in L2).  A row whose t = k * inv lies below the
+// first bin holds u_e = u_1, above the last one u_e = 0.  Consumers interpolate exactly as the transform's own
+// expansion does (np.interp semantics of fft.py:102-107).
 // ---------------------------------------------------------------------------------------------------------
 constexpr int TAB_R = 4, TAB_CT = 256, TAB_NST = 6;
 constexpr int TAB_STAGE_DOUBLES = TAB_R * SIX_K + TAB_R * 8 + TAB_R * 4;       // matter rows, coefficient records, table parameters
-constexpr size_t TAB_SMEM = (size_t)TAB_NST * TAB_STAGE_DOUBLES * sizeof(double) + 2 * TAB_NST * sizeof(unsigned long long);
 
 struct SixTabArgs {
-  int nz, nm, nk, ldk, nmp, JS, J;
-  long long spec_stride;
-  const double *um, *coef, *zoff, *ks, *Pzk, *tab, *tmeta;
-  double kstar;
-  double *p1h, *p2h;
+  int nm, nk, ldk, nmp, JS, J;
+  const double *um, *coef, *tab, *tmeta;
+  SixOut out;
 };
 
 // what a thread keeps of one (row, wavenumber) between issuing the two table loads and using them
@@ -518,35 +489,25 @@ __device__ __forceinline__ double tab_value(const TabLerp& r, double u1) {
 
 __global__ void __launch_bounds__(TAB_CT + 32, 1) power_six_tab_kernel(const SixTabArgs a) {
   extern __shared__ __align__(128) unsigned char tab_smem[];
-  double* ring = reinterpret_cast<double*>(tab_smem);
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)TAB_NST * TAB_STAGE_DOUBLES);
-  unsigned long long* empty = full + TAB_NST;
+  const BulkRing ring(tab_smem, TAB_NST, TAB_STAGE_DOUBLES, TAB_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int z = blockIdx.y, k0 = blockIdx.x * SIX_K;
   const int segk = min(SIX_K, a.ldk - k0);
   const long long zrow = (long long)z * a.nm, zrowp = (long long)z * a.nmp;
   const double tJ = (double)a.J;
   const int nit = (a.nm + TAB_R - 1) / TAB_R;
-  if (tid == 0) {
-    for (int s = 0; s < TAB_NST; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, TAB_CT / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   __syncthreads();
 
   if (warp == TAB_CT / 32) {            // ---- producer warp: one elected lane drives the TMA unit ----
     if (lane == 0) {
       const unsigned segb = (unsigned)segk * 8u;
       for (int it = 0; it < nit; ++it) {
-        const int s = it % TAB_NST;
-        const unsigned ph = (unsigned)(it / TAB_NST) & 1u;
-        mbar_wait(empty + s, ph ^ 1u);
         const int m0 = it * TAB_R, rows = min(TAB_R, a.nm - m0);
-        double* st = ring + (size_t)s * TAB_STAGE_DOUBLES;
-        mbar_expect_tx(full + s, (unsigned)rows * (segb + 64u + 32u));
+        const RingStage st = ring.acquire(ring.slot(it), (unsigned)rows * (segb + 64u + 32u));
         for (int r = 0; r < rows; ++r)
-          bulk_g2s(st + r * SIX_K, a.um + (zrow + m0 + r) * (long long)a.ldk + k0, segb, full + s);
-        bulk_g2s(st + TAB_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, full + s);
-        bulk_g2s(st + TAB_R * SIX_K + TAB_R * 8, a.tmeta + (zrowp + m0) * 4, (unsigned)rows * 32u, full + s);
+          bulk_g2s(st.p + r * SIX_K, a.um + (zrow + m0 + r) * (long long)a.ldk + k0, segb, st.full);
+        bulk_g2s(st.p + TAB_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
+        bulk_g2s(st.p + TAB_R * SIX_K + TAB_R * 8, a.tmeta + (zrowp + m0) * 4, (unsigned)rows * 32u, st.full);
       }
     }
     return;
@@ -556,16 +517,11 @@ __global__ void __launch_bounds__(TAB_CT + 32, 1) power_six_tab_kernel(const Six
   //      (from the stage's parameter records, as soon as they have landed) before stage i is accumulated ----
   const bool active = 2 * tid < segk;
   const int kc = min(k0 + 2 * tid, a.nk - 1), kc1 = min(k0 + 2 * tid + 1, a.nk - 1);
-  const double kx = a.ks[kc], ky = a.ks[kc1];
-  double2 acc[9];
-#pragma unroll
-  for (int q = 0; q < 9; ++q) acc[q] = make_double2(0.0, 0.0);
+  const double kx = a.out.ks[kc], ky = a.out.ks[kc1];
+  double acc[2][9] = {};
   TabLerp cur[TAB_R][2], nxt[TAB_R][2];
   auto issue = [&](int it, TabLerp (&dst)[TAB_R][2]) {
-    const int s = it % TAB_NST;
-    const unsigned ph = (unsigned)(it / TAB_NST) & 1u;
-    mbar_wait(full + s, ph);
-    const double4* pm = reinterpret_cast<const double4*>(ring + (size_t)s * TAB_STAGE_DOUBLES + TAB_R * SIX_K + TAB_R * 8);
+    const double4* pm = reinterpret_cast<const double4*>(ring.wait(ring.slot(it)) + TAB_R * SIX_K + TAB_R * 8);
     const int m0 = it * TAB_R, rows = min(TAB_R, a.nm - m0);
 #pragma unroll
     for (int r = 0; r < TAB_R; ++r) {
@@ -578,14 +534,13 @@ __global__ void __launch_bounds__(TAB_CT + 32, 1) power_six_tab_kernel(const Six
   };
   if (active) issue(0, cur);
   for (int it = 0; it < nit; ++it) {
-    const int s = it % TAB_NST;
-    const unsigned ph = (unsigned)(it / TAB_NST) & 1u;
+    const RingSlot slot = ring.slot(it);
     const int rows = min(TAB_R, a.nm - it * TAB_R);
-    const double* st = ring + (size_t)s * TAB_STAGE_DOUBLES;
+    const double* st = ring.stage(slot);
     if (active) {
       if (it + 1 < nit) issue(it + 1, nxt);
     } else {
-      mbar_wait(full + s, ph);
+      ring.wait(slot);
     }
     if (active) {
       const double4* pm = reinterpret_cast<const double4*>(st + TAB_R * SIX_K + TAB_R * 8);
@@ -594,56 +549,22 @@ __global__ void __launch_bounds__(TAB_CT + 32, 1) power_six_tab_kernel(const Six
         if (r < rows) {
           const double2 um = *reinterpret_cast<const double2*>(st + r * SIX_K + 2 * tid);
           const double u1 = pm[r].y;
-          const double2 ue = make_double2(tab_value(cur[r][0], u1), tab_value(cur[r][1], u1));
-          const double2* c = reinterpret_cast<const double2*>(st + TAB_R * SIX_K + r * 8);
-          const double2 c01 = c[0], c23 = c[1], c45 = c[2], c67 = c[3];
-          const double A1 = c01.x, c1 = c01.y, c2 = c23.x, B1 = c23.y, B2 = c45.x, D1 = c45.y, D2 = c67.x;
-#define HMV_SIX(c)                                                          \
-  {                                                                         \
-    const double q1 = um.c * um.c, q2 = ue.c * ue.c, q3 = um.c * ue.c;      \
-    acc[0].c = fma(A1, q1, acc[0].c);                                       \
-    acc[1].c = fma(A1, q2, acc[1].c);                                       \
-    acc[2].c = fma(A1, q3, acc[2].c);                                       \
-    acc[3].c = fma(c1, um.c, fma(c2, q1, acc[3].c));                        \
-    acc[4].c = fma(B1, um.c, fma(B2, q1, acc[4].c));                        \
-    acc[5].c = fma(B1, ue.c, fma(B2, q3, acc[5].c));                        \
-    acc[6].c = fma(D1, um.c, acc[6].c);                                     \
-    acc[7].c = fma(D1, ue.c, acc[7].c);                                     \
-    acc[8].c = fma(D2, um.c, acc[8].c);                                     \
-  }
-          HMV_SIX(x)
-          HMV_SIX(y)
-#undef HMV_SIX
+          const SixCoef c = six_coef(st + TAB_R * SIX_K + r * 8);
+          six_fma(acc[0], c, um.x, tab_value(cur[r][0], u1));
+          six_fma(acc[1], c, um.y, tab_value(cur[r][1], u1));
         }
       }
 #pragma unroll
       for (int r = 0; r < TAB_R; ++r) { cur[r][0] = nxt[r][0]; cur[r][1] = nxt[r][1]; }
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + s);
+    ring.release(slot);
   }
   if (!active) return;
-  const long long S = a.spec_stride;
-  const double zo0 = a.zoff[2 * z], zo1 = a.zoff[2 * z + 1];
 #pragma unroll
   for (int e = 0; e < 2; ++e) {
     const int k = k0 + 2 * tid + e;
     if (k >= a.nk) break;
-    double sv[9];
-#pragma unroll
-    for (int q = 0; q < 9; ++q) sv[q] = e ? acc[q].y : acc[q].x;
-    const long long o = (long long)z * a.nk + k;
-    if (a.p1h) {
-      const double r = a.ks[k] / a.kstar, damp = 1.0 - exp(-r * r);          // hmvec.py:526
-#pragma unroll
-      for (int q = 0; q < 6; ++q) a.p1h[q * S + o] = sv[q] * damp;
-    }
-    if (a.p2h) {                                                           // hmvec.py:572
-      const double P = a.Pzk[o];
-      const double Lm = sv[6] + zo0, Le = sv[7] + zo0, Lg = sv[8] + zo1;
-      a.p2h[0 * S + o] = P * Lm * Lm; a.p2h[1 * S + o] = P * Le * Le; a.p2h[2 * S + o] = P * Lm * Le;
-      a.p2h[3 * S + o] = P * Lg * Lg; a.p2h[4 * S + o] = P * Lg * Lm; a.p2h[5 * S + o] = P * Lg * Le;
-    }
+    six_epilogue(a.out, z, a.nk, k, acc[e]);
   }
 }
 
@@ -656,32 +577,29 @@ __global__ void __launch_bounds__(TAB_CT + 32, 1) power_six_tab_kernel(const Six
 // wavenumbers from the halo's table row in L2 exactly as the transform's expansion does (fft.py:102-107).
 // Work is proportional to the interpolated elements (37 % on the LARGE grid).
 // ---------------------------------------------------------------------------------------------------------
-#ifndef HMV_OT_ORDER
-#define HMV_OT_ORDER 1        // 1: k tiles slow and descending (expensive tiles of every redshift first), 0: z slow
-#endif
-#ifndef HMV_OT_ZC
-#define HMV_OT_ZC 100         // ... within chunks of this many redshifts
-#endif
-#ifndef HMV_OT_T
-#define HMV_OT_T 256          // threads per CTA (a thread owns two adjacent wavenumbers)
-#define HMV_OT_MINB 2         // CTAs per SM the register allocation aims at
-#define HMV_OT_UNROLL 6       // halos in flight per thread in the interior loop
-#endif
-// Measured on a 67-z slab (gpurun_out/r2_ot_variants.txt): 6 halos in flight 1.02 ms against 1.10 with 4 (8 spills);
-// prefetch instructions (L1 or L2) for the table line of the halo 4 / 8 / 16 positions ahead: 1.20-1.25 ms -- slower,
-// the extra address arithmetic costs more than the earlier arrival saves.  A ninth warp that walks the halo lists ahead
-// of the others and asks L2 for every halo's whole table segment with coalesced prefetches (32 / 96 / 256 halos
-// ahead): 1.60 ms against 1.03 (gpurun_out/r2_ot_pfw.txt) -- the gathers are not waiting for DRAM alone.
-constexpr int OT_T = HMV_OT_T, OT_K = 2 * OT_T, OT_UNROLL = HMV_OT_UNROLL;
+// 256 threads per CTA (a thread owns two adjacent wavenumbers), register allocation for 2 CTAs per SM, 6 halos in
+// flight per thread in the interior loop.  Measured on a B200 on a 67-z slab: 6 halos in flight
+// 1.02 ms against 1.10 with 4 (8 spills); prefetch instructions (L1 or L2) for the table line of the halo 4 / 8 / 16
+// positions ahead: 1.20-1.25 ms -- slower, the extra address arithmetic costs more than the earlier arrival saves.  A
+// ninth warp that walks the halo lists ahead of the others and asks L2 for every halo's whole table segment with
+// coalesced prefetches (32 / 96 / 256 halos ahead): 1.60 ms against 1.03 -- the gathers are
+// not waiting for DRAM alone.
+constexpr int OT_T = 256, OT_K = 2 * OT_T, OT_MINB = 2, OT_UNROLL = 6;
+// CTA order: k tiles are the slow index, highest k first, within chunks of OT_ZC redshifts.  A tile's cost is the
+// number of halos it has to interpolate (none at low k, where every halo holds u_1), so the expensive tiles of every
+// redshift go first and the launch drains on the trivial ones.  Measured on a B200 against redshift-slow
+// order: 25 z 0.454 -> 0.385 ms, 67 z 1.013 -> 0.858, 100 z 1.49 -> 1.33, 200 z 2.63 -> 2.52 (chunks of
+// 100; 2.58 unchunked, 2.74 with chunks of 32 or 64).
+constexpr int OT_ZC = 100;
 
 // launch position -> (redshift, first wavenumber of the tile) of power_one_tab_kernel's tile-slow order
 __host__ __device__ __forceinline__ void ot_cta(int id, int nz, int nk, int& z, int& k0) {
-  const int T = (nk + OT_K - 1) / OT_K, per = HMV_OT_ZC * T;
+  const int T = (nk + OT_K - 1) / OT_K, per = OT_ZC * T;
   const int c = id / per, r = id - c * per;
-  const int left = nz - c * HMV_OT_ZC;
-  const int nzc = left < HMV_OT_ZC ? left : HMV_OT_ZC;
+  const int left = nz - c * OT_ZC;
+  const int nzc = left < OT_ZC ? left : OT_ZC;
   const int tr = r / nzc;
-  z = c * HMV_OT_ZC + (r - tr * nzc);
+  z = c * OT_ZC + (r - tr * nzc);
   k0 = (T - 1 - tr) * OT_K;
 }
 
@@ -692,7 +610,7 @@ struct OneTabArgs {
   double *p1h, *p2h;
 };
 
-__global__ void __launch_bounds__(OT_T, HMV_OT_MINB) power_one_tab_kernel(const OneTabArgs a) {
+__global__ void __launch_bounds__(OT_T, OT_MINB) power_one_tab_kernel(const OneTabArgs a) {
   extern __shared__ __align__(16) unsigned char ot_smem[];
   double4* prm = reinterpret_cast<double4*>(ot_smem);              // per interpolated halo: {inv, u_1, a, b} (t = a + b u)
   double2* prm2 = reinterpret_cast<double2*>(prm + a.nm);          //                        {c4, w2}
@@ -700,17 +618,8 @@ __global__ void __launch_bounds__(OT_T, HMV_OT_MINB) power_one_tab_kernel(const 
   __shared__ double red[3][OT_T / 32];
   __shared__ int nlist, nlist2, wcnt[OT_T / 32], wcnt2[OT_T / 32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-#if HMV_OT_ORDER
-  // k tiles are the slow index, highest k first, within chunks of HMV_OT_ZC redshifts: a tile's cost is the number of
-  // halos it has to interpolate (none at low k, where every halo holds u_1), so the expensive tiles of every redshift
-  // go first and the launch drains on the trivial ones.  Measured against redshift-slow order (gpurun_out/
-  // r2_ot_order*.txt): 25 z 0.454 -> 0.385 ms, 67 z 1.013 -> 0.858, 100 z 1.49 -> 1.33, 200 z 2.63 -> 2.52 (chunks of
-  // 100; 2.58 unchunked, 2.74 with chunks of 32 or 64).
   int z, k0;
   ot_cta(blockIdx.x, a.nz, a.nk, z, k0);
-#else
-  const int z = blockIdx.y, k0 = blockIdx.x * OT_K;
-#endif
   const long long zrow = (long long)z * a.nm, zrowp = (long long)z * a.nmp;
   const double tJ = (double)a.J;
   // wavenumber range of the tile (any order of ks)
@@ -825,10 +734,7 @@ __global__ void __launch_bounds__(OT_T, HMV_OT_MINB) power_one_tab_kernel(const 
     const int k = k0 + 2 * tid + e;
     if (k >= a.nk) break;
     const long long o = (long long)z * a.nk + k;
-    if (a.p1h) {
-      const double r = a.ks[k] / a.kstar;
-      a.p1h[o] = ((e ? p1y : p1x) + h1) * (1.0 - exp(-r * r));                                               // hmvec.py:526
-    }
+    if (a.p1h) a.p1h[o] = ((e ? p1y : p1x) + h1) * damp_1h(a.ks[k], a.kstar);
     if (a.p2h) {
       const double I = (e ? iAy : iAx) + hA + a.zoff[2 * z];
       a.p2h[o] = a.Pzk[o] * I * I;                                                                           // hmvec.py:572
@@ -838,12 +744,13 @@ __global__ void __launch_bounds__(OT_T, HMV_OT_MINB) power_one_tab_kernel(const 
 
 // ---------------------------------------------------------------------------------------------------------
 // Spectra-only fusion: the six spectra with the NFW matter profile evaluated IN the reduction instead of being read
-// from a cube.  u_NFW(k|M,z) depends on the halo only through (c, a = r_s (1+z)) and a 42-coefficient series, so a
-// 384-byte per-halo record replaces an 8*nk-byte cube row: the kernel streams only the electron cube (half the
-// HBM traffic of power_six_kernel and no 32 GB NFW store/reload) and spends the freed time in the FP64 pipe.
-//   rec[z][m][48] = { A[0..42) series coefficients, c, a, a*c, ln(1+c), 1/m_c, 0 }
-// Same ring/mbarrier structure as power_six_kernel; stage = SIX_R rows x (4 KB of u_e + 64 B coefficients + 384 B
-// NFW record).  k tiles are the slow grid dimension, highest k first: the Si/Ci-heavy tiles are scheduled first.
+// from a cube.  u_NFW(k|M,z) is a function of s = k r_s c (1+z) given by piecewise polynomials (nfw_poly.cuh,
+// k_nfw.cu), so a per-halo record of FREC doubles -- the halo's NFWP_REC polynomial coefficients, then
+// {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0} -- replaces an 8*nk-byte cube row: the kernel streams only the electron
+// cube (half the HBM traffic of power_six_kernel and no 32 GB NFW store/reload) and spends the freed time in the FP64
+// pipe on the Horner chains.  Beyond the last polynomial interval (s > 64) u_NFW takes its closed form (Si/Ci).
+// Same ring as power_six_kernel; stage = SIX_R rows x (4 KB of u_e + 64 B coefficients + FREC doubles of NFW record).
+// k tiles are the slow grid dimension, highest k first: the tiles that reach the closed form are scheduled first.
 // ---------------------------------------------------------------------------------------------------------
 // {min, max} of ks over [b*tile, (b+1)*tile) for each block b (one warp per block)
 __global__ void tile_range_kernel(int nk, int tile, const double* __restrict__ ks, double* __restrict__ tilek) {
@@ -862,33 +769,14 @@ constexpr int FREC = NFWP_REC + 6;          // per-halo record of the fused kern
                                             // {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0}
 constexpr int FSX_NST = 6;
 constexpr int FSX_STAGE_DOUBLES = SIX_R * SIX_K + SIX_R * 8 + SIX_R * FREC;
-constexpr size_t FSX_SMEM = (size_t)FSX_NST * FSX_STAGE_DOUBLES * sizeof(double) + 2 * FSX_NST * sizeof(unsigned long long);
 
 struct FusedArgs {
-  int nz, nm, nk, ldk;
-  long long spec_stride;
+  int nm, nk, ldk;
   const double *ue, *coef, *rec48, *prec;
-  const double *zoff, *ks, *Pzk;
-  double kstar;
-  double *p1h, *p2h;
+  SixOut out;
 };
 
 constexpr int FSX_CT = 512;   // consumer threads: one k each (16 warps keep the FP64 pipe fed through the Horner chains)
-
-#define HMV_SIX1(um, ue, cp)                                                          \
-  {                                                                                   \
-    const double2 c01 = (cp)[0], c23 = (cp)[1], c45 = (cp)[2], c67 = (cp)[3];         \
-    const double q1 = um * um, q2 = ue * ue, q3 = um * ue;                            \
-    acc[0] = fma(c01.x, q1, acc[0]);                                                  \
-    acc[1] = fma(c01.x, q2, acc[1]);                                                  \
-    acc[2] = fma(c01.x, q3, acc[2]);                                                  \
-    acc[3] = fma(c01.y, um, fma(c23.x, q1, acc[3]));                                  \
-    acc[4] = fma(c23.y, um, fma(c45.x, q1, acc[4]));                                  \
-    acc[5] = fma(c23.y, ue, fma(c45.x, q3, acc[5]));                                  \
-    acc[6] = fma(c45.y, um, acc[6]);                                                  \
-    acc[7] = fma(c45.y, ue, acc[7]);                                                  \
-    acc[8] = fma(c67.x, um, acc[8]);                                                  \
-  }
 
 // u_NFW of one wavenumber for two halo rows at once (two interleaved Horner chains).  The 32 adjacent wavenumbers of a
 // warp almost always share an interval, so the per-lane coefficient loads are shared-memory broadcasts; the loop runs
@@ -925,9 +813,7 @@ __device__ __forceinline__ void nfw_poly_pair(const NfwpTables& T, const double*
 __global__ void __launch_bounds__(FSX_CT + 32, 1) power_six_nfw_kernel(const FusedArgs a) {
   extern __shared__ __align__(128) unsigned char six_smem[];
   __shared__ NfwpTables T;
-  double* ring = reinterpret_cast<double*>(six_smem);
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)FSX_NST * FSX_STAGE_DOUBLES);
-  unsigned long long* empty = full + FSX_NST;
+  const BulkRing ring(six_smem, FSX_NST, FSX_STAGE_DOUBLES, FSX_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int z = blockIdx.x, k0 = (gridDim.y - 1 - blockIdx.y) * SIX_K;
   const int segk = min(SIX_K, a.ldk - k0);
@@ -935,49 +821,36 @@ __global__ void __launch_bounds__(FSX_CT + 32, 1) power_six_nfw_kernel(const Fus
   const int nit = (a.nm + SIX_R - 1) / SIX_R;
   const int k = k0 + tid;
   const bool active = tid < FSX_CT && k < a.nk;
-  const double kk = __ldg(a.ks + min(k, a.nk - 1));       // idle lanes evaluate a valid wavenumber and discard it
+  const double kk = __ldg(a.out.ks + min(k, a.nk - 1));   // idle lanes evaluate a valid wavenumber and discard it
   nfwp_tables_init(T, tid);
-  if (tid == 0) {
-    for (int s = 0; s < FSX_NST; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, FSX_CT / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   __syncthreads();
+  RingSlot slot;
 
   if (warp == FSX_CT / 32) {            // ---- producer warp ----
     if (lane == 0) {
       const unsigned segb = (unsigned)segk * 8u;
-      int s = 0;
-      unsigned ph = 0;
-      for (int it = 0; it < nit; ++it) {
-        mbar_wait_sleep(empty + s, ph ^ 1u);
+      for (int it = 0; it < nit; ++it, ring.advance(slot)) {
         const int m0 = it * SIX_R, rows = min(SIX_R, a.nm - m0);
-        double* st = ring + (size_t)s * FSX_STAGE_DOUBLES;
-        mbar_expect_tx(full + s, (unsigned)rows * (segb + 64u + FREC * 8u));
+        const RingStage st = ring.acquire<true>(slot, (unsigned)rows * (segb + 64u + FREC * 8u));
         for (int r = 0; r < rows; ++r) {
-          bulk_g2s(st + r * SIX_K, a.ue + (zrow + m0 + r) * (long long)a.ldk + k0, segb, full + s);
-          double* rr = st + SIX_R * SIX_K + SIX_R * 8 + r * FREC;
-          bulk_g2s(rr, a.prec + (zrow + m0 + r) * NFWP_REC, NFWP_REC * 8u, full + s);
-          bulk_g2s(rr + NFWP_REC, a.rec48 + (zrow + m0 + r) * NFW_NREC + 42, 48u, full + s);
+          bulk_g2s(st.p + r * SIX_K, a.ue + (zrow + m0 + r) * (long long)a.ldk + k0, segb, st.full);
+          double* rr = st.p + SIX_R * SIX_K + SIX_R * 8 + r * FREC;
+          bulk_g2s(rr, a.prec + (zrow + m0 + r) * NFWP_REC, NFWP_REC * 8u, st.full);
+          bulk_g2s(rr + NFWP_REC, a.rec48 + (zrow + m0 + r) * NFW_NREC + 42, 48u, st.full);
         }
-        bulk_g2s(st + SIX_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, full + s);
-        if (++s == FSX_NST) { s = 0; ph ^= 1u; }
+        bulk_g2s(st.p + SIX_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
       }
     }
     return;
   }
 
   // ---- consumers: thread owns wavenumber k over the whole mass axis ----
-  double acc[9];
-#pragma unroll
-  for (int q = 0; q < 9; ++q) acc[q] = 0.0;
-  int s = 0;
-  unsigned ph = 0;
-  const double* st = ring;
-  for (int it = 0, mleft = a.nm; it < nit; ++it, mleft -= SIX_R) {
+  double acc[9] = {};
+  for (int it = 0, mleft = a.nm; it < nit; ++it, mleft -= SIX_R, ring.advance(slot)) {
     const int rows = min(SIX_R, mleft);
+    const double* st = ring.wait(slot);
     const double* recs = st + SIX_R * SIX_K + SIX_R * 8;
-    const double2* cfs = reinterpret_cast<const double2*>(st + SIX_R * SIX_K);
-    mbar_wait(full + s, ph);
+    const double* cfs = st + SIX_R * SIX_K;
 #pragma unroll 1
     for (int r = 0; r < rows; r += 2) {
       const double* r0 = recs + r * FREC;
@@ -985,40 +858,22 @@ __global__ void __launch_bounds__(FSX_CT + 32, 1) power_six_nfw_kernel(const Fus
       const double* r1 = two ? r0 + FREC : r0;
       double um0, um1;
       nfw_poly_pair(T, r0, r1, kk, um0, um1);
-      const double ue0 = st[r * SIX_K + min(tid, segk - 1)];
-      HMV_SIX1(um0, ue0, cfs + r * 4)
-      if (two) {
-        const double ue1 = st[(r + 1) * SIX_K + min(tid, segk - 1)];
-        HMV_SIX1(um1, ue1, cfs + (r + 1) * 4)
-      }
+      six_fma(acc, six_coef(cfs + r * 8), um0, st[r * SIX_K + min(tid, segk - 1)]);
+      if (two) six_fma(acc, six_coef(cfs + (r + 1) * 8), um1, st[(r + 1) * SIX_K + min(tid, segk - 1)]);
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + s);
-    st += FSX_STAGE_DOUBLES;
-    if (++s == FSX_NST) { s = 0; ph ^= 1u; st = ring; }
+    ring.release(slot);
   }
   if (!active) return;
-  const long long S = a.spec_stride;
-  const double zo0 = a.zoff[2 * z], zo1 = a.zoff[2 * z + 1];
-  const long long o = (long long)z * a.nk + k;
-  if (a.p1h) {
-    const double r = kk / a.kstar, damp = 1.0 - exp(-r * r);          // hmvec.py:526
-#pragma unroll
-    for (int q = 0; q < 6; ++q) a.p1h[q * S + o] = acc[q] * damp;
-  }
-  if (a.p2h) {                                                         // hmvec.py:572
-    const double P = a.Pzk[o];
-    const double Lm = acc[6] + zo0, Le = acc[7] + zo0, Lg = acc[8] + zo1;
-    a.p2h[0 * S + o] = P * Lm * Lm; a.p2h[1 * S + o] = P * Le * Le; a.p2h[2 * S + o] = P * Lm * Le;
-    a.p2h[3 * S + o] = P * Lg * Lg; a.p2h[4 * S + o] = P * Lg * Lm; a.p2h[5 * S + o] = P * Lg * Le;
-  }
+  six_epilogue(a.out, z, a.nk, k, acc);
 }
-#undef HMV_SIX1
+
+static bool aligned16(const void* p) { return ((unsigned long long)p & 15ull) == 0; }
 
 static int tracer_args(const hmv_tracer* t, const char* which, TracerArgs* out) {
   HMV_REQUIRE(t != nullptr, "hmv_power: tracer %s is null", which);
   HMV_REQUIRE(t->kind >= 0 && t->kind <= 2, "hmv_power: tracer %s has unknown kind %d", which, t->kind);
   HMV_REQUIRE(t->us_d != nullptr, "hmv_power: tracer %s has no profile cube", which);
+  HMV_REQUIRE(aligned16(t->us_d) && aligned16(t->uc_d), "hmv_power: cubes must be 16-byte aligned (tracer %s)", which);
   if (t->kind == 1)
     HMV_REQUIRE(t->Nc_d && t->Ns_d && t->NcNs_d && t->NsNsm1_d && t->ngal_d, "hmv_power: hod tracer %s lacks occupation arrays", which);
   out->kind = t->kind; out->Nc = t->Nc_d; out->Ns = t->Ns_d; out->NcNs = t->NcNs_d; out->NsNsm1 = t->NsNsm1_d;
@@ -1026,12 +881,43 @@ static int tracer_args(const hmv_tracer* t, const char* which, TracerArgs* out) 
   return HMV_OK;
 }
 
+// lets `kernel` use `bytes` of dynamic shared memory
+template <class Kernel>
+static int smem_opt_in(Kernel kernel, const char* name, size_t bytes) {
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) return fail(HMV_E_CUDA, "%s smem opt-in (%zu B): %s", name, bytes, cudaGetErrorString(e));
+  return HMV_OK;
+}
+
+// The part the three six-spectra entry points share: the checks of the common arguments (after the caller's own, so
+// that a rejected call launches nothing), the spec_stride default and the coefficient prep.  `streamed` are the cubes
+// or tables the kernel reads with bulk copies: non-null and 16-byte aligned.  The prep writes ws[z][m][8] and zoff.
+static int six_setup(const char* fn, int nz, int nm, int nk, int ldk, std::initializer_list<const double*> streamed,
+                     const double* ms_d, const double* ks_d, const double* nzm_d, const double* bh_d,
+                     const double* Pzk_d, double rho_m0, double kstar, const double* Nc_d, const double* Ns_d,
+                     const double* NcNs_d, const double* NsNsm1_d, const double* ngal_d, double* ws_d, double* zoff,
+                     long long spec_stride, double* p1h_d, double* p2h_d, cudaStream_t st, SixOut& out) {
+  HMV_REQUIRE(nz > 0 && nm >= 2 && nk > 0 && ldk >= nk, "%s: bad sizes (nz=%d nm=%d nk=%d ldk=%d)", fn, nz, nm, nk, ldk);
+  HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && Nc_d && Ns_d && NcNs_d && NsNsm1_d && ngal_d && ws_d, "%s: null pointer", fn);
+  for (const double* p : streamed) HMV_REQUIRE(p != nullptr, "%s: null pointer", fn);
+  HMV_REQUIRE(p2h_d == nullptr || Pzk_d != nullptr, "%s: P2h requested without Pzk", fn);
+  bool al = (ldk & 1) == 0 && aligned16(ws_d);
+  for (const double* p : streamed) al = al && aligned16(p);
+  HMV_REQUIRE(al, "%s: cubes, tables and workspace must be 16-byte aligned with even ldk (bulk async copies)", fn);
+  HMV_REQUIRE(spec_stride == 0 || spec_stride >= (long long)nz * nk, "%s: spec_stride smaller than nz*nk", fn);
+  out.spec_stride = spec_stride ? spec_stride : (long long)nz * nk;
+  out.zoff = zoff; out.ks = ks_d; out.Pzk = Pzk_d; out.kstar = kstar; out.p1h = p1h_d; out.p2h = p2h_d;
+  power_six_prep_kernel<<<nz, 256, 0, st>>>(nm, ms_d, nzm_d, bh_d, rho_m0, Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, ws_d,
+                                            zoff);
+  return check_launch("power_six_prep_kernel");
+}
+
 }  // namespace hmv
 using namespace hmv;
 
 extern "C" long long hmv_power_ws_doubles(int nz, int nm) {
   if (nz <= 0 || nm <= 0) return 0;
-  return 8LL * nz * nm + 2LL * nz;   // hmv_power: 7 coefficient rows; hmv_power_six: [z][m][8] records; + zoff
+  return 8LL * nz * nm + 2LL * nz;   // [z][m][8] coefficient records + zoff[z][2]
 }
 
 extern "C" int hmv_power(int nz, int nm, int nk, int ldk, const double* ms_d, const double* ks_d,
@@ -1039,7 +925,7 @@ extern "C" int hmv_power(int nz, int nm, int nk, int ldk, const double* ms_d, co
                          const hmv_tracer* A, const hmv_tracer* B, double* ws_d, double* p1h_d, double* p2h_d,
                          void* stream) {
   HMV_REQUIRE(nz > 0 && nm >= 2 && nk > 0 && ldk >= nk, "hmv_power: bad sizes (nz=%d nm=%d nk=%d ldk=%d)", nz, nm, nk, ldk);
-  HMV_REQUIRE((ldk & 1) == 0 && ((unsigned long long)ws_d & 15ull) == 0,
+  HMV_REQUIRE((ldk & 1) == 0 && aligned16(ws_d),
               "hmv_power: ldk must be even and the workspace 16-byte aligned (bulk async copies); ldk=%d", ldk);
   HMV_REQUIRE(nz <= 65535, "hmv_power: nz=%d exceeds grid.y limit 65535", nz);
   HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && ws_d, "hmv_power: null pointer");
@@ -1072,22 +958,21 @@ extern "C" int hmv_power(int nz, int nm, int nk, int ldk, const double* ms_d, co
       return q.ncube++;
     };
     q.rusA = role(usA); q.rucA = role(ucA); q.rusB = role(usB); q.rucB = role(ucB);
-    for (int c = 0; c < q.ncube; ++c)
-      if ((unsigned long long)q.cube[c] & 15ull) return fail(HMV_E_ARG, "hmv_power: cubes must be 16-byte aligned");
     if (q.form == 0 && q.ncube == 1 && q.rusA == 0 && q.rusB == 0 && q.rucA < 0 && q.rucB < 0) {
       // one cube, no central-profile cube: the streamlined kernel (uc == 1 is folded into aA, aB)
-      cudaError_t e = cudaFuncSetAttribute(power_one_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ONE_SMEM);
-      if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_one_kernel smem opt-in (%zu B): %s", ONE_SMEM, cudaGetErrorString(e));
+      const size_t smem = BulkRing::smem_bytes(ONE_NST, ONE_STAGE_DOUBLES);
+      int r = smem_opt_in(power_one_kernel, "power_one_kernel", smem);
+      if (r) return r;
       dim3 grid(cdiv(ldk, ONE_K), nz);
-      power_one_kernel<<<grid, ONE_CT + 32, ONE_SMEM, st>>>(q);
+      power_one_kernel<<<grid, ONE_CT + 32, smem, st>>>(q);
       return check_launch("power_one_kernel");
     }
-    const size_t stage = ((size_t)q.ncube * PR_R * PR_K + PR_R * 8) * sizeof(double);
-    q.nst = (int)((200 * 1024) / stage);
+    const int stage_doubles = q.ncube * PR_R * PR_K + PR_R * 8;
+    q.nst = (int)((200 * 1024) / (stage_doubles * sizeof(double)));
     if (q.nst > 6) q.nst = 6;
-    const size_t smem = q.nst * stage + 2 * q.nst * sizeof(unsigned long long);
-    cudaError_t e = cudaFuncSetAttribute(power_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_pair_kernel smem opt-in (%zu B): %s", smem, cudaGetErrorString(e));
+    const size_t smem = BulkRing::smem_bytes(q.nst, stage_doubles);
+    int r = smem_opt_in(power_pair_kernel, "power_pair_kernel", smem);
+    if (r) return r;
     dim3 grid(cdiv(ldk, PR_K), nz);
     power_pair_kernel<<<grid, PR_CT + 32, smem, st>>>(q);
     return check_launch("power_pair_kernel");
@@ -1110,32 +995,20 @@ extern "C" int hmv_power_six(int nz, int nm, int nk, int ldk, const double* ms_d
                              double kstar, const double* um_d, const double* ue_d, const double* Nc_d,
                              const double* Ns_d, const double* NcNs_d, const double* NsNsm1_d, const double* ngal_d,
                              double* ws_d, long long spec_stride, double* p1h_d, double* p2h_d, void* stream) {
-  HMV_REQUIRE(nz > 0 && nm >= 2 && nk > 0 && ldk >= nk, "hmv_power_six: bad sizes");
-  HMV_REQUIRE((ldk & 1) == 0, "hmv_power_six: ldk must be even; got %d", ldk);
   HMV_REQUIRE(nz <= 65535, "hmv_power_six: nz=%d exceeds grid.y limit 65535", nz);
-  HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && um_d && ue_d && Nc_d && Ns_d && NcNs_d && NsNsm1_d && ngal_d && ws_d,
-              "hmv_power_six: null pointer");
-  HMV_REQUIRE(p2h_d == nullptr || Pzk_d != nullptr, "hmv_power_six: P2h requested without Pzk");
-  HMV_REQUIRE((ldk & 1) == 0 && (((unsigned long long)um_d | (unsigned long long)ue_d | (unsigned long long)ws_d) & 15ull) == 0,
-              "hmv_power_six: cubes and workspace must be 16-byte aligned with even ldk (bulk async copies)");
   cudaStream_t st = (cudaStream_t)stream;
-  const long long cs = (long long)nz * nm;
-  double* coef = ws_d;
-  double* zoff = ws_d + 8 * cs;
-  power_six_prep_kernel<<<nz, 256, 0, st>>>(nm, ms_d, nzm_d, bh_d, rho_m0, Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, coef,
-                                            zoff);
-  int rc = check_launch("power_six_prep_kernel");
-  if (rc) return rc;
   SixArgs a;
-  HMV_REQUIRE(spec_stride == 0 || spec_stride >= (long long)nz * nk, "hmv_power_six: spec_stride smaller than nz*nk");
-  a.spec_stride = spec_stride ? spec_stride : (long long)nz * nk;
-  a.nz = nz; a.nm = nm; a.nk = nk; a.ldk = ldk; a.um = um_d; a.ue = ue_d; a.coef = coef;
-  a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d; a.kstar = kstar; a.p1h = p1h_d; a.p2h = p2h_d;
-  cudaError_t e = cudaFuncSetAttribute(power_six_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SIX_SMEM);
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_six_kernel smem opt-in (%zu B): %s", SIX_SMEM, cudaGetErrorString(e));
+  int rc = six_setup("hmv_power_six", nz, nm, nk, ldk, {um_d, ue_d}, ms_d, ks_d, nzm_d, bh_d, Pzk_d, rho_m0, kstar,
+                     Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, ws_d, ws_d + 8LL * nz * nm, spec_stride, p1h_d, p2h_d, st,
+                     a.out);
+  if (rc) return rc;
+  a.nm = nm; a.nk = nk; a.ldk = ldk; a.um = um_d; a.ue = ue_d; a.coef = ws_d;
+  const size_t smem = BulkRing::smem_bytes(SIX_NST, SIX_STAGE_DOUBLES);
+  rc = smem_opt_in(power_six_kernel, "power_six_kernel", smem);
+  if (rc) return rc;
   a.tk = wave_tile(nz, ldk, SIX_K, 1);
   dim3 grid(cdiv(ldk, a.tk), nz);
-  power_six_kernel<<<grid, SIX_CT + 32, SIX_SMEM, st>>>(a);
+  power_six_kernel<<<grid, SIX_CT + 32, smem, st>>>(a);
   return check_launch("power_six_kernel");
 }
 
@@ -1149,32 +1022,22 @@ extern "C" int hmv_power_six_tab(int nz, int nm, int nk, int ldk, const double* 
                                  double kstar, const double* um_d, const double* etab_d, int nxs, const double* Nc_d,
                                  const double* Ns_d, const double* NcNs_d, const double* NsNsm1_d, const double* ngal_d,
                                  double* ws_d, long long spec_stride, double* p1h_d, double* p2h_d, void* stream) {
-  HMV_REQUIRE(nz > 0 && nm >= 2 && nk > 0 && ldk >= nk && nxs >= 4, "hmv_power_six_tab: bad sizes");
+  HMV_REQUIRE(nxs >= 4, "hmv_power_six_tab: bad sizes (nxs=%d)", nxs);
   HMV_REQUIRE(nz <= 65535, "hmv_power_six_tab: nz=%d exceeds grid.y limit 65535", nz);
-  HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && um_d && etab_d && Nc_d && Ns_d && NcNs_d && NsNsm1_d && ngal_d && ws_d,
-              "hmv_power_six_tab: null pointer");
-  HMV_REQUIRE(p2h_d == nullptr || Pzk_d != nullptr, "hmv_power_six_tab: P2h requested without Pzk");
-  HMV_REQUIRE((ldk & 1) == 0 && (((unsigned long long)um_d | (unsigned long long)etab_d | (unsigned long long)ws_d) & 15ull) == 0,
-              "hmv_power_six_tab: cube, tables and workspace must be 16-byte aligned with even ldk (bulk async copies)");
   cudaStream_t st = (cudaStream_t)stream;
-  const long long cs = (long long)nz * nm;
-  double* coef = ws_d;
-  double* zoff = ws_d + 8 * cs;
-  power_six_prep_kernel<<<nz, 256, 0, st>>>(nm, ms_d, nzm_d, bh_d, rho_m0, Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, coef,
-                                            zoff);
-  int rc = check_launch("power_six_prep_kernel");
-  if (rc) return rc;
   SixTabArgs a;
-  HMV_REQUIRE(spec_stride == 0 || spec_stride >= (long long)nz * nk, "hmv_power_six_tab: spec_stride smaller than nz*nk");
-  a.spec_stride = spec_stride ? spec_stride : (long long)nz * nk;
-  a.nz = nz; a.nm = nm; a.nk = nk; a.ldk = ldk; a.um = um_d; a.coef = coef; a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d;
-  a.kstar = kstar; a.p1h = p1h_d; a.p2h = p2h_d;
+  int rc = six_setup("hmv_power_six_tab", nz, nm, nk, ldk, {um_d, etab_d}, ms_d, ks_d, nzm_d, bh_d, Pzk_d, rho_m0,
+                     kstar, Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, ws_d, ws_d + 8LL * nz * nm, spec_stride, p1h_d,
+                     p2h_d, st, a.out);
+  if (rc) return rc;
+  a.nm = nm; a.nk = nk; a.ldk = ldk; a.um = um_d; a.coef = ws_d;
   a.JS = (int)hmv_profile_table_stride(nxs); a.J = nxs / 2; a.nmp = cdiv(nm, 16) * 16;
   a.tab = etab_d; a.tmeta = etab_d + (size_t)nz * a.nmp * (size_t)a.JS;
-  cudaError_t e = cudaFuncSetAttribute(power_six_tab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TAB_SMEM);
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_six_tab_kernel smem opt-in (%zu B): %s", TAB_SMEM, cudaGetErrorString(e));
+  const size_t smem = BulkRing::smem_bytes(TAB_NST, TAB_STAGE_DOUBLES);
+  rc = smem_opt_in(power_six_tab_kernel, "power_six_tab_kernel", smem);
+  if (rc) return rc;
   dim3 grid(cdiv(ldk, SIX_K), nz);
-  power_six_tab_kernel<<<grid, TAB_CT + 32, TAB_SMEM, st>>>(a);
+  power_six_tab_kernel<<<grid, TAB_CT + 32, smem, st>>>(a);
   return check_launch("power_six_tab_kernel");
 }
 
@@ -1186,8 +1049,10 @@ extern "C" int hmv_power_tab(int nz, int nm, int nk, const double* ms_d, const d
   HMV_REQUIRE(kind == 0 || kind == 2, "hmv_power_tab: kind must be 0 (matter profile) or 2 (pressure profile)");
   HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && tab_d && ws_d, "hmv_power_tab: null pointer");
   HMV_REQUIRE(p2h_d == nullptr || Pzk_d != nullptr, "hmv_power_tab: P2h requested without Pzk");
-  HMV_REQUIRE((((unsigned long long)tab_d | (unsigned long long)ws_d) & 15ull) == 0, "hmv_power_tab: tables and workspace must be 16-byte aligned");
+  HMV_REQUIRE(aligned16(tab_d) && aligned16(ws_d), "hmv_power_tab: tables and workspace must be 16-byte aligned");
   HMV_REQUIRE(nxs / 2 <= 4096 && nm < (1 << 19), "hmv_power_tab: nxs <= 8192 and nm < 2^19 (packed row ids)");
+  const size_t smem = (size_t)nm * (sizeof(double4) + sizeof(double2) + sizeof(int)) + 16;
+  if (smem > 200 * 1024) return fail(HMV_E_LIMIT, "hmv_power_tab: nm=%d needs %zu B of shared memory", nm, smem);
   cudaStream_t st = (cudaStream_t)stream;
   const long long cs = (long long)nz * nm;
   double* coef = ws_d;
@@ -1198,20 +1063,13 @@ extern "C" int hmv_power_tab(int nz, int nm, int nk, const double* ms_d, const d
   int rc = check_launch("power_prep_kernel");
   if (rc) return rc;
   OneTabArgs a;
-  a.nm = nm; a.nk = nk; a.coef = coef; a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d; a.kstar = kstar; a.p1h = p1h_d; a.p2h = p2h_d;
+  a.nm = nm; a.nk = nk; a.nz = nz; a.coef = coef; a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d; a.kstar = kstar;
+  a.p1h = p1h_d; a.p2h = p2h_d;
   a.JS = (int)hmv_profile_table_stride(nxs); a.J = nxs / 2; a.nmp = cdiv(nm, 16) * 16;
   a.tab = tab_d; a.tmeta = tab_d + (size_t)nz * a.nmp * (size_t)a.JS;
-  const size_t smem = (size_t)nm * (sizeof(double4) + sizeof(double2) + sizeof(int)) + 16;
-  if (smem > 200 * 1024) return fail(HMV_E_LIMIT, "hmv_power_tab: nm=%d needs %zu B of shared memory", nm, smem);
-  cudaError_t e = cudaFuncSetAttribute(power_one_tab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_one_tab_kernel smem opt-in (%zu B): %s", smem, cudaGetErrorString(e));
-#if HMV_OT_ORDER
-  dim3 grid((unsigned)nz * cdiv(nk, OT_K));
-  a.nz = nz;
-#else
-  dim3 grid(cdiv(nk, OT_K), nz);
-#endif
-  power_one_tab_kernel<<<grid, OT_T, smem, st>>>(a);
+  rc = smem_opt_in(power_one_tab_kernel, "power_one_tab_kernel", smem);
+  if (rc) return rc;
+  power_one_tab_kernel<<<(unsigned)nz * cdiv(nk, OT_K), OT_T, smem, st>>>(a);
   return check_launch("power_one_tab_kernel");
 }
 
@@ -1226,14 +1084,8 @@ extern "C" int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* 
                                  const double* ue_d, const double* Nc_d, const double* Ns_d, const double* NcNs_d,
                                  const double* NsNsm1_d, const double* ngal_d, double* ws_d, long long spec_stride,
                                  double* p1h_d, double* p2h_d, void* stream) {
-  HMV_REQUIRE(nz > 0 && nm >= 2 && nk > 0 && ldk >= nk, "hmv_power_six_nfw: bad sizes");
-  HMV_REQUIRE(nz <= 2147483647 && cdiv(ldk, SIX_K) <= 65535, "hmv_power_six_nfw: grid limit");
-  HMV_REQUIRE(zs_d && ms_d && ks_d && nzm_d && bh_d && cs_d && rvir_d && ue_d && Nc_d && Ns_d && NcNs_d && NsNsm1_d &&
-                  ngal_d && ws_d, "hmv_power_six_nfw: null pointer");
-  HMV_REQUIRE(p2h_d == nullptr || Pzk_d != nullptr, "hmv_power_six_nfw: P2h requested without Pzk");
-  HMV_REQUIRE((ldk & 1) == 0 && (((unsigned long long)ue_d | (unsigned long long)ws_d) & 15ull) == 0,
-              "hmv_power_six_nfw: cube and workspace must be 16-byte aligned with even ldk (bulk async copies)");
-  HMV_REQUIRE(spec_stride == 0 || spec_stride >= (long long)nz * nk, "hmv_power_six_nfw: spec_stride smaller than nz*nk");
+  HMV_REQUIRE(cdiv(ldk, SIX_K) <= 65535, "hmv_power_six_nfw: grid limit");
+  HMV_REQUIRE(zs_d && cs_d && rvir_d, "hmv_power_six_nfw: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   const long long cs = (long long)nz * nm;
   double* coef = ws_d;
@@ -1241,23 +1093,21 @@ extern "C" int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* 
   double* prec = rec48 + NFW_NREC * cs;
   double* zoff = prec + NFWP_REC * cs;
   double* kmax_dev = zoff + 2 * nz + ((2 * nz) & 1);
-  power_six_prep_kernel<<<nz, 256, 0, st>>>(nm, ms_d, nzm_d, bh_d, rho_m0, Nc_d, Ns_d, NcNs_d, NsNsm1_d, ngal_d, coef,
-                                            zoff);
-  int rc = check_launch("power_six_prep_kernel");
+  FusedArgs a;
+  int rc = six_setup("hmv_power_six_nfw", nz, nm, nk, ldk, {ue_d}, ms_d, ks_d, nzm_d, bh_d, Pzk_d, rho_m0, kstar, Nc_d,
+                     Ns_d, NcNs_d, NsNsm1_d, ngal_d, ws_d, zoff, spec_stride, p1h_d, p2h_d, st, a.out);
   if (rc) return rc;
   tile_range_kernel<<<1, 32, 0, st>>>(nk, nk, ks_d, kmax_dev);          // {min, max} of ks
   rc = check_launch("tile_range_kernel");
   if (rc) return rc;
   rc = nfw_poly_records(cs, nm, 1, kmax_dev + 1, zs_d, cs_d, rvir_d, rec48, prec, st);
   if (rc) return rc;
-  FusedArgs a;
-  a.nz = nz; a.nm = nm; a.nk = nk; a.ldk = ldk; a.spec_stride = spec_stride ? spec_stride : (long long)nz * nk;
-  a.ue = ue_d; a.coef = coef; a.rec48 = rec48; a.prec = prec; a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d; a.kstar = kstar;
-  a.p1h = p1h_d; a.p2h = p2h_d;
-  cudaError_t e = cudaFuncSetAttribute(power_six_nfw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FSX_SMEM);
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "power_six_nfw_kernel smem opt-in (%zu B): %s", FSX_SMEM, cudaGetErrorString(e));
+  a.nm = nm; a.nk = nk; a.ldk = ldk; a.ue = ue_d; a.coef = coef; a.rec48 = rec48; a.prec = prec;
+  const size_t smem = BulkRing::smem_bytes(FSX_NST, FSX_STAGE_DOUBLES);
+  rc = smem_opt_in(power_six_nfw_kernel, "power_six_nfw_kernel", smem);
+  if (rc) return rc;
   dim3 grid(nz, cdiv(ldk, SIX_K));
-  power_six_nfw_kernel<<<grid, FSX_CT + 32, FSX_SMEM, st>>>(a);
+  power_six_nfw_kernel<<<grid, FSX_CT + 32, smem, st>>>(a);
   return check_launch("power_six_nfw_kernel");
 }
 
@@ -1270,12 +1120,6 @@ extern "C" int hmv_debug_wave_tile(int nz, int ldk) {
 extern "C" int hmv_debug_tab_order(int nz, int nk, int* z_out, int* k0_out) {
   HMV_REQUIRE(nz > 0 && nk > 0 && z_out && k0_out, "hmv_debug_tab_order: bad arguments");
   const int T = cdiv(nk, OT_K);
-  for (int i = 0; i < nz * T; ++i) {
-#if HMV_OT_ORDER
-    ot_cta(i, nz, nk, z_out[i], k0_out[i]);
-#else
-    z_out[i] = i / T; k0_out[i] = (i % T) * OT_K;
-#endif
-  }
+  for (int i = 0; i < nz * T; ++i) ot_cta(i, nz, nk, z_out[i], k0_out[i]);
   return OT_K;
 }

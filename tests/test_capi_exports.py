@@ -3,7 +3,10 @@ import ctypes
 import os
 import re
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+HMV_E_ARG, HMV_E_LIMIT = -1, -3             # include/hmvec_b200.h
 
 
 def _declared():
@@ -31,6 +34,30 @@ def test_binding_covers_header_and_reports_errors():
     assert rc == -1 and "bad sizes" in capi.last_error()
     rc = capi.lib.hmv_hod(3, 10, None, None, None, None, 0, None, None, None, None, None, None, None, None, None)
     assert rc == -1 and "null pointer" in capi.last_error()
+
+
+def test_k5_rejects_before_any_launch():
+    """Every argument and limit check of the mass-integral entry points runs before their first launch: with valid-
+    looking dummy device pointers and no GPU, a rejected call returns its own error, never a CUDA one."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("dummy device pointers must never reach a launch on a GPU")
+    from hmvec_b200 import _capi as capi
+    L = capi.lib
+    ptr = [ctypes.c_void_p(0x10000 + 0x100 * i) for i in range(16)]     # non-null, 16-byte aligned, never dereferenced
+    nz, nm, nk, ldk = 2, 40, 30, 32
+    t = capi.Tracer()
+    t.kind = 0
+    t.us_d = 0x20008                                                     # misaligned cube
+    rc = L.hmv_power(nz, nm, nk, ldk, *ptr[:5], 1.0, 1.0, ctypes.byref(t), ctypes.byref(t), *ptr[5:8], None)
+    assert rc == HMV_E_ARG and "16-byte aligned" in capi.last_error()
+    rc = L.hmv_power_six(nz, nm, nk, ldk, *ptr[:5], 1.0, 1.0, *ptr[5:13], nz * nk - 1, *ptr[13:15], None)
+    assert rc == HMV_E_ARG and "hmv_power_six: spec_stride" in capi.last_error()
+    rc = L.hmv_power_six_tab(nz, nm, nk, ldk, *ptr[:5], 1.0, 1.0, *ptr[5:7], 64, *ptr[7:13], nz * nk - 1,
+                             *ptr[13:15], None)
+    assert rc == HMV_E_ARG and "hmv_power_six_tab: spec_stride" in capi.last_error()
+    rc = L.hmv_power_tab(nz, 4000, nk, *ptr[:5], 1.0, 1.0, 2, ptr[5], 64, *ptr[6:9], None)
+    assert rc == HMV_E_LIMIT and "shared memory" in capi.last_error()
 
 
 def test_no_cpu_fallback_in_product():

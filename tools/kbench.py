@@ -1,12 +1,14 @@
 #!/usr/bin/env python
-"""Kernel-level A/B bench on a z-slab of the LARGE grid: times hmv_profile_transform (K1), hmv_uk_nfw (K2) and
-hmv_power_six (K5) alone with CUDA events, for one or several builds of the library (same C ABI), and compares the
-cubes each build writes with those of the first one.
+"""Kernel-level A/B bench on a z-slab of the LARGE grid: times hmv_profile_transform (K1), hmv_uk_nfw (K2) and every
+K5 mass-integral entry point alone with CUDA events, for one or several builds of the library (same C ABI), and
+compares the cubes and spectra each build writes with those of the first one.
 
-    python tools/kbench.py --nz 25 --libs hmvec_b200/libhmvec_b200.so,gpurun_out/lib_v2.so [--reps 10] [--pres]
+    python tools/kbench.py --nz 25 --libs hmvec_b200/libhmvec_b200.so,variants/lib_v2.so [--reps 10]
+    python tools/kbench.py --kernels k5 --libs old,new,old,new      # variants/lib_old.so, ... (tools/build_variant.sh)
 
 Each build runs in its own process (HMV_LIB selects the library).  Run on a GPU box."""
 import argparse
+import ctypes as C
 import json
 import os
 import subprocess
@@ -44,15 +46,53 @@ def child(a):
         capi.check(L.hmv_uk_nfw(nz, nm, nk, ldk, ptr(d["zs"]), ptr(d["ks"]), g.kmax, ptr(d["cs"]), ptr(d["rvir"]),
                                 ptr(d["nfw_ws"]), ptr(g.um), st), "hmv_uk_nfw")
 
-    def k5():
-        capi.check(L.hmv_power_six(nz, nm, nk, ldk, ptr(d["ms"]), ptr(d["ks"]), ptr(d["nzm"]), ptr(d["bh"]),
-                                   ptr(d["Pzk"]), g.rho_m0, float(g.p['kstar_damping']), ptr(g.um), ptr(g.ue),
-                                   ptr(d["Nc"]), ptr(d["Ns"]), ptr(d["NcNs"]), ptr(d["NsNsm1"]), ptr(d["ngal"]),
-                                   ptr(d["pow_ws"]), nz * nk, ptr(g.p1), ptr(g.p2), st), "hmv_power_six")
+    # K5 on the same slab: hmv_power for mm / gg / me / ge runs power_one_kernel, and power_pair_kernel with one and
+    # with two cubes; hmv_power_tab reads the pipeline's pressure tables, hmv_power_six_tab electron tables made here
+    E = lambda *s: torch.empty(s, dtype=torch.float64, device="cuda")
+    ws, ws_nfw = E(int(L.hmv_power_ws_doubles(nz, nm))), E(int(L.hmv_power_six_nfw_ws_doubles(nz, nm)))
+    etab = torch.zeros(int(L.hmv_profile_table_doubles(nz, nm, g.nxs)), dtype=torch.float64, device="cuda")
+    tr_ws = E(int(L.hmv_profile_transform_ws_doubles(nz, nm, g.nxs)))
+    capi.check(L.hmv_profile_tables(nz, nm, nk, ptr(d["zs"]), ptr(d["ks"]), g.kmax, ptr(d["rs"]), ptr(d["cmax"]),
+                                    ptr(d["xc"]), ptr(d["alpha"]), ptr(d["expo"]), ptr(d["amp"]), ptr(d["oscale"]),
+                                    g.gamma, g.xmax, g.nxs, 1, ptr(tr_ws), ptr(etab), st), "hmv_profile_tables")
+    hod = [ptr(d[k]) for k in ("Nc", "Ns", "NcNs", "NsNsm1", "ngal")]
+
+    def tracer(kind, u):
+        t = capi.Tracer()
+        t.kind, t.us_d = kind, u.data_ptr()
+        if kind == 1:
+            t.Nc_d, t.Ns_d, t.NcNs_d, t.NsNsm1_d, t.ngal_d = (d[k].data_ptr() for k in ("Nc", "Ns", "NcNs", "NsNsm1", "ngal"))
+        return t
+
+    tm, te, tg = tracer(0, g.um), tracer(0, g.ue), tracer(1, g.um)
+    k5_out = {}
+
+    def spectra(name, n):
+        k5_out[name] = (E(n, nz, nk), E(n, nz, nk))
+        return [ptr(x) for x in k5_out[name]]
+
+    base = (ptr(d["ms"]), ptr(d["ks"]), ptr(d["nzm"]), ptr(d["bh"]), ptr(d["Pzk"]), g.rho_m0, float(g.p['kstar_damping']))
+    k5_calls = {
+        "k5_six": (L.hmv_power_six, (nz, nm, nk, ldk, *base, ptr(g.um), ptr(g.ue), *hod, ptr(ws), 0,
+                                     *spectra("k5_six", 6), st)),
+        "k5_six_tab": (L.hmv_power_six_tab, (nz, nm, nk, ldk, *base, ptr(g.um), ptr(etab), g.nxs, *hod, ptr(ws), 0,
+                                             *spectra("k5_six_tab", 6), st)),
+        "k5_six_nfw": (L.hmv_power_six_nfw, (nz, nm, nk, ldk, ptr(d["zs"]), *base, ptr(d["cs"]), ptr(d["rvir"]),
+                                             ptr(g.ue), *hod, ptr(ws_nfw), 0, *spectra("k5_six_nfw", 6), st)),
+        "k5_tab_yy": (L.hmv_power_tab, (nz, nm, nk, *base, 2, ptr(g.ytab), g.p_nxs, ptr(ws), *spectra("k5_tab_yy", 1),
+                                        st)),
+    }
+    for name, A, B in (("mm", tm, tm), ("gg", tg, tg), ("me", tm, te), ("ge", tg, te)):
+        k5_calls["k5_" + name] = (L.hmv_power, (nz, nm, nk, ldk, *base, C.byref(A), C.byref(B), ptr(ws),
+                                                *spectra("k5_" + name, 1), st))
+
+    def k5(name):
+        fn, args = k5_calls[name]
+        return lambda: capi.check(fn(*args), name)
 
     out = {"lib": os.environ.get("HMV_LIB", "default"), "nz": nz}
-    for name, fn in (("k1", k1), ("k2", k2), ("k5", k5)):
-        if name not in a.kernels:
+    for name, fn in [("k1", k1), ("k2", k2)] + [(name, k5(name)) for name in k5_calls]:
+        if name.split("_")[0] not in a.kernels:
             continue
         for _ in range(3):
             fn()
@@ -67,8 +107,11 @@ def child(a):
         out[name + "_min"] = float(np.min(ts))
     # samples of the cubes for the parity comparison between builds
     rows = slice(None, None, 37)
-    np.savez(a.dump, ue=g.ue[:, rows, :nk].cpu().numpy(), um=g.um[:, rows, :nk].cpu().numpy(),
-             p1=g.p1.cpu().numpy(), p2=g.p2.cpu().numpy())
+    dump = dict(ue=g.ue[:, rows, :nk].cpu().numpy(), um=g.um[:, rows, :nk].cpu().numpy())
+    for name, (p1, p2) in k5_out.items():
+        if name + "_ms" in out:
+            dump[name + "_p1"], dump[name + "_p2"] = p1.cpu().numpy(), p2.cpu().numpy()
+    np.savez(a.dump, **dump)
     print("KBENCH " + json.dumps(out), flush=True)
 
 
@@ -86,7 +129,8 @@ def main():
     a.kernels = a.kernels.split(",")
     if a.child:
         return child(a)
-    libs = [l for l in a.libs.split(",") if l] or [os.path.join(ROOT, "hmvec_b200", "libhmvec_b200.so")]
+    libs = [l if os.path.exists(l) else os.path.join(ROOT, "variants", "lib_%s.so" % l) for l in a.libs.split(",") if l]
+    libs = libs or [os.path.join(ROOT, "hmvec_b200", "libhmvec_b200.so")]
     ref = None
     for i, lib in enumerate(libs):
         env = dict(os.environ, HMV_LIB=os.path.abspath(lib))
@@ -100,15 +144,16 @@ def main():
             continue
         res = json.loads(line[0][7:])
         cur = dict(np.load(dump))
+        os.remove(dump)
         if ref is None:
             ref = cur
         else:
-            for k in ("ue", "um", "p1", "p2"):
+            for k in ref:
                 sc = np.max(np.abs(ref[k]))
                 res["dmax_" + k] = float(np.max(np.abs(cur[k] - ref[k])) / sc)
-            with np.errstate(all="ignore"):
-                for k in ("p1", "p2"):
-                    rel = np.abs(cur[k] - ref[k]) / np.abs(ref[k])
+                if k not in ("ue", "um"):
+                    with np.errstate(all="ignore"):
+                        rel = np.abs(cur[k] - ref[k]) / np.abs(ref[k])
                     res["rel_" + k] = float(np.nanmax(np.where(np.isfinite(rel), rel, 0.0)))
         print("KBENCH " + json.dumps(res), flush=True)
 
