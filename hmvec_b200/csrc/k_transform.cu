@@ -19,17 +19,11 @@
 // (0.74 wavefronts/cycle/SM: the 32 table addresses of a B fragment are effectively random, ~6 wavefronts per
 // fragment) -- ncu evidence in profiles/.
 //
-// Two launch plans (hmv_set_transform_mode):
-//   0 (default)  profile_transform_ws_kernel: ONE persistent kernel (second half of this file) -- two independent
-//                8-warp groups per SM, each evaluating + transforming 16 halos and then interpolating + storing their
-//                rows, so that one group's tensor-core phase overlaps the other's store phase.  The same kernel also
-//                runs the two phases as separate launches around a resident table array (hmv_profile_tables /
-//                hmv_profile_expand: consumers that only integrate over M read the tables and never need the cube);
-//   1            profile_transform_kernel: one CTA owns 8 halos and runs evaluation, sums and interpolation one after
-//                the other with the bin table in shared memory; because the number of bins a halo needs grows like
-//                M^(1/3) (10 ... N/2), CTAs are launched in four bin-count classes whose shared-memory footprints
-//                (33 / 49 / 82 / 176 KB) let the many small halos run several CTAs per SM.  N too large for 8 halos'
-//                bin tables in shared memory (> ~6400) falls back to a DFMA rotation recurrence.
+// One launch plan: profile_transform_ws_kernel, ONE persistent kernel -- two independent 8-warp groups per SM, each
+// evaluating + transforming 16 halos and then interpolating + storing their rows, so that one group's tensor-core phase
+// overlaps the other's store phase.  The same kernel also runs the two phases as separate launches around a resident
+// table array (hmv_profile_tables / hmv_profile_expand: consumers that only integrate over M read the tables and never
+// need the cube).  Every entry point reads ks, the workspace and the cube / tables with 16-byte accesses.
 #include <cstdlib>
 #include "common.cuh"
 #include "gnfw_eval.cuh"
@@ -37,7 +31,8 @@
 namespace hmv {
 
 struct TParams {
-  int nz, nm, nk, ldk, N, J, JS, nmg, do_mass_norm, jlo, jhi;
+  int nz, nm, nk, ldk, N, J, JS, nmg, do_mass_norm;
+  int jlo, jhi;           // unused; removing them shifts every later field's constant-bank offset in the kernel
   double gamma, dx, step, kt1, kmax;
   const double *zs, *ks, *rs, *cmax, *xc, *alpha, *expo, *amp, *outscale, *sintab, *rkt;
   const double* rho;      // user-supplied samples rho[z][m][n] = rho(x_n) (generic_profile_fft with any profile), or NULL
@@ -46,17 +41,15 @@ struct TParams {
   const double *ts_a1, *ts_tw, *ts_a2;   // fragment-ordered twiddle tables (global)
   const int* jn_cta;
   double* uk;
-  // table mode (persistent kernel only): the finished bin tables go to tab[z][nmp][JS] (nmp = nm rounded up to 16) with
+  // table mode: the finished bin tables go to tab[z][nmp][JS] (nmp = nm rounded up to 16) with
   // {k -> bin factor, u_1, bin count, 0} per halo in tmeta[z][nmp][4], instead of a per-CTA slot that is reused
   double *tab, *tmeta;
   int phases;             // bit 0: compute the tables, bit 1: interpolate + store the rows
 };
 
-// samples evaluated per chunk.  The two large bin-count classes hold 704 (every Battaglia/README halo has <= 690
-// samples inside its theta-cut, so one chunk = one evaluation phase and one seeding of the sine recurrences per
-// pass); longer profiles simply take more chunks.  The two small classes and the DFMA fallback use 256, which keeps
-// their shared-memory footprint at 3 CTAs per SM (measured: 704 was slower for them).
-constexpr int NCH_MMA = 704, NCH_ROT = 256;
+// samples evaluated per chunk: every Battaglia/README halo has <= 690 samples inside its theta-cut, so one chunk = one
+// evaluation phase and one seeding of the sine recurrences per item; longer profiles simply take more chunks.
+constexpr int NCH_MMA = 704;
 
 // {sin, cos}(2 pi m/N) for m < N: seeds of the tensor-core path (read with __ldg, 16 bytes per entry)
 __global__ void sine_table_kernel(int N, double2* __restrict__ tab, double kt1, double* __restrict__ rkt) {
@@ -84,7 +77,7 @@ __global__ void kmax_kernel(int nk, const double* __restrict__ ks, double* __res
   }
 }
 
-// bins needed by each CTA (group of HB halos): jn = floor(kmax * max_h(rs (1+z)) / kt_1) + 2, capped at N/2
+// bins needed by each item (group of HB halos): jn = floor(kmax * max_h(rs (1+z)) / kt_1) + 2, capped at N/2
 __global__ void bin_count_kernel(int nz, int nm, int nmg, int HB, int J, double kmax_host, double kt1,
                                  const double* __restrict__ zs, const double* __restrict__ rs,
                                  int* __restrict__ jn_cta, int* __restrict__ work_counter,
@@ -102,234 +95,15 @@ __global__ void bin_count_kernel(int nz, int nm, int nmg, int HB, int J, double 
   jn_cta[b] = (int)fmin((double)J, floor(kmax * amax / kt1) + 2.0);
 }
 
-// U[halo][bin] += sum_n gs[n][halo] sin(2 pi bin (n0+n)/N) on the tensor cores: D[8 halos][8 bins] += A[8][4] B[4][8]
-// per mma.sync m8n8k4.  Lane (kq = lane%4, nq = lane/4) supplies A = gs[sample nn+kq][halo nq] and, per tile t,
-// B = sin(phi_j (n0+nn+kq)) for bin j = jw + 8 t + nq, and owns D[halo nq][bins 2kq, 2kq+1] of every tile.
-template <int NT>
-__device__ __forceinline__ void accum_mma(const double2* __restrict__ tab, const double* __restrict__ gs,
-                                          double* __restrict__ Us, int JS, int N, int n0, int nlen, int jw, int jn,
-                                          int lane) {
-  constexpr int HB = 8;
-  const int kq = lane & 3, nq = lane >> 2;
-  double bc[NT], bp[NT], tc[NT], c[NT][2];
-#pragma unroll
-  for (int t = 0; t < NT; ++t) {
-    const int jj = jw + 8 * t + nq;
-    const unsigned j = (jj <= jn) ? (unsigned)jj : 0u;          // bin 0: sin == 0, contributes nothing
-    const unsigned ph = (j * (unsigned)(n0 + kq)) % (unsigned)N;  // j*n < 2^31 (checked on the host)
-    const unsigned st = (4u * j) % (unsigned)N;                   // phase advance per 4 samples
-    const unsigned pp = ph >= st ? ph - st : ph + (unsigned)N - st;
-    bc[t] = __ldg(tab + ph).x;
-    bp[t] = __ldg(tab + pp).x;
-    tc[t] = 2.0 * __ldg(tab + st).y;
-    c[t][0] = 0.0; c[t][1] = 0.0;
-  }
-  const double* ga = gs + kq * HB + nq;
-#pragma unroll 2
-  for (int nn = 0; nn < nlen; nn += 4) {
-    const double a = ga[nn * HB];
-#pragma unroll
-    for (int t = 0; t < NT; ++t) {
-      asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                   : "+d"(c[t][0]), "+d"(c[t][1]) : "d"(a), "d"(bc[t]));
-      const double bn = fma(tc[t], bc[t], -bp[t]);
-      bp[t] = bc[t];
-      bc[t] = bn;
-    }
-  }
-#pragma unroll
-  for (int t = 0; t < NT; ++t) {
-    const int b0 = jw + 8 * t + 2 * kq;
-    if (b0 <= jn) Us[(size_t)nq * JS + b0] += c[t][0];
-    if (b0 + 1 <= jn) Us[(size_t)nq * JS + b0 + 1] += c[t][1];
-  }
-}
-
-template <int HB, int TT, bool TABLE, int MAXNJ, int NCH>
-__global__ void __launch_bounds__(TT, (TABLE && TT == 256) ? (MAXNJ <= 4 ? 3 : 2) : 1) profile_transform_kernel(const TParams p) {
-  extern __shared__ double smem[];
-  double* Us = smem;                          // [HB][JS]
-  double* gs = Us + (size_t)HB * p.JS;        // [NCH][HB]
-  double* red = gs + NCH * HB;                // [32]
-  __shared__ double h_cmax[HB], h_lxc[HB], h_alpha[HB], h_expo[HB], h_amp[HB], h_a[HB], h_oscale[HB];
-  __shared__ double h_k1[HB], h_kJ[HB], h_inv[HB], h_u1[HB];
-  __shared__ int h_valid[HB];
-
-  const int tid = threadIdx.x;
-  const int jn = p.jn_cta[blockIdx.x];
-  if (jn <= p.jlo || jn > p.jhi) return;      // not this launch's bin-count class (uniform over the CTA)
-  const int z = blockIdx.x / p.nmg;
-  const int mg = p.nmg - 1 - (blockIdx.x - z * p.nmg);  // heavy (large-M, many-bin) groups are scheduled first
-  const int m0 = mg * HB;
-  const double opz = 1.0 + p.zs[z];
-
-  if (tid < HB) {
-    const int m = m0 + tid;
-    const bool ok = m < p.nm;
-    const long long r = (long long)z * p.nm + (ok ? m : p.nm - 1);
-    h_valid[tid] = ok;
-    h_cmax[tid] = ok ? p.cmax[r] : -1.0;
-    h_lxc[tid] = log(p.xc[r]);
-    h_alpha[tid] = p.alpha[r];
-    h_expo[tid] = p.expo[r];
-    h_amp[tid] = p.amp[r];
-    const double a = p.rs[r] * opz;           // kout_j = kt_j / rs / (1+z)      (fft.py:92)
-    h_a[tid] = a;
-    h_oscale[tid] = p.outscale ? p.outscale[r] : 1.0;
-    h_k1[tid] = p.kt1 / a;
-    h_inv[tid] = a / p.kt1;
-    h_kJ[tid] = ((double)p.J * p.kt1) / a;
-  }
-  __syncthreads();
-
-  // sample and bin bounds shared by the HB halos of this CTA
-  double cmx = -1.0;
-#pragma unroll
-  for (int h = 0; h < HB; ++h) cmx = fmax(cmx, h_cmax[h]);
-  const int nb = (cmx > 0.0) ? (int)fmin((double)p.N, floor(cmx / p.dx) + 2.0) : 0;
-
-  const double2* T = reinterpret_cast<const double2*>(p.sintab);
-  for (int h = 0; h < HB; ++h)
-    for (int j = tid; j <= jn + 1; j += TT) Us[(size_t)h * p.JS + j] = 0.0;
-  __syncthreads();
-
-  const double twoN = 2.0 / (double)p.N;
-  double msum[HB];
-#pragma unroll
-  for (int h = 0; h < HB; ++h) msum[h] = 0.0;
-
-  for (int n0 = 0; n0 < nb; n0 += NCH) {
-    {  // ---- evaluate x*y for the chunk's samples, all HB halos per sample (theta-cut: x <= cmax, fft.py:79-81);
-       //      samples up to the next multiple of 4 past the chunk's end are zero-filled for the 4-sample MMA steps
-      const int nfill = min(NCH, ((nb - n0) + 3) & ~3);
-      for (int sn = tid; sn < nfill; sn += TT) {
-        const int n = n0 + sn;
-        const double x = (double)(n + 1) * p.dx;
-        const double lx = log(x);
-        const double w = (n == 0 || n == p.N - 1) ? 0.5 * p.dx : p.dx;  // np.trapz weights on xs (fft.py:84)
-#pragma unroll
-        for (int h = 0; h < HB; ++h) {
-          double v = 0.0;
-          if (n < p.N && x <= h_cmax[h]) {
-            const double lt = lx - h_lxc[h];
-            // amp * t^gamma * (1+t^alpha)^(-expo)
-            const double rho = h_amp[h] * exp(p.gamma * lt - h_expo[h] * log1p(exp(h_alpha[h] * lt)));
-            v = x * rho;
-            msum[h] = fma(w * x, v, msum[h]);
-          }
-          gs[sn * HB + h] = v;
-        }
-      }
-    }
-    __syncthreads();
-    const int nlen = min(NCH, nb - n0);
-    if constexpr (TABLE) {
-      static_assert(!TABLE || HB == 8, "the tensor-core path contracts 8 halos per tile");
-      // bins 1..jn in tiles of 8; each pass gives every warp NT consecutive tiles (NT sized to what is left)
-      constexpr int NW = TT / 32;
-      const int warp = tid >> 5, lane = tid & 31;
-      const int ntile = (jn + 7) >> 3;
-      for (int t0 = 0; t0 < ntile;) {
-        const int per = (ntile - t0 + NW - 1) / NW;        // tiles each warp still has to take
-        // NT in {1,2,3,4,6,8}: the smallest allowed count >= per (capped by MAXNJ), so that the last pass is not
-        // padded to the next power of two
-        const int nt = per >= 7 ? 8 : per >= 5 ? 6 : per;
-        const int ntc = nt > MAXNJ ? MAXNJ : nt;
-        const int jw = 1 + 8 * (t0 + warp * ntc);
-        if (jw <= jn) {
-          switch (ntc) {
-            case 8: if constexpr (MAXNJ >= 8) accum_mma<8>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-            case 6: if constexpr (MAXNJ >= 8) accum_mma<6>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-            case 4: accum_mma<4>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-            case 3: accum_mma<3>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-            case 2: accum_mma<2>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-            default: accum_mma<1>(T, gs, Us, p.JS, p.N, n0, nlen, jw, jn, lane); break;
-          }
-        }
-        t0 += ntc * NW;
-      }
-    } else {
-      for (int j = tid + 1; j <= jn; j += TT) {
-        double s, c, S, C;
-        sincospi(twoN * (double)(((long long)j * n0) % p.N), &s, &c);  // exact phase of sample n0
-        sincospi(twoN * (double)j, &S, &C);
-        double acc[HB];
-#pragma unroll
-        for (int h = 0; h < HB; ++h) acc[h] = 0.0;
-        for (int nn = 0; nn < nlen; ++nn) {
-          const double* g = gs + nn * HB;
-#pragma unroll
-          for (int h = 0; h < HB; ++h) acc[h] = fma(g[h], s, acc[h]);
-          const double s2 = fma(s, C, c * S);
-          c = fma(c, C, -s * S);
-          s = s2;
-        }
-#pragma unroll
-        for (int h = 0; h < HB; ++h) Us[(size_t)h * p.JS + j] += acc[h];
-      }
-    }
-    __syncthreads();
-  }
-
-  // ---- mass norm (fft.py:83-87) and u_j = U_j / kt_j / mnorm (fft.py:91) ----
-  double scale[HB];
-#pragma unroll
-  for (int h = 0; h < HB; ++h) {
-    const double mn = p.do_mass_norm ? block_sum(msum[h], red) : 1.0;
-    scale[h] = p.step / mn * h_oscale[h];
-  }
-  for (int j = tid + 1; j <= jn; j += TT) {
-    const double ikt = 1.0 / ((double)j * p.kt1);
-#pragma unroll
-    for (int h = 0; h < HB; ++h) Us[(size_t)h * p.JS + j] *= scale[h] * ikt;
-  }
-  __syncthreads();
-  if (tid < HB) h_u1[tid] = Us[(size_t)tid * p.JS + 1];
-  __syncthreads();
-
-  // ---- interpolation onto the target ks (fft.py:102-107): hold u_1 below bin 1, zero above bin J ----
-  // t = k / kout_1 is the fractional bin index: t < 1 -> u_1 (np.interp's left=), t > J -> 0 (right=), else the
-  // two neighbouring bins.  Per-halo constants live in registers; the only shared-memory traffic is U[j], U[j+1].
-  double inv[HB], u1[HB];
-#pragma unroll
-  for (int h = 0; h < HB; ++h) { inv[h] = h_inv[h]; u1[h] = h_u1[h]; }
-  const int nvalid = min(HB, p.nm - m0);
-  const double tJ = (double)p.J;
-  double* out0 = p.uk + ((long long)z * p.nm + m0) * (long long)p.ldk;
-  for (int k = tid; k < p.nk; k += TT) {
-    const double kk = __ldg(p.ks + k);
-    double* o = out0 + k;
-#pragma unroll
-    for (int h = 0; h < HB; ++h) {
-      if (h < nvalid) {
-        const double t = kk * inv[h];
-        double v = u1[h];
-        if (t >= 1.0) {
-          if (t > tJ) {
-            v = 0.0;
-          } else {
-            const double* U = Us + (size_t)h * p.JS;
-            const int j = min(min((int)t, p.J - 1), jn);   // <= jn: stays inside the bins this CTA computed
-            const double u0 = U[j];
-            v = fma(t - (double)j, U[j + 1] - u0, u0);
-          }
-        }
-        o[(long long)h * p.ldk] = v;
-      }
-    }
-  }
-}
-
-
 // =====================================================================================================================
-// Warp-specialised persistent form of the same transform (the default path).
+// The persistent, warp-specialised transform kernel.
 //
-// The class kernels above run their three phases -- GNFW evaluation, tensor-core sine sums, interpolation + store --
-// one after the other inside a CTA, and the heavy classes fit one CTA per SM, so the FP64 pipe idles while the rows are
-// stored and the store path idles while the pipe works (ncu: 48 % tensor-pipe active, 8 % DRAM in the heaviest class).
-// Here ONE 512-thread CTA per SM holds TWO independent groups of 8 warps, each with its own 90 KB sample buffer and its
-// own bin table in global memory (only the bins an item needs are touched, so the tables live in the 126 MB L2).  A
-// group pulls (z, 16-halo group) items from a global atomic queue and runs, for each item,
+// Why two groups: an earlier design ran evaluation, sine sums and stores one after the other in one CTA per SM, and the
+// FP64 pipe idled while rows were stored and the store path idled while the pipe worked (ncu: 48 % tensor-pipe active,
+// 8 % DRAM on its heaviest halos).  ONE 512-thread CTA per SM holds TWO independent groups of 8 warps, each with its
+// own 90 KB sample buffer and its own bin table in global memory (only the bins an item needs are touched, so the
+// tables live in the 126 MB L2).  A group pulls (z, 16-halo group) items from a global atomic queue and runs, for
+// each item,
 //   phase 1: evaluate the samples into its buffer, run the DMMA sine sums, write the normalised bin table u_j;
 //   phase 2: interpolate the 16 rows onto the target ks and store them.  A warp owns 256-wide k blocks and walks the 16
 //            rows of the item for each block: the wavenumbers stay in registers for all rows (no shared-memory copy of
@@ -347,9 +121,6 @@ __global__ void __launch_bounds__(TT, (TABLE && TT == 256) ? (MAXNJ <= 4 ? 3 : 2
 // (DMMA-bound) groups alternate in every SM's queue instead of arriving as one heavy and one light phase; the last
 // redshifts behind a short mixed head (see ws_item, launch_transform_ws) run jointly heavy-first so the queue drains on light items.
 // The parameters of the next item are fetched into registers while the current one is being transformed.
-#ifndef HMV_K1_ABL
-#define HMV_K1_ABL 0       // measurement builds only, bit mask: 1 skip the sample evaluation, 2 skip the sine sums,
-#endif                     // 4 consumers skip the rows, 8 consumers store every block as a fill, 64 constant blocks are not stored
 constexpr int WS_HB = 16, WS_NG = 2, WS_GT = 256, WS_MAXCTA = 192;
 constexpr int WS_GS_DOUBLES = (NCH_MMA / 4) * 64;      // one sample buffer: 16 halos x NCH_MMA samples
 // sum over the lanes of the caller's parity (even lanes hold halos 0-7, odd lanes halos 8-15)
@@ -677,26 +448,6 @@ __device__ __forceinline__ void accum_two_stage(const TParams& p, const double* 
   }
 }
 
-#ifndef HMV_K1_STORE
-#define HMV_K1_STORE 0
-#endif
-__device__ __forceinline__ void ws_store(double2* p, double2 v) {
-#if HMV_K1_STORE == 0
-  __stcs(p, v);
-#elif HMV_K1_STORE == 1
-  *p = v;
-#elif HMV_K1_STORE == 2
-  __stwt(p, v);
-#else
-  __stcg(p, v);
-#endif
-}
-#if HMV_K1_ABL & 16
-#define WS_NU 1
-#else
-#define WS_NU 4
-#endif
-
 struct WsGroupShared {                        // per group
   double h_cmax[WS_HB], h_lxc[WS_HB], h_alpha[WS_HB], h_expo[WS_HB], h_amp[WS_HB], h_oscale[WS_HB], h_inv[WS_HB];
   double u1[WS_HB];                           // bin 1 of the finished table (np.interp's left value)
@@ -794,17 +545,13 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
     const int ts_k = (((nb + TS_P - 1) / TS_P) + 3) >> 2;                       // stage-1 k-steps: n1 < 4 ts_k
     const int ts_r = p.ts_Q > 0 ? ((jn / p.ts_Q + 1) + 7) >> 3 : 0;             // j1 tiles
     bool two = false;
-#if !(HMV_K1_ABL & 32)
     if (single && p.ts_Q > 0 && ts_k <= TS_S && ts_r <= TS_RMAX) {
       const long long direct = 2LL * ((nb + 3) >> 2) * ((jn + 7) >> 3);
       const long long staged = (long long)WS_HB * p.ts_QT * (2 * TS_U * ts_k + 4 * TS_U * ts_r);
-#ifndef HMV_K1_TS_NUM
-#define HMV_K1_TS_NUM 5
-#define HMV_K1_TS_DEN 4
-#endif
-      two = HMV_K1_TS_NUM * staged < HMV_K1_TS_DEN * direct;
+      // a 5/4 margin, because the two-stage form also pays for slice staging, twiddles and group barriers; 5/4
+      // measured best among the thresholds tried
+      two = 5 * staged < 4 * direct;
     }
-#endif
 
     double msum[8];                          // this lane's half of the halos (hoff ...)
 #pragma unroll
@@ -815,7 +562,6 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
       const int nfill = min(NCH_MMA, ((nb - n0) + 3) & ~3);
       // thread pair (2i, 2i+1) shares a sample: even lanes evaluate halos 0-7, odd lanes halos 8-15, the eight
       // chains of a thread in lock-step (gnfw_eval.cuh); samples outside a halo's theta-cut are masked afterwards
-#if !(HMV_K1_ABL & 1)
       if (p.rho) {
         // samples supplied by the caller (rhofunc_x evaluated elsewhere, fft.py:76-81): x * rho(x) inside the cut
         for (int sn = gt >> 1; sn < nfill; sn += WS_GT / 2) {
@@ -858,9 +604,6 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
           gs[two ? h * NCH_MMA + sn : ws_gs_index(sn, h)] = v;
         }
       }
-#else
-      msum[0] = 1.0;
-#endif
       if (single && p.do_mass_norm) {
 #pragma unroll
         for (int h = 0; h < 8; ++h) {
@@ -880,7 +623,6 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
         scale0 = p.step / mn0 * G.h_oscale[nq];
         scale1 = p.step / mn1 * G.h_oscale[nq + 8];
       }
-#if !(HMV_K1_ABL & 2)
       const int nlen = min(NCH_MMA, nb - n0);
       constexpr int NW = WS_GT / 32;
       const int ntile = (jn + 7) >> 3;
@@ -919,9 +661,6 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
       }
       }
 #undef HMV_WS_ACC
-#else
-      if (gt < WS_HB) G.u1[gt] = scale0;
-#endif
       group_bar(g);                          // the chunk's samples are consumed, its sums are in the table
     }
 
@@ -964,7 +703,6 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
     // enough of those in flight (ncu: long_scoreboard was the top stall of this phase).  k blocks are handed out
     // through a counter in shared memory, starting at the first block that is not a pure hold-u_1 fill: the expensive
     // (interpolated) blocks go first and the group's warps finish within one cheap fill block of each other.
-#if !(HMV_K1_ABL & 4)
     if (p.phases & 2) {
       const int nvalid = min(WS_HB, p.nm - m0);
       double* out0 = p.uk + ((long long)z * p.nm + m0) * (long long)p.ldk;
@@ -1025,21 +763,16 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
           const double tf = kf * inv_r, tl = kl * inv_r;
           cls = (tl < 1.0) ? 0 : (tf > tJ) ? 1 : (tf >= 1.0 && tl <= tJ) ? 2 : 3;
         }
-#if HMV_K1_ABL & 8
-        cls = 0;
-#endif
         for (int row = r0; row < r1; ++row) {
           const int c = __shfl_sync(0xffffffffu, cls, row);
           double2* orow = reinterpret_cast<double2*>(out0 + (long long)row * p.ldk) + base + lane;
           const double* Uh = tabbase + (size_t)(row - r0) * tabstride;
           if (c < 2) {
-#if !(HMV_K1_ABL & 64)                       // ablation 64: constant blocks are not stored (timing only)
             const double fv = c ? 0.0 : G.u1[row];
             const double2 v = make_double2(fv, fv);
 #pragma unroll
-            for (int u = 0; u < WS_NU; ++u)
-              if (whole || base + lane + 32 * u < npair) ws_store(orow + 32 * u, v);
-#endif
+            for (int u = 0; u < 4; ++u)
+              if (whole || base + lane + 32 * u < npair) __stcs(orow + 32 * u, v);
           } else if (c == 2) {
             const double inv = G.h_inv[row];
             unsigned jc[8], jo[8];
@@ -1057,8 +790,8 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
             }
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-              ws_store(orow + 32 * u, make_double2(fma(af[2 * u], uo[2 * u] - ua[2 * u], ua[2 * u]),
-                                                  fma(af[2 * u + 1], uo[2 * u + 1] - ua[2 * u + 1], ua[2 * u + 1])));
+              __stcs(orow + 32 * u, make_double2(fma(af[2 * u], uo[2 * u] - ua[2 * u], ua[2 * u]),
+                                                fma(af[2 * u + 1], uo[2 * u + 1] - ua[2 * u + 1], ua[2 * u + 1])));
           } else {
             const double inv = G.h_inv[row], u1 = G.u1[row];
             WsLerp e[8];
@@ -1077,7 +810,7 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
             for (int u = 0; u < 4; ++u) {
               const double2 v = make_double2(ws_lerp_finish(e[2 * u], ua[2 * u], uo[2 * u], u1),
                                              ws_lerp_finish(e[2 * u + 1], ua[2 * u + 1], uo[2 * u + 1], u1));
-              if (whole || base + lane + 32 * u < npair) ws_store(orow + 32 * u, v);
+              if (whole || base + lane + 32 * u < npair) __stcs(orow + 32 * u, v);
             }
           }
         }
@@ -1090,20 +823,37 @@ profile_transform_ws_kernel(const TParams p, double* ring, int* work_counter, in
         }
       }
     }
-#endif
     group_bar(g);                            // every warp is done with the table, u1 and this item's h_*
     publish();                               // next item's parameters (ordered by the next trip's first barrier)
     item = nxt;
   }
 }
 
-// row stride of the persistent kernel's bin tables: bins 0 .. J+1, rounded up to whole 16-byte words
+// row stride of the bin tables: bins 0 .. J+1, rounded up to whole 16-byte words
 static int ws_js(int nxs) { return (nxs / 2 + 3) & ~1; }
-static bool ws_ring_fits(int nxs) {
-  return (size_t)WS_MAXCTA * WS_NG * WS_HB * (size_t)ws_js(nxs) * sizeof(double) <= ((size_t)8 << 30);   // only the bins a group needs are ever touched; covers every N the phase index allows (N < 65536)
-}
 
-static int g_transform_mode = 0;   // 0: warp-specialised persistent kernel; 1: bin-count-class kernels
+// two-stage form available: N divisible by TS_P (tables: QT q tiles)
+static int ts_qtiles(int nxs) { return (nxs % TS_P == 0 && nxs / TS_P >= 16) ? (nxs / TS_P + 7) / 8 : 0; }
+
+// Workspace of the transform, as offsets in doubles from ws_d (16-byte aligned): the {sin,cos} table, the bin count of
+// every (z, 16-halo item) as ints, the queue head (int) + the device max(ks), 1/kt_j for j <= J+1, one [16][JS] bin
+// table per group of the persistent kernel, the two-stage tables.  The bin tables and the two-stage tables are read as
+// double2, so they start on even offsets.
+struct K1Ws {
+  size_t jn, head, rkt, ring, ts, total;
+};
+static K1Ws k1_ws_layout(int nz, int nm, int nxs) {
+  auto even = [](size_t n) { return (n + 1) & ~(size_t)1; };
+  const int QT = ts_qtiles(nxs);
+  K1Ws w;
+  w.jn = 2 * (size_t)nxs;
+  w.head = w.jn + ((size_t)nz * cdiv(nm, WS_HB) + 1) / 2;
+  w.rkt = w.head + 2;
+  w.ring = even(w.rkt + nxs / 2 + 2);
+  w.ts = even(w.ring + (size_t)WS_MAXCTA * WS_NG * WS_HB * ws_js(nxs));
+  w.total = w.ts + (QT ? (size_t)QT * TS_SLICE + TS_A2_DOUBLES : 0);
+  return w;
+}
 
 // stride through the mass groups with a step near nmg/phi^2 that is coprime to nmg (a permutation of 0..nmg-1)
 static int ws_stride(int nmg) {
@@ -1136,62 +886,30 @@ static int launch_transform_ws(const TParams& p, double* ring, int* counter, cud
   cudaError_t e = cudaGetDevice(&dev);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
   if (e != cudaSuccess) return fail(HMV_E_CUDA, "profile_transform: %s", cudaGetErrorString(e));
-  TParams q = p;
-  q.nmg = cdiv(p.nm, WS_HB);
-  q.jlo = 0; q.jhi = p.J; q.JS = ws_js(p.N);
-  const int nitems = q.nz * q.nmg;
+  const int nitems = p.nz * p.nmg;
   const int grid = nitems < nsm ? nitems : (nsm < WS_MAXCTA ? nsm : WS_MAXCTA);
-  const int stride = ws_stride(q.nmg);
+  const int stride = ws_stride(p.nmg);
   size_t smem = (size_t)WS_NG * WS_GS_DOUBLES * sizeof(double);
-  if (q.ts_Q > 0) smem += (size_t)(TS_A2_DOUBLES + WS_NG * TS_SLICE) * sizeof(double);
+  if (p.ts_Q > 0) smem += (size_t)(TS_A2_DOUBLES + WS_NG * TS_SLICE) * sizeof(double);
   e = cudaFuncSetAttribute(profile_transform_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return fail(HMV_E_CUDA, "profile_transform smem opt-in (%zu B): %s", smem, cudaGetErrorString(e));
-  const int ntail = ws_tail(q.nz, q.nmg, grid);
-  profile_transform_ws_kernel<<<grid, WS_NG * WS_GT, smem, st>>>(q, ring, counter, nitems, stride, ntail);
+  const int ntail = ws_tail(p.nz, p.nmg, grid);
+  profile_transform_ws_kernel<<<grid, WS_NG * WS_GT, smem, st>>>(p, ring, counter, nitems, stride, ntail);
   return check_launch("profile_transform_ws_kernel");
-}
-
-template <int HB, int NCH>
-static size_t transform_smem(int JS) {
-  return ((size_t)HB * JS + (size_t)NCH * HB + 32) * sizeof(double);
-}
-
-template <int HB, int TT, bool TABLE, int MAXNJ, int NCH>
-static int launch_transform(const TParams& p, int jlo, int jhi, int JS, cudaStream_t st) {
-  const size_t smem = transform_smem<HB, NCH>(JS);
-  auto kern = profile_transform_kernel<HB, TT, TABLE, MAXNJ, NCH>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "profile_transform smem opt-in (%zu B): %s", smem, cudaGetErrorString(e));
-  TParams q = p;
-  q.nmg = cdiv(p.nm, HB);
-  q.jlo = jlo; q.jhi = jhi; q.JS = JS;
-  kern<<<q.nz * q.nmg, TT, smem, st>>>(q);
-  return check_launch("profile_transform_kernel");
 }
 
 }  // namespace hmv
 using namespace hmv;
 
-// two-stage form available: N divisible by TS_P (tables: QT q tiles)
-static int ts_qtiles(int nxs) { return (nxs % TS_P == 0 && nxs / TS_P >= 16) ? (nxs / TS_P + 7) / 8 : 0; }
-static long long ts_table_doubles(int nxs) {
-  const int QT = ts_qtiles(nxs);
-  return QT ? 2 + (long long)QT * (TS_A1_SLICE + TS_TW_SLICE) + TS_A2_DOUBLES : 0;
-}
-
 extern "C" long long hmv_profile_transform_ws_doubles(int nz, int nm, int nxs) {
   if (nz <= 0 || nm <= 0 || nxs <= 0) return 0;
-  // {sin,cos} table (2 doubles per phase) + one int per CTA (bin counts; a CTA holds at least one halo)
-  long long n = 2LL * nxs + 2 + ((long long)nz * nm + 1) / 2 + 2 + 2 + (nxs / 2 + 2);   // ..., queue head, 1/kt_j
-  if (ws_ring_fits(nxs)) n += 1 + (long long)WS_MAXCTA * WS_NG * WS_HB * ws_js(nxs) + ts_table_doubles(nxs);   // bin tables of the persistent kernel + two-stage twiddles
-  return n;
+  return (long long)k1_ws_layout(nz, nm, nxs).total;
 }
 
+// Kept for ABI stability: 0 selects the persistent kernel, the one launch plan there is.
 extern "C" int hmv_set_transform_mode(int mode) {
-  HMV_REQUIRE(mode == 0 || mode == 1, "hmv_set_transform_mode: mode must be 0 (persistent) or 1 (bin-count classes)");
-  g_transform_mode = mode;
+  HMV_REQUIRE(mode == 0, "hmv_set_transform_mode: mode %d does not exist; 0 is the only launch plan (the "
+              "bin-count-class plan, mode 1, was removed)", mode);
   return HMV_OK;
 }
 
@@ -1207,8 +925,12 @@ static int profile_transform_impl(int nz, int nm, int nk, int ldk, const double*
   HMV_REQUIRE(zs_d && ks_d && rs_d && ws_d && ((phases & 2) == 0 || uk_d) &&
               ((phases & 1) == 0 || (cmax_d && (rho_d || (xc_d && alpha_d && expo_d && amp_d)))),
               "hmv_profile_transform: null pointer");
-  TParams p;
-  p.nz = nz; p.nm = nm; p.nk = nk; p.ldk = ldk; p.N = nxs; p.J = nxs / 2; p.JS = p.J + 2;
+  HMV_REQUIRE((((size_t)ks_d | (size_t)ws_d | (size_t)uk_d | (size_t)tab_d) & 15) == 0 && (ldk & 1) == 0,
+              "hmv_profile_transform: ks, ws, uk and tab must be 16-byte aligned with even ldk (16-byte loads and "
+              "stores); ldk=%d", ldk);
+  const K1Ws w = k1_ws_layout(nz, nm, nxs);
+  TParams p = {};                              // jlo, jhi stay 0
+  p.nz = nz; p.nm = nm; p.nk = nk; p.ldk = ldk; p.N = nxs; p.J = nxs / 2; p.JS = ws_js(nxs); p.nmg = cdiv(nm, WS_HB);
   p.do_mass_norm = do_mass_norm;
   p.gamma = gamma;
   p.dx = xmax / nxs;                           // xs = linspace(0,xmax,nxs+1)[1:]           (fft.py:73)
@@ -1216,90 +938,36 @@ static int profile_transform_impl(int nz, int nm, int nk, int ldk, const double*
   p.kt1 = (1.0 * (1.0 / (nxs * p.step))) * 2.0 * M_PI;  // rfftfreq(N,step)[1]*2pi          (fft.py:50)
   p.kmax = kmax;
   p.zs = zs_d; p.ks = ks_d; p.rs = rs_d; p.cmax = cmax_d; p.xc = xc_d; p.alpha = alpha_d; p.expo = expo_d;
-  p.amp = amp_d; p.outscale = outscale_d; p.uk = uk_d; p.nmg = 0; p.sintab = ws_d; p.jlo = 0; p.jhi = p.J;
+  p.amp = amp_d; p.outscale = outscale_d; p.uk = uk_d; p.sintab = ws_d;
   p.rho = rho_d;
   p.tab = tab_d; p.phases = phases;
-  p.tmeta = tab_d ? tab_d + (size_t)nz * (size_t)(cdiv(nm, WS_HB) * WS_HB) * (size_t)ws_js(nxs) : nullptr;
-  int* jn_cta = reinterpret_cast<int*>(ws_d + 2 * (size_t)nxs + 2);
+  p.tmeta = tab_d ? tab_d + (size_t)nz * (size_t)(p.nmg * WS_HB) * (size_t)p.JS : nullptr;
+  int* jn_cta = reinterpret_cast<int*>(ws_d + w.jn);
   p.jn_cta = jn_cta;
-  double* after_jn = ws_d + 2 * (size_t)nxs + 2 + ((size_t)nz * nm + 1) / 2 + 2;
-  int* counter = reinterpret_cast<int*>(after_jn);
-  double* rkt = after_jn + 2;
-  double* ring = rkt + (nxs / 2 + 2);
-  ring += ((size_t)(ring - ws_d) & 1);                  // 16-byte aligned rows (ws_d is): phase 2 copies them as double2
-  p.rkt = rkt;
-  p.ts_Q = 0; p.ts_QT = 0; p.ts_a1 = p.ts_tw = p.ts_a2 = nullptr;
+  int* counter = reinterpret_cast<int*>(ws_d + w.head);
+  double* kmax_dev = ws_d + w.head + 1;
+  p.rkt = ws_d + w.rkt;
   cudaStream_t st = (cudaStream_t)stream;
-  auto bin_counts = [&](int HB) {
-    const int nmg = cdiv(nm, HB);
-    double* kmax_dev = reinterpret_cast<double*>(counter) + 1;       // second double of the queue-head slot
-    kmax_kernel<<<1, 1024, 0, st>>>(nk, ks_d, kmax_dev);
-    bin_count_kernel<<<cdiv((long long)nz * nmg, 256), 256, 0, st>>>(nz, nm, nmg, HB, p.J, kmax, p.kt1, zs_d, rs_d, jn_cta,
-                                                                     counter, kmax_dev);
-    return check_launch("bin_count_kernel");
-  };
-  const bool aligned16 = (((size_t)ks_d | (size_t)uk_d | (size_t)ws_d | (size_t)tab_d) & 15) == 0 && (ldk & 1) == 0;
-  if (tab_d && !(ws_ring_fits(nxs) && aligned16))
-    return fail(HMV_E_LIMIT, "hmv_profile_tables/expand: need 16-byte aligned ks/uk/ws/tab, even ldk and nxs < 65536");
-  if ((g_transform_mode == 0 || tab_d) && ws_ring_fits(nxs) && aligned16) {
-    // persistent warp-specialised kernel: sine table, bin counts, one launch
-    sine_table_kernel<<<cdiv(nxs, 256), 256, 0, st>>>(nxs, reinterpret_cast<double2*>(ws_d), p.kt1, rkt);
-    int rc = check_launch("sine_table_kernel");
+  sine_table_kernel<<<cdiv(nxs, 256), 256, 0, st>>>(nxs, reinterpret_cast<double2*>(ws_d), p.kt1, ws_d + w.rkt);
+  int rc = check_launch("sine_table_kernel");
+  if (rc) return rc;
+  kmax_kernel<<<1, 1024, 0, st>>>(nk, ks_d, kmax_dev);
+  bin_count_kernel<<<cdiv((long long)nz * p.nmg, 256), 256, 0, st>>>(nz, nm, p.nmg, WS_HB, p.J, kmax, p.kt1, zs_d, rs_d,
+                                                                       jn_cta, counter, kmax_dev);
+  rc = check_launch("bin_count_kernel");
+  if (rc) return rc;
+  const int QT = ts_qtiles(nxs);
+  if (QT) {
+    double* tabs = ws_d + w.ts;
+    p.ts_Q = nxs / TS_P; p.ts_QT = QT;
+    p.ts_a1 = tabs; p.ts_tw = tabs + (size_t)QT * TS_A1_SLICE; p.ts_a2 = tabs + (size_t)QT * (TS_A1_SLICE + TS_TW_SLICE);
+    const int nthr = QT * TS_U * 2 * 32 > TS_A2_DOUBLES ? QT * TS_U * 2 * 32 : TS_A2_DOUBLES;
+    twostage_tables_kernel<<<cdiv(nthr, 256), 256, 0, st>>>(nxs, p.ts_Q, QT, tabs, tabs + (size_t)QT * TS_A1_SLICE,
+                                                           tabs + (size_t)QT * (TS_A1_SLICE + TS_TW_SLICE));
+    rc = check_launch("twostage_tables_kernel");
     if (rc) return rc;
-    rc = bin_counts(WS_HB);
-    if (rc) return rc;
-    const int QT = ts_qtiles(nxs);
-    if (QT) {
-      double* tabs = ring + (size_t)WS_MAXCTA * WS_NG * WS_HB * (size_t)ws_js(nxs);
-      tabs += ((size_t)(tabs - ws_d) & 1);              // 16-byte alignment of the double2 twiddles
-      p.ts_Q = nxs / TS_P; p.ts_QT = QT;
-      p.ts_a1 = tabs; p.ts_tw = tabs + (size_t)QT * TS_A1_SLICE; p.ts_a2 = tabs + (size_t)QT * (TS_A1_SLICE + TS_TW_SLICE);
-      const int nthr = QT * TS_U * 2 * 32 > TS_A2_DOUBLES ? QT * TS_U * 2 * 32 : TS_A2_DOUBLES;
-      twostage_tables_kernel<<<cdiv(nthr, 256), 256, 0, st>>>(nxs, p.ts_Q, QT, tabs, tabs + (size_t)QT * TS_A1_SLICE,
-                                                             tabs + (size_t)QT * (TS_A1_SLICE + TS_TW_SLICE));
-      rc = check_launch("twostage_tables_kernel");
-      if (rc) return rc;
-    }
-    return launch_transform_ws(p, ring, counter, st);
   }
-  if (rho_d)
-    return fail(HMV_E_LIMIT, "hmv_profile_transform_samples: needs the persistent kernel (16-byte aligned ks/uk/ws, even ldk, "
-                "transform mode 0, nxs < 65536)");
-  const size_t budget = 226 * 1024;   // 227 KB opt-in limit minus the static per-halo arrays
-  const int J = p.J;
-  if (transform_smem<8, NCH_MMA>(J + 2) <= budget) {
-    // table path, three bin-count classes (a CTA whose bin count is outside (jlo, jhi] exits immediately)
-    sine_table_kernel<<<cdiv(nxs, 256), 256, 0, st>>>(nxs, reinterpret_cast<double2*>(ws_d), p.kt1, nullptr);
-    int rc = check_launch("sine_table_kernel");
-    if (rc) return rc;
-    rc = bin_counts(8);
-    if (rc) return rc;
-    const int jA = 254, jB = 510, jC = 1022;           // class upper bounds: 4 / 3 / 2 / 1 CTAs fit per SM
-    auto hi = [&](int j) { return j < J ? j : J; };
-    if (J > jC) {
-      rc = launch_transform<8, 512, true, 8, NCH_MMA>(p, jC, J, J + 2, st);            // heavy CTAs first
-      if (rc) return rc;
-    }
-    if (J > jB) {
-      rc = launch_transform<8, 256, true, 8, NCH_MMA>(p, jB, hi(jC), hi(jC) + 2, st);
-      if (rc) return rc;
-    }
-    if (J > jA) {
-      rc = launch_transform<8, 256, true, 4, NCH_ROT>(p, jA, hi(jB), hi(jB) + 2, st);
-      if (rc) return rc;
-    }
-    return launch_transform<8, 256, true, 4, NCH_ROT>(p, 0, hi(jA), hi(jA) + 2, st);
-  }
-  // large N: rotation recurrence, widest halo batch whose bin table fits
-#define HMV_ROT(HBV)                                                                   \
-  if (transform_smem<HBV, NCH_ROT>(J + 2) <= budget) {                                 \
-    const int rc = bin_counts(HBV);                                                    \
-    return rc ? rc : launch_transform<HBV, 256, false, 1, NCH_ROT>(p, 0, J, J + 2, st);            \
-  }
-  HMV_ROT(8) HMV_ROT(4) HMV_ROT(2) HMV_ROT(1)
-#undef HMV_ROT
-  return fail(HMV_E_LIMIT, "hmv_profile_transform: nxs=%d needs %zu B of shared memory per halo (limit %zu)", nxs,
-              transform_smem<1, NCH_ROT>(J + 2), budget);
+  return launch_transform_ws(p, ws_d + w.ring, counter, st);
 }
 
 extern "C" int hmv_profile_transform(int nz, int nm, int nk, int ldk, const double* zs_d, const double* ks_d,

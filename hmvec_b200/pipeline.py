@@ -184,7 +184,7 @@ class GridSix(object):
             self.cl = E(self.ncl, self.nl)
             self.h_cl = torch.empty((self.ncl, self.nl), dtype=torch.float64).pin_memory()
         self.launches_per_run = 0
-        self.transform_mode = 0
+        self.transform_mode = 0      # the transform's only launch plan; bench.py sets this attribute and reads it back
         self._ev = None
         self._Pfull = None
         self._Ppack = None
@@ -391,8 +391,7 @@ class GridSix(object):
                                            ptr(d["cmax"]), ptr(d["xc"]), ptr(d["alpha"]), ptr(d["expo"]), ptr(d["amp"]),
                                            ptr(d["oscale"]), self.gamma, self.xmax, self.nxs, 1, ptr(d["tr_ws"]),
                                            ptr(self.ue), st), "hmv_profile_transform")
-        # gnfw_params, sine_table, bin_count + one persistent kernel (or the four bin-count classes)
-        self._n += 4 if self.transform_mode == 0 else 7
+        self._n += 4                 # gnfw_params, sine_table, bin_count + the persistent transform kernel
 
     def _st_pressure(self, ws):
         # Compton-y profile (hmvec.py:252-316): pressure GNFW, no mass norm, scaled by 4 pi sigma_T/(m_e c^2)
@@ -416,7 +415,7 @@ class GridSix(object):
                                                ptr(d["y_amp"]), ptr(d["y_oscale"]), float(p['battaglia_pres_gamma']),
                                                self.p_xmax, self.p_nxs, 0, ptr(ws), ptr(self.uy), st),
                        "hmv_profile_transform(pressure)")
-        self._n += 4 if self.transform_mode == 0 else 7
+        self._n += 4
 
     def _st_six(self, overlap_d2h):
         # z-chunked so that (in e2e mode) the device->host copy of a finished chunk overlaps the next chunk's kernel

@@ -90,13 +90,15 @@ int hmv_gnfw_params(int kind, int nz, int nm, const double* zs_d, const double* 
  * Per halo: samples x_n=(n+1) xmax/nxs, theta-cut at cmax, trapezoid mass norm, the rFFT-equivalent sine
  * sums U_j = step sum_n x_n y_n sin(2 pi j n/N), u_j = U_j/kt_j/mnorm, kout_j = kt_j/rs/(1+z), then linear
  * interpolation onto ks (hold u_1 below the first bin, 0 above the last).  The (z,M,x) cube is never stored.
- * outscale_d may be NULL (=1).  do_mass_norm as in generic_profile_fft.  ks need not be sorted.
- * ws_d: workspace of hmv_profile_transform_ws_doubles(nz,nm,nxs) doubles (sine table, per-CTA bin counts, work-queue
- * head and the per-CTA ring of bin tables), 16-byte aligned. */
+ * outscale_d may be NULL (=1).  do_mass_norm as in generic_profile_fft.  ks need not be sorted.  ks_d, uk_d and ws_d
+ * must be 16-byte aligned and ldk even (HMV_E_ARG otherwise), as for the other three transform entry points.
+ * ws_d: workspace of hmv_profile_transform_ws_doubles(nz,nm,nxs) doubles (sine table, per-item bin counts, work-queue
+ * head and the per-group bin tables of the persistent kernel). */
 long long hmv_profile_transform_ws_doubles(int nz, int nm, int nxs);
-/* Process-wide choice of the transform's launch plan: 0 (default) = one persistent, warp-specialised kernel (producer
- * warps: samples + tensor-core sine sums; consumer warps: interpolation + row stores, overlapped through a ring of bin
- * tables); 1 = the earlier four bin-count-class kernels (kept for A/B measurements).  Same results either way. */
+/* The transform has one launch plan: a persistent kernel with two 8-warp groups per SM, each group evaluating the
+ * samples and running the tensor-core sine sums of 16 halos and then interpolating and storing their rows, so that one
+ * group's sums overlap the other's stores.  Mode 0 selects it and is accepted for ABI stability; any other mode
+ * returns HMV_E_ARG. */
 int hmv_set_transform_mode(int mode);
 int hmv_profile_transform(int nz, int nm, int nk, int ldk, const double* zs_d, const double* ks_d,
                           double kmax /* hint for max(ks); the kernels also reduce ks on the device and use the larger of the two */, const double* rs_d,

@@ -60,6 +60,37 @@ def test_k5_rejects_before_any_launch():
     assert rc == HMV_E_LIMIT and "shared memory" in capi.last_error()
 
 
+def test_k1_rejects_before_any_launch():
+    """The transform has one launch plan, selected by mode 0 alone, and its four entry points all read ks, the workspace
+    and the cube or tables with 16-byte accesses: a misaligned pointer or an odd ldk is refused before the first
+    launch (dummy device pointers, no GPU), never routed to another kernel."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("dummy device pointers must never reach a launch on a GPU")
+    from hmvec_b200 import _capi as capi
+    L = capi.lib
+    assert L.hmv_set_transform_mode(0) == 0
+    assert L.hmv_set_transform_mode(1) == HMV_E_ARG
+    ptr = [ctypes.c_void_p(0x10000 + 0x100 * i) for i in range(12)]     # non-null, 16-byte aligned, never dereferenced
+    bad = ctypes.c_void_p(0x20008)                                       # misaligned
+    nz, nm, nk, nxs = 2, 40, 30, 5000
+    calls = {
+        "transform, odd ldk": lambda: L.hmv_profile_transform(nz, nm, nk, 31, ptr[0], ptr[1], 1.0, *ptr[2:9], 1.0,
+                                                              20.0, nxs, 1, ptr[9], ptr[10], None),
+        "transform, misaligned ks": lambda: L.hmv_profile_transform(nz, nm, nk, 32, ptr[0], bad, 1.0, *ptr[2:9], 1.0,
+                                                                    20.0, nxs, 1, ptr[9], ptr[10], None),
+        "tables, misaligned ws": lambda: L.hmv_profile_tables(nz, nm, nk, ptr[0], ptr[1], 1.0, *ptr[2:9], 1.0, 20.0,
+                                                              nxs, 1, bad, ptr[10], None),
+        "expand, misaligned ws": lambda: L.hmv_profile_expand(nz, nm, nk, 32, ptr[0], ptr[1], 1.0, ptr[2], 20.0, nxs,
+                                                              bad, ptr[3], ptr[4], None),
+        "samples, misaligned ws": lambda: L.hmv_profile_transform_samples(nz, nm, nk, 32, ptr[0], ptr[1], 1.0,
+                                                                          *ptr[2:6], 20.0, nxs, 1, bad, ptr[6], None),
+    }
+    for what, call in calls.items():
+        rc = call()
+        assert rc == HMV_E_ARG and "16-byte aligned" in capi.last_error(), (what, rc, capi.last_error())
+
+
 def test_no_cpu_fallback_in_product():
     """The product package must not import the oracle (or the reference) anywhere."""
     pkg = os.path.join(ROOT, "hmvec_b200")
