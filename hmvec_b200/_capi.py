@@ -83,6 +83,11 @@ _SIGS = {
                                _p, _p, _p]),
     "hmv_limber": (_i, [_i, _p, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p]),
     "hmv_limber_multi": (_i, [_i, C.POINTER(LimberJob), _i, _p, _i, _i, _i, _p, _p, _p]),
+    "hmv_trispec_1h_ws_doubles": (_ll, [_i, _i, _i, _i]),
+    "hmv_trispec_1h": (_i, [_i, _i, _i, _i, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p, _p, _p]),
+    "hmv_cl_cov_1h_ws_doubles": (_ll, [_i, _i, _i, _i]),
+    "hmv_cl_cov_1h": (_i, [_i, _i, _i, _i, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p, _p, _p,
+                           _p, _p, _p]),
     "hmv_ksz_nvv_integral": (_i, [_i, _i, _p, _p, _ll, _p, _ll, _p, _ll, _p, _p, _p]),
     "hmv_pack_sum": (_i, [_i, _i, _i, C.POINTER(_p), C.POINTER(_p), _p, _p]),
     "hmv_peer_alloc": (_i, [_ll, C.POINTER(_p), C.c_char_p]),

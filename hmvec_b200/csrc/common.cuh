@@ -72,6 +72,16 @@ __device__ __forceinline__ double trapz_weight(const double* __restrict__ x, int
   return 0.5 * (hi - lo);
 }
 
+__device__ __forceinline__ int interval(const double* __restrict__ x, int n, double v) {
+  // largest i in [0, n-2] with x[i] <= v  (v already clamped to [x[0], x[n-1]])
+  int lo = 0, hi = n - 1;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (x[mid] <= v) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
 // ---- mbarrier / bulk-copy primitives (PTX; SASS: SYNCS.*, UBLKCP) ----------------------------------------------
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {

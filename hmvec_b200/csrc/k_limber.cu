@@ -6,16 +6,6 @@
 
 namespace hmv {
 
-__device__ __forceinline__ int interval(const double* __restrict__ x, int n, double v) {
-  // largest i in [0, n-2] with x[i] <= v  (v already clamped to [x[0], x[n-1]])
-  int lo = 0, hi = n - 1;
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if (x[mid] <= v) lo = mid; else hi = mid;
-  }
-  return lo;
-}
-
 __device__ __forceinline__ void limber_warp(int nl, const double* __restrict__ ells, int nzp, int nk, int ldp,
                                             const double* __restrict__ zs, const double* __restrict__ ks,
                                             const double* __restrict__ P, const double* __restrict__ P2, int ngz,

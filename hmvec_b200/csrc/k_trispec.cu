@@ -1,0 +1,231 @@
+// k_trispec.cu -- the 1-halo trispectrum of profile tracers and the non-Gaussian Limber covariance of C_l it projects to.
+// The reference has no counterpart.  Definitions (DESIGN.md §3.7): with legs t_X(z,m,k) = a_X(z,m) u_X(z,m,k),
+// a = M/rho_m0 (matter) or 1 (pressure), u linear in k on the ks grid and clamped to its ends,
+//   T^{ABCD}(k1,k2;z) = sum_m w_m n(z,m) t_A(k1) t_B(k1) t_C(k2) t_D(k2)                         (w_m: trapezoid on ms)
+//   Cov^{AB,CD}(l,l') = sum_z zeta_z pref_z T((l+1/2)/chi_z, (l'+1/2)/chi_z; z),  pref = H^3 W_A W_B W_C W_D/chi^6/(4 pi fsky)
+// (zeta_z: trapezoid on zs, 1 for a single redshift).  No 1-halo damping factor is applied.
+//
+// Both are one FP64 contraction over K = (z, m): a panel kernel writes P1[K][l] = w_m n (zeta pref) t_A t_B at k1 and
+// P2[K][l'] = t_C t_D at k2, and sigma2_gemm_kernel<MT, A K-major> forms C = P1^T P2 on the tensor pipe -- over all of
+// K with a fixed-order split-k reduction for the covariance, batched over z (K = m, one batch item per split index)
+// for the trispectrum.  A last kernel sums the splits in a fixed order and drops the padding column.
+#include "common.cuh"
+#include "gemm_f64.cuh"
+
+namespace hmv {
+
+constexpr int TP_T = 256, TP_MROWS = 32;   // panel kernel: columns per CTA, mass rows per CTA
+
+struct TrispecLegs {
+  const double* u[4];   // cubes [nz][nm][ldk] of A, B (k1 panel) and C, D (k2 panel)
+  int matter[4];        // 1: a = M/rho_m0, 0: a = 1
+};
+
+// interpolation interval and weight of k on ks, k clamped to [ks[0], ks[nk-1]] (as hmv_limber)
+__device__ __forceinline__ void k_locate(const double* __restrict__ ks, int nk, double k, int& j, double& f) {
+  k = fmin(fmax(k, ks[0]), ks[nk - 1]);
+  j = interval(ks, nk, k);
+  HMV_DEV_ASSERT(j >= 0 && j + 1 < nk);
+  f = (k - ks[j]) / (ks[j + 1] - ks[j]);
+}
+
+__device__ __forceinline__ double k_lerp(const double* __restrict__ row, int j, double f) {
+  const double a = row[j];
+  return fma(f, row[j + 1] - a, a);
+}
+
+// One CTA: redshift blockIdx.y, columns blockIdx.x*TP_T.., mass rows blockIdx.z*TP_MROWS.. of both panels.  A column's
+// interval and weight are the same on every mass row, so each thread locates its k once.  Rows m in [nm, nmp) and
+// columns in [n, ld) are written as zeros (the contraction reads whole 16-byte words).  chis == nullptr: 3D mode, q
+// are wavenumbers; otherwise q are multipoles, k = (q + 1/2)/chi_z and row weights carry zeta_z pref_z.
+__global__ void __launch_bounds__(TP_T) trispec_panel_kernel(int nz, int nm, int nmp, int nk, int ldk,
+                                                             const double* __restrict__ ks, const double* __restrict__ ms,
+                                                             const double* __restrict__ nzm, double rho_m0,
+                                                             const TrispecLegs L, int n1, int ld1,
+                                                             const double* __restrict__ q1, int n2, int ld2,
+                                                             const double* __restrict__ q2, const double* __restrict__ zs,
+                                                             const double* __restrict__ chis,
+                                                             const double* __restrict__ pref, double* __restrict__ P1,
+                                                             double* __restrict__ P2) {
+  const int z = blockIdx.y, l = blockIdx.x * TP_T + threadIdx.x;
+  const int m0 = blockIdx.z * TP_MROWS, m1 = min(nmp, m0 + TP_MROWS);
+  HMV_DEV_ASSERT(z < nz && (nmp == nm || nmp == nm + 1));
+  const bool c1 = l < n1, c2 = l < n2;
+  double zfac = 1.0, inv_chi = 0.0;
+  if (chis) {
+    zfac = pref[z] * (nz > 1 ? trapz_weight(zs, z, nz) : 1.0);
+    inv_chi = 1.0 / chis[z];
+  }
+  int j1 = 0, j2 = 0;
+  double f1 = 0.0, f2 = 0.0;
+  if (c1) k_locate(ks, nk, chis ? (q1[l] + 0.5) * inv_chi : q1[l], j1, f1);
+  if (c2) k_locate(ks, nk, chis ? (q2[l] + 0.5) * inv_chi : q2[l], j2, f2);
+  for (int m = m0; m < m1; ++m) {
+    const long long K = (long long)z * nmp + m;
+    double v1 = 0.0, v2 = 0.0;
+    if (m < nm) {
+      const long long row = ((long long)z * nm + m) * ldk;
+      const double a = ms[m] / rho_m0;
+      if (c1) {
+        const double wn = trapz_weight(ms, m, nm) * nzm[(long long)z * nm + m] * zfac;
+        v1 = wn * (L.matter[0] ? a : 1.0) * k_lerp(L.u[0] + row, j1, f1) * (L.matter[1] ? a : 1.0) *
+             k_lerp(L.u[1] + row, j1, f1);
+      }
+      if (c2) v2 = (L.matter[2] ? a : 1.0) * k_lerp(L.u[2] + row, j2, f2) * (L.matter[3] ? a : 1.0) *
+                   k_lerp(L.u[3] + row, j2, f2);
+    }
+    if (l < ld1) P1[K * ld1 + l] = v1;
+    if (l < ld2) P2[K * ld2 + l] = v2;
+  }
+}
+
+// out[b][i][j] = sum_s part[b*ns + s][i][j] (fixed order: deterministic), j < n2 of the ld2-wide rows
+__global__ void trispec_reduce_kernel(long long n, int ns, int n1, int n2, int ld2, const double* __restrict__ part,
+                                      double* __restrict__ out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const long long per = (long long)n1 * n2;
+  const long long b = i / per, r = i - b * per;
+  const long long row = r / n2, col = r - row * n2;
+  const long long stride = (long long)n1 * ld2;
+  const double* p = part + b * ns * stride + row * ld2 + col;
+  double s = 0.0;
+  for (int q = 0; q < ns; ++q) s += p[q * stride];
+  out[i] = s;
+}
+
+// ---- launch plan: a function of the shapes only, so that the workspace size and the launch agree ----------------------
+struct TrispecPlan {
+  int mt;               // 8*mt output rows per CTA
+  int nmp, ld1, ld2;    // mass rows and panel widths, padded to even
+  long long K;          // nz * nmp
+  int kchunk, nsplit;   // K range of one split index, split indices per batch item
+  int nbatch;           // 1 (covariance) or nz (trispectrum)
+};
+
+static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2) {
+  TrispecPlan p;
+  p.mt = n1 <= 32 ? 4 : n1 <= 64 ? 8 : n1 <= 128 ? 16 : 26;
+  p.nmp = nm + (nm & 1);
+  p.ld1 = n1 + (n1 & 1);
+  p.ld2 = n2 + (n2 & 1);
+  p.K = (long long)nz * p.nmp;
+  if (!proj) {                       // one batch item per redshift: its K range is its nmp mass rows
+    p.kchunk = p.nmp;
+    p.nsplit = 1;
+    p.nbatch = nz;
+    return p;
+  }
+  // Split K so that the grid is about sixteen waves of resident CTAs (148 SMs; MT = 26 runs one CTA per SM): the last
+  // wave is then a small fraction of the run.  CTAs are issued tile-fastest, so the resident ones walk the same K range
+  // together and every panel row comes from HBM about once, the other tiles finding it in L2.  At least eight k
+  // steps per split.
+  const long long tiles = (long long)cdiv(p.ld2, SG_BN) * cdiv(n1, 8 * p.mt);
+  const long long slots = 148LL * (p.mt > 16 ? 1 : 2);
+  long long s = 16 * slots / tiles;
+  if (s < 1) s = 1;
+  if (s > 64) s = 64;
+  const long long maxs = (p.K + 8 * SG_BK - 1) / (8 * SG_BK);
+  if (s > maxs) s = maxs;
+  p.kchunk = cdiv(cdiv(p.K, s), SG_BK) * SG_BK;
+  p.nsplit = cdiv(p.K, p.kchunk);
+  p.nbatch = 1;
+  return p;
+}
+
+static long long trispec_ws(const TrispecPlan& p, int n1) {
+  return p.K * (p.ld1 + p.ld2) + (long long)p.nbatch * p.nsplit * n1 * p.ld2;
+}
+
+static long long trispec_ws_doubles(bool proj, int nz, int nm, int n1, int n2) {
+  if (nz <= 0 || nm <= 0 || n1 <= 0 || n2 <= 0) return 0;
+  return trispec_ws(trispec_plan(proj, nz, nm, n1, n2), n1);
+}
+
+template <int MT>
+static cudaError_t trispec_gemm(const TrispecPlan& p, int n1, const double* P1, const double* P2, double* part,
+                                cudaStream_t st) {
+  const size_t smem = (size_t)sg_smem_doubles<MT, true>() * sizeof(double);
+  cudaError_t e = cudaFuncSetAttribute(sigma2_gemm_kernel<MT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem);
+  if (e != cudaSuccess) return e;
+  dim3 grid(cdiv(p.ld2, SG_BN), cdiv(n1, 8 * MT), p.nbatch * p.nsplit);
+  sigma2_gemm_kernel<MT, true><<<grid, SG_T, smem, st>>>(n1, p.ld2, (int)p.K, p.kchunk, P1, P2, part,
+                                                         (long long)n1 * p.ld2, p.ld1);
+  return cudaSuccess;
+}
+
+static int trispec_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                       const double* ms_d, const double* nzm_d, double rho_m0, const double* const* u_h,
+                       const int* kind_h, int n1, const double* q1_d, int n2, const double* q2_d, const double* zs_d,
+                       const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream) {
+  HMV_REQUIRE(nz >= 1 && nm >= 1 && nk >= 2 && n1 >= 1 && n2 >= 1,
+              "%s: sizes must be >= 1 and nk >= 2 (nz=%d nm=%d nk=%d n1=%d n2=%d)", who, nz, nm, nk, n1, n2);
+  HMV_REQUIRE(ldk >= nk && (ldk & 1) == 0, "%s: ldk must be even and >= nk (ldk=%d nk=%d)", who, ldk, nk);
+  HMV_REQUIRE(ks_d && ms_d && nzm_d && u_h && kind_h && q1_d && q2_d && ws_d && out_d, "%s: null pointer", who);
+  HMV_REQUIRE(!proj || (zs_d && chis_d && pref_d), "%s: null pointer (zs, chis or pref)", who);
+  TrispecLegs L;
+  for (int i = 0; i < 4; ++i) {
+    HMV_REQUIRE(u_h[i], "%s: null pointer (cube %d)", who, i);
+    HMV_REQUIRE(kind_h[i] == 0 || kind_h[i] == 2, "%s: cube %d: kind %d is neither 0 (matter) nor 2 (pressure)", who, i,
+                kind_h[i]);
+    HMV_REQUIRE(((size_t)u_h[i] & 15) == 0, "%s: cube %d must be 16-byte aligned", who, i);
+    L.u[i] = u_h[i];
+    L.matter[i] = kind_h[i] == 0;
+  }
+  HMV_REQUIRE(((size_t)ws_d & 15) == 0, "%s: workspace must be 16-byte aligned", who);
+  if (nz > 65535) return fail(HMV_E_LIMIT, "%s: nz=%d exceeds 65535 (grid y of the panel kernel)", who, nz);
+  const TrispecPlan p = trispec_plan(proj, nz, nm, n1, n2);
+  if (p.K > (1LL << 30))
+    return fail(HMV_E_LIMIT, "%s: nz * nm = %lld exceeds 2^30 (32-bit k index of the contraction)", who, p.K);
+  double* P1 = ws_d;
+  double* P2 = P1 + p.K * p.ld1;
+  double* part = P2 + p.K * p.ld2;
+  cudaStream_t st = (cudaStream_t)stream;
+  dim3 pg(cdiv(p.ld1 > p.ld2 ? p.ld1 : p.ld2, TP_T), nz, cdiv(p.nmp, TP_MROWS));
+  trispec_panel_kernel<<<pg, TP_T, 0, st>>>(nz, nm, p.nmp, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, L, n1, p.ld1, q1_d, n2,
+                                            p.ld2, q2_d, zs_d, proj ? chis_d : nullptr, pref_d, P1, P2);
+  int rc = check_launch("trispec_panel_kernel");
+  if (rc) return rc;
+  cudaError_t e;
+  switch (p.mt) {
+    case 4: e = trispec_gemm<4>(p, n1, P1, P2, part, st); break;
+    case 8: e = trispec_gemm<8>(p, n1, P1, P2, part, st); break;
+    case 16: e = trispec_gemm<16>(p, n1, P1, P2, part, st); break;
+    default: e = trispec_gemm<26>(p, n1, P1, P2, part, st); break;
+  }
+  if (e != cudaSuccess) return fail(HMV_E_CUDA, "%s: sigma2_gemm_kernel smem opt-in: %s", who, cudaGetErrorString(e));
+  rc = check_launch("sigma2_gemm_kernel<A K-major>");
+  if (rc) return rc;
+  const long long n = (long long)p.nbatch * n1 * n2;
+  trispec_reduce_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, p.nsplit, n1, n2, p.ld2, part, out_d);
+  return check_launch("trispec_reduce_kernel");
+}
+
+}  // namespace hmv
+
+using namespace hmv;
+
+extern "C" long long hmv_trispec_1h_ws_doubles(int nz, int nm, int nk1, int nk2) {
+  return trispec_ws_doubles(false, nz, nm, nk1, nk2);
+}
+
+extern "C" int hmv_trispec_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                              const double* nzm_d, double rho_m0, const double* const* u_h, const int* kind_h, int nk1,
+                              const double* k1_d, int nk2, const double* k2_d, double* ws_d, double* out_d,
+                              void* stream) {
+  return trispec_run("hmv_trispec_1h", false, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, u_h, kind_h, nk1, k1_d, nk2,
+                     k2_d, nullptr, nullptr, nullptr, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_cl_cov_1h_ws_doubles(int nz, int nm, int nl1, int nl2) {
+  return trispec_ws_doubles(true, nz, nm, nl1, nl2);
+}
+
+extern "C" int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                             const double* nzm_d, double rho_m0, const double* const* u_h, const int* kind_h, int nl1,
+                             const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                             const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream) {
+  return trispec_run("hmv_cl_cov_1h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, u_h, kind_h, nl1, ells1_d, nl2,
+                     ells2_d, zs_d, chis_d, pref_d, ws_d, out_d, stream);
+}

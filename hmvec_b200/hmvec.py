@@ -910,6 +910,99 @@ class HaloModel(Cosmology):
         self._check_hods()
         return {t: h1[i] for i, t in enumerate(tags)}, {t: h2[i] for i, t in enumerate(tags)}
 
+    # ------------------------------------------------------------------ 1-halo trispectrum and C_l covariance
+    def _trispec_legs(self, names):
+        """Device cubes and kinds of four profile tracers: matter profile first, then pressure profile.  A table-backed
+        profile is expanded to its cube (DeviceCubes.device)."""
+        cubes, kinds = [], []
+        for n in names:
+            if n in self.uk_profiles:
+                cubes.append(self.uk_profiles.device(n))
+                kinds.append(_KIND_MATTER)
+            elif n in self.pk_profiles:
+                cubes.append(self.pk_profiles.device(n))
+                kinds.append(_KIND_PRESSURE)
+            elif n in self.hods:
+                raise ValueError("%r is an HOD: its 1-halo trispectrum needs occupation moments up to fourth order, "
+                                 "which the HOD does not define" % (n,))
+            else:
+                raise ValueError("no matter or pressure profile named %r" % (n,))
+        if not np.all(np.diff(self._ks64) > 0):
+            raise ValueError("the model's ks must be strictly increasing for the trispectrum's interpolation")
+        return cubes, kinds
+
+    @staticmethod
+    def _positive(x, what):
+        x = np.asarray(x, dtype=np.float64).reshape(-1)
+        if x.size == 0 or not np.all(np.isfinite(x)) or not np.all(x > 0):
+            raise ValueError("%s must be a non-empty list of positive finite values" % what)
+        return x
+
+    def _trispec_call(self, fn, names, q1, q2, extra, out_shape):
+        cubes, kinds = self._trispec_legs(names)
+        nz, nm = self._nz, self._nm
+        ws = self._workspace('trispec', getattr(capi.lib, fn + '_ws_doubles')(nz, nm, q1.size, q2.size))
+        out = self._empty(*out_shape)
+        q1_d, q2_d = self._dev(q1), self._dev(q2)
+        u_h = (C.c_void_p * 4)(*[c.data_ptr() for c in cubes])
+        capi.check(getattr(capi.lib, fn)(nz, nm, self._nk, self._ldk, capi.ptr(self._ks_d), capi.ptr(self._ms_d),
+                                         capi.ptr(self._nzm_d), self._rho_m0, u_h, (C.c_int * 4)(*kinds), q1.size,
+                                         capi.ptr(q1_d), q2.size, capi.ptr(q2_d), *[capi.ptr(e) for e in extra],
+                                         capi.ptr(ws), capi.ptr(out), capi.stream()), fn)
+        return self._host(out)
+
+    def get_trispectrum_1halo(self, ks1, ks2=None, name="nfw", name2=None, name3=None, name4=None):
+        """1-halo trispectrum T^{ABCD}(k1, k2; z) = sum_M w_M n(z,M) t_A(k1) t_B(k1) t_C(k2) t_D(k2), [nz, nk1, nk2].
+
+        No counterpart in the reference (Cooray & Hu 2001, eq. 17).  A profile tracer's leg is t = (M/rho_m0) u(k|M,z)
+        for a matter profile and u(k|M,z) for a pressure profile, the weights of get_power_1halo; w_M is the trapezoid
+        weight on ms.  u is interpolated linearly in k on `ks`, and k outside [ks[0], ks[-1]] is clamped to the edge.
+        No 1-halo damping factor (1 - exp(-(k/k*)^2)) is applied.  Names resolve as matter profile, then pressure
+        profile; HODs raise ValueError.  Defaults: name2 = name, name3 = name, name4 = name3, ks2 = ks1.  ks1 and ks2
+        need not be sorted."""
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        k1 = self._positive(ks1, "ks1")
+        k2 = k1 if ks2 is None else self._positive(ks2, "ks2")
+        return self._trispec_call('hmv_trispec_1h', (name, name2, name3, name4), k1, k2, (),
+                                  (self._nz, k1.size, k2.size))
+
+    def get_cl_cov_1halo(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
+                         ells2=None):
+        """Non-Gaussian (1-halo) Limber covariance Cov(C_l^{AB}, C_l'^{CD}), [len(ells), len(ells2)]:
+
+            1/(4 pi fsky) sum_z zeta_z H^3 W_A W_B W_C W_D / chi^6 T^{ABCD}((l+1/2)/chi, (l'+1/2)/chi; z)
+
+        with the window convention of limber_integral (C = int dz H W1 W2/chi^2 P), zeta_z the trapezoid weight on
+        self.zs (1 for a single redshift) and T as in get_trispectrum_1halo (no 1-halo damping).  Each window is a
+        scalar or an [nz] array on self.zs: lensing_window(zs, lzs) for kappa, 1 for Compton-y (1/H is inside the y
+        profile).  Defaults: name2 = name, name3 = name, name4 = name3, ells2 = ells; multipoles need not be sorted.
+        Not available on a z-sharded model (the z sum would need a cross-rank reduction)."""
+        if self._zcomm is not None:
+            raise NotImplementedError("get_cl_cov_1halo on a z-sharded model: the z sum spans the ranks")
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        l1 = self._positive(ells, "ells")
+        l2 = l1 if ells2 is None else self._positive(ells2, "ells2")
+        fsky = float(fsky)
+        if not (0.0 < fsky <= 1.0):
+            raise ValueError("fsky must lie in (0, 1]")
+        if len(windows) != 4:
+            raise ValueError("windows must hold four entries (A, B, C, D)")
+        W = np.ones(self._nz)
+        for w in windows:
+            w = np.asarray(w, dtype=np.float64)
+            if w.ndim > 1 or (w.ndim == 1 and w.size != self._nz):
+                raise ValueError("each window must be a scalar or an array of length nz=%d" % self._nz)
+            W = W * w
+        chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
+        H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
+        pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
+        extra = (self._zs_d, self._dev(chis), self._dev(pref))
+        return self._trispec_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+
 
     # ------------------------------------------------------------------ cluster-lensing helper
     def kappa_2h_profiles(self, thetas, Ms, zsource, delta=200, rho='mean', rho_at_z=True, lmin=100, lmax=10000,

@@ -284,6 +284,32 @@ int hmv_debug_k1_order(int nz, int nm, int grid, int* z_out, int* q_out);
 int hmv_debug_wave_tile(int nz, int ldk);
 int hmv_debug_tab_order(int nz, int nk, int* z_out, int* k0_out);
 
+/* ---- 1-halo trispectrum and the non-Gaussian Limber covariance of C_l ----------------------------------------------
+ * No counterpart in the reference.  The 1-halo term of the power-spectrum covariance (Cooray & Hu 2001, ApJ 554, 56,
+ * eq. 17; Cooray & Sheth 2002, Phys. Rep. 372, 1, §6.2) and its Limber projection (Komatsu & Seljak 2002, MNRAS 336,
+ * 1256, eq. 14 for the tSZ), with the window convention of hmv_limber (C = int dz H W1 W2/chi^2 P).  A profile
+ * tracer's leg is t_X(z,m,k) = a_X u_X(z,m,k): kind 0 (matter) a = M/rho_m0, kind 2 (pressure) a = 1, as in hmv_power;
+ * u is linear in k on ks (strictly increasing, nk >= 2) with k clamped to [ks[0], ks[nk-1]] as in hmv_limber.
+ *   T^{ABCD}(k1,k2;z) = sum_m w_m n(z,m) t_A(k1) t_B(k1) t_C(k2) t_D(k2)      w_m: trapezoid weight on ms
+ *   Cov^{AB,CD}(l,l') = sum_z zeta_z pref[z] T((l+1/2)/chi[z], (l'+1/2)/chi[z]; z)
+ * with zeta_z the trapezoid weight on zs (1 when nz == 1) and pref[z] = H^3 W_A W_B W_C W_D / chi^6 / (4 pi f_sky)
+ * supplied by the caller (W = the lensing window for kappa, 1 for Compton-y).  No 1-halo damping (1 - e^{-(k/k*)^2}).
+ * u_h / kind_h: HOST arrays of the four cubes [nz][nm][ldk] (A, B at k1; C, D at k2) and their kinds (0 or 2).
+ * k1/k2 and ells1/ells2 need not be sorted.  Cubes and ws_d must be 16-byte aligned and ldk even (HMV_E_ARG);
+ * nz <= 65535 and nz * nm <= 2^30 (HMV_E_LIMIT).  Every check is made before the first launch.
+ * One FP64 tensor-core contraction over (z, m): panels of t_A t_B (weights folded in) and t_C t_D in ws_d, then the
+ * sigma^2 GEMM (mma.sync m8n8k4) with a fixed-order split-k reduction: repeated calls give identical results.
+ * hmv_trispec_1h: out_d [nz][nk1][nk2].  hmv_cl_cov_1h: out_d [nl1][nl2].  ws_d: *_ws_doubles() doubles. */
+long long hmv_trispec_1h_ws_doubles(int nz, int nm, int nk1, int nk2);
+int hmv_trispec_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                   double rho_m0, const double* const* u_h, const int* kind_h, int nk1, const double* k1_d, int nk2,
+                   const double* k2_d, double* ws_d, double* out_d, void* stream);
+long long hmv_cl_cov_1h_ws_doubles(int nz, int nm, int nl1, int nl2);
+int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                  double rho_m0, const double* const* u_h, const int* kind_h, int nl1, const double* ells1_d, int nl2,
+                  const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d, double* ws_d,
+                  double* out_d, void* stream);
+
 /* ---- f2: kSZ consumer -- the short-wavelength integral of the velocity-reconstruction noise
  * (ksz.py:299-336, Nvv_core_integral):  out[b] = trapz_kS( kS Pge[b,kS]^2 / (Pgg_tot[b,kS] C_tot(chi* kS)) ) with
  * non-finite integrand values set to zero (ksz.py:98-100).  b = 0..nb-1 runs over the (mu,kL) plane when the spectra
