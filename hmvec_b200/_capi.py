@@ -116,10 +116,6 @@ for _name, (_res, _args) in _SIGS.items():
 
 EXPORTS = tuple(_SIGS)
 
-if os.environ.get("HMV_NFW_MODE"):             # A/B measurements of the NFW evaluation (see the header)
-    if lib.hmv_set_nfw_mode(int(os.environ["HMV_NFW_MODE"])) != 0:
-        raise ImportError("hmvec_b200: bad HMV_NFW_MODE=%r" % os.environ["HMV_NFW_MODE"])
-
 
 def last_error():
     return lib.hmv_last_error().decode("utf-8", "replace")

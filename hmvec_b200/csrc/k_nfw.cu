@@ -3,120 +3,28 @@
 // The reference evaluates  u = [sin x (Si X - Si x) - sin(cx)/X + cos x (Ci X - Ci x)]/m_c,  X=(1+c)x, x = k r_s (1+z),
 // with two scipy.special.sici calls per (z,M,k).  That closed form is the integral
 //        u(x; c) = (1/m_c) int_0^c  t/(1+t)^2  sinc(x t) dt .
-// Two evaluations are built on it (hmv_set_nfw_mode):
-//   0 (default)  per-halo piecewise polynomials in (x c)^2 on 21 fixed intervals up to x c = 64 whose coefficients come
-//                from one FP64 tensor-core contraction (second half of this file), the closed form's asymptotic
-//                branch beyond;
-//   1            the Maclaurin series in y = (x c)^2 for x c <= 16,
-//                    u = sum_n A_n y^n ,  A_n = (-1)^n c^2 Itilde_n / ((2n+1)! m_c) ,  Itilde_n = int_0^1 s^(2n+1)/(1+cs)^2 ds ,
-//                with per-halo coefficients from a small pre-pass (three-term recurrence in the moment order for
-//                c >= 1.5, 64-point Gauss-Legendre below; 5 to 39 FMAs per element, < 1e-11 relative), and the Si/Ci
-//                form with the device routines of sici.cuh beyond -- round 1's path, kept as the cross-check of the
-//                polynomial tables (one CTA per halo row, 256-wide k chunks, 8 elements per lane).
-#include "common.cuh"
-#include "nfw_device.cuh"
-#include "nfw_poly.cuh"
-
-namespace hmv {
-
-constexpr int NFW_T = 256, NFW_E = 8, NFW_CH = 32 * NFW_E;
-
-// max of ks over each NFW_CH-wide chunk: lets both passes classify a chunk with one load
-__global__ void nfw_chunkmax_kernel(int nk, const double* __restrict__ ks, double* __restrict__ kcmax) {
-  const int chunk = blockIdx.x, lane = threadIdx.x;
-  double m = 0.0;
-  for (int k = chunk * NFW_CH + lane; k < min(nk, (chunk + 1) * NFW_CH); k += 32) m = fmax(m, ks[k]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if (lane == 0) kcmax[chunk] = m;
-}
-
-// A CTA first sweeps the chunks that lie entirely in the series regime, then the remaining ones (some element with
-// x c > 16), which need the Si/Ci routines.  MODE 0/1 run only one of the two parts (kept for profiling them apart);
-// the library launches MODE 2, both in one kernel, so that the store-bound and the FP64-bound halves overlap.
-template <int MODE>   // 0 series only, 1 tail only, 2 both in one launch
-__global__ void __launch_bounds__(NFW_T, MODE ? 3 : 4) uk_nfw_kernel(int nk, int ldk, const double* __restrict__ ks,
-                                                        const double* __restrict__ coef,
-                                                        const double* __restrict__ kcmax, double kmax,
-                                                        double* __restrict__ uk) {
-  __shared__ __align__(16) double A[NFW_NREC];
-  const long long row = blockIdx.x;                   // row = z*nm + m
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const double* rec = coef + row * NFW_NREC;
-  const double ac = __ldg(rec + 44);
-  if (MODE == 1) {   // rows whose whole k-range is in the series regime have nothing to do here
-    if (kmax * ac <= NFW_XC_MAX) return;
-  }
-  if (threadIdx.x < NFW_NREC) A[threadIdx.x] = __ldg(rec + threadIdx.x);
-  __syncthreads();
-  double* out = uk + row * (long long)ldk;
-  const int nchunks = (nk + NFW_CH - 1) / NFW_CH;
-  if (MODE != 1) {
-    for (int chunk = warp; chunk < nchunks; chunk += NFW_T / 32) {
-      const double xcm = __ldg(kcmax + chunk) * ac;
-      if (xcm > NFW_XC_MAX) continue;                 // left to the tail pass
-      const int kbase = chunk * NFW_CH + lane;
-      const int nt = nfw_terms(xcm);                  // warp-uniform trip count
-      double y[NFW_E], u[NFW_E];
-#pragma unroll
-      for (int e = 0; e < NFW_E; ++e) {
-        const double xc = __ldg(ks + min(kbase + 32 * e, nk - 1)) * ac;
-        y[e] = xc * xc;
-      }
-      const double top = A[nt - 1];
-#pragma unroll
-      for (int e = 0; e < NFW_E; ++e) u[e] = top;
-      for (int i = nt - 2; i >= 1; i -= 2) {
-        const double2 a2 = *reinterpret_cast<const double2*>(A + i - 1);
-#pragma unroll
-        for (int e = 0; e < NFW_E; ++e) u[e] = fma(u[e], y[e], a2.y);
-#pragma unroll
-        for (int e = 0; e < NFW_E; ++e) u[e] = fma(u[e], y[e], a2.x);
-      }
-#pragma unroll
-      for (int e = 0; e < NFW_E; ++e) {
-        const int k = kbase + 32 * e;
-        if (k < nk) out[k] = u[e];
-      }
-    }
-  }
-  if (MODE != 0 && kmax * ac > NFW_XC_MAX) {
-    // every warp visits every tail chunk and takes its own 32-wide slice of it: the Si/Ci work of a row is spread
-    // evenly over the CTA's warps however few chunks are in the tail
-    static_assert(NFW_T / 32 == NFW_E, "one slice per warp");
-    const double c = A[42], a = A[43], ln1pc = A[45], inv_mc = A[46];
-    for (int cb = 0; cb < nchunks; cb += 32) {        // 32 chunks per ballot: visit only the tail chunks
-      const int cc = cb + lane;
-      unsigned tail = __ballot_sync(0xffffffffu, cc < nchunks && __ldg(kcmax + min(cc, nchunks - 1)) * ac > NFW_XC_MAX);
-      while (tail) {
-        const int chunk = cb + __ffs(tail) - 1;
-        tail &= tail - 1;
-        const int k = chunk * NFW_CH + 32 * warp + lane;
-        if (k < nk) {
-          const double kk = __ldg(ks + k), xc = kk * ac;
-          out[k] = (xc <= NFW_XC_MAX) ? nfw_horner(A, nfw_terms(xc), xc * xc) : nfw_bracket(kk * a, c, ln1pc) * inv_mc;
-        }
-      }
-    }
-  }
-}
-
-
-// =====================================================================================================================
-// Piecewise-polynomial form (the default path).  u_NFW depends on the halo through c alone once written in s = x c,
+//
+// Here it is evaluated as piecewise polynomials.  u_NFW depends on the halo through c alone once written in s = x c,
 // and is smooth in y = s^2: on 21 fixed intervals of s (edges 0,1,2,4,...,16,20,...,64) a per-halo polynomial of degree
-// 5..13 in the interval's local variable t reproduces it to < 7e-12 of the interval's max|u| for 1.2 <= c <= 25
-// (tools/gen_nfw_poly_tables.py --check, mpmath) -- where the Maclaurin series needs 5..39 terms, stops at s = 16, and
-// the closed form beyond costs ~90 FP64 instructions per element.  Work per element drops from ~25 to ~13 FP64
-// instructions on the LARGE grid (66 % of the elements have s <= 1: degree 5), which turns the kernel from
-// FP64-issue-bound into store-bound.
-//   nfw_poly_record_kernel : per halo, u at the Chebyshev nodes of every interval its k range reaches (series for
-//                            s <= 16, closed form beyond), times the node->monomial matrix of the interval
-//   uk_nfw_poly_kernel     : one CTA per halo row, 256-wide k chunks; a chunk whose min and max s fall into one
+// 5..13 in the interval's local variable t reproduces it to < 2e-11 of the interval's max|u| for 0.6 <= c <= 25
+// (tools/gen_nfw_poly_tables.py --check, mpmath), at ~13 FP64 instructions per element on the LARGE grid (66 % of the
+// elements have s <= 1: degree 5) where the closed form costs ~90: the kernel is store-bound.  Beyond s = 64 u_NFW
+// takes the closed form (nfw_bracket / nfw_bracket_far of sici.cuh).
+//   nfw_chunk_kernel       : per 256-wide k chunk, min and max of ks, and padded copies of ks and ks^2
+//   nfw_poly_gemm_kernel   : per halo, one record of NFW_REC doubles (polynomial coefficients and halo constants) from
+//                            one FP64 tensor-core contraction
+//   uk_nfw_poly_kernel     : one warp per halo row, 256-wide k chunks; a chunk whose min and max s fall into one
 //                            interval runs Horner with warp-uniform coefficients (one shared-memory load per 16 FMAs);
 //                            a chunk that straddles interval edges looks the coefficients up per element; elements
 //                            beyond s = 64 (6.8 % on the LARGE grid, all with x > 4) take the closed form's asymptotic
 //                            branch.  No assumption on the order of ks (chunk min/max come from a pre-pass).
+#include "common.cuh"
+#include "nfw_poly.cuh"
+
+namespace hmv {
+
+constexpr int NFW_T = 256, NFW_CH = 256;              // threads per CTA, wavenumbers per chunk
+
 // per 256-wide chunk: min and max of ks; copies of ks and ks^2 padded to whole chunks (last value repeated), so the
 // cube kernel reads 16-byte pairs without bounds checks
 __global__ void nfw_chunk_kernel(int nk, const double* __restrict__ ks, double* __restrict__ kcmin,
@@ -146,7 +54,8 @@ __global__ void nfw_chunk_kernel(int nk, const double* __restrict__ ks, double* 
 // node->monomial matrices cancel inside W).  No Si/Ci, no series, no per-node branches: per 16 halos, 64 reciprocals
 // per lane and 37 x 16 x 2 mma.sync m8n8k4 (SASS DMMA) with W resident in shared memory.  Checked against mpmath for
 // 0.6 <= c <= 25: same error as exact node values (< 2e-11 of an interval's max|u|, the truncation error).
-// Also writes the per-halo constants {c, a = r_s (1+z), a c, ln(1+c), 1/m_c} into slots 42..46 of the 48-double record.
+// The coefficients fill slots [0, NFWP_REC) of the halo's record, the constants {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0}
+// the last six.
 constexpr int NFWP_MAXCH = 128;                          // chunks whose min/max the cube kernel keeps in shared memory
 constexpr int NFWP_NT = (NFWP_REC + 7) / 8;              // 8-wide coefficient tiles
 constexpr size_t NFWP_GEMM_SMEM = ((size_t)NFWP_Q * NFWP_WLD + 2 * NFWP_Q) * sizeof(double);
@@ -156,7 +65,7 @@ __global__ void __launch_bounds__(256, 1) nfw_poly_gemm_kernel(long long rows, i
                                                                const double* __restrict__ zs,
                                                                const double* __restrict__ cs,
                                                                const double* __restrict__ rvir,
-                                                               double* __restrict__ rec48, double* __restrict__ prec) {
+                                                               double* __restrict__ rec) {
   extern __shared__ __align__(16) double gsm[];
   double* Wsm = gsm;                                     // [Q][WLD]
   double2* gl = reinterpret_cast<double2*>(gsm + (size_t)NFWP_Q * NFWP_WLD);   // {tau_q, w_q tau_q}
@@ -185,7 +94,7 @@ __global__ void __launch_bounds__(256, 1) nfw_poly_gemm_kernel(long long rows, i
       const double inv_mc = 1.0 / mc, pref = c * c * inv_mc;
       const double av = ok ? __ldg(rvir + row) / c * (1.0 + __ldg(zs + row / nm)) : 0.0;   // x = k r_s (1+z), hmvec.py:342,349
       if (ok && t4 == 0) {
-        double2* r = reinterpret_cast<double2*>(rec48 + row * NFW_NREC + 42);
+        double2* r = reinterpret_cast<double2*>(rec + row * NFW_REC + NFWP_REC);
         r[0] = make_double2(c, av); r[1] = make_double2(av * c, ln1pc); r[2] = make_double2(inv_mc, 0.0);
       }
       ivtop = max(ivtop, ok ? min(NFWP_NI - 1, nfwp_interval(kmax * av * c)) : 0);
@@ -223,7 +132,7 @@ __global__ void __launch_bounds__(256, 1) nfw_poly_gemm_kernel(long long rows, i
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt) {
             const long long row = grp * 16 + g + 8 * mt;
-            if (row < rows) *reinterpret_cast<double2*>(prec + row * NFWP_REC + r) = make_double2(acc[j][mt][0], acc[j][mt][1]);
+            if (row < rows) *reinterpret_cast<double2*>(rec + row * NFW_REC + r) = make_double2(acc[j][mt][0], acc[j][mt][1]);
           }
         }
       }
@@ -257,31 +166,23 @@ __device__ __noinline__ double nfwp_element(const double* R, const NfwpTables& T
 // its row's record into its own shared-memory slice, sweeps the leading chunks that lie entirely below s = 1 (two
 // thirds of the LARGE grid's elements) in a tight loop with the six coefficients in registers, and takes the remaining
 // chunks through the general route.  A lane owns four 16-byte pairs of a 256-wide chunk (coalesced 16-byte stores).
-#ifndef HMV_NFWP_MINB
-#define HMV_NFWP_MINB 3     // CTAs per SM the register allocation aims at (4 = 64 registers: measured below)
-#endif
-__global__ void __launch_bounds__(NFW_T, HMV_NFWP_MINB) uk_nfw_poly_kernel(long long rows, int nk, int ldk,
+// Three CTAs per SM is what the register allocation aims at (four would cap it at 64 registers).
+__global__ void __launch_bounds__(NFW_T, 3) uk_nfw_poly_kernel(long long rows, int nk, int ldk,
                                                                 const double* __restrict__ ksp,
                                                                 const double* __restrict__ k2p,
-                                                                const double* __restrict__ rec48,
-                                                                const double* __restrict__ prec,
+                                                                const double* __restrict__ rec,
                                                                 const double* __restrict__ kcmin,
                                                                 const double* __restrict__ kcmax,
                                                                 double* __restrict__ uk) {
-  __shared__ __align__(16) double Rall[NFW_T / 32][NFWP_REC + 6];      // record, then {c, a, a c, ln(1+c), 1/m_c, 0}
+  __shared__ __align__(16) double Rall[NFW_T / 32][NFW_REC];
   __shared__ NfwpTables T;
   __shared__ double2 cmm[NFWP_MAXCH];                       // {min, max} of ks per chunk (when they fit)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long row = (long long)blockIdx.x * (NFW_T / 32) + warp;
   double* Rr = Rall[warp];
-  if (row < rows) {
-    static_assert(NFWP_REC % 2 == 0 && NFW_NREC % 2 == 0, "record copy layout");
-    for (int i = lane; i < NFWP_REC / 2 + 3; i += 32) {
-      if (i < NFWP_REC / 2) cp_async16(Rr + 2 * i, prec + row * NFWP_REC + 2 * i);
-      else cp_async16(Rr + NFWP_REC + 2 * (i - NFWP_REC / 2), rec48 + row * NFW_NREC + 42 + 2 * (i - NFWP_REC / 2));
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  }
+  const double* src = rec + min(row, rows - 1) * NFW_REC;   // a warp past the last row copies that row, then returns
+  for (int i = lane; i < NFW_REC / 2; i += 32) cp_async16(Rr + 2 * i, src + 2 * i);
+  asm volatile("cp.async.commit_group;" ::: "memory");
   nfwp_tables_init(T, tid);
   const int nchunks = (nk + NFW_CH - 1) / NFW_CH;
   const bool cmm_sm = nchunks <= NFWP_MAXCH;
@@ -435,7 +336,7 @@ __global__ void __launch_bounds__(NFW_T, HMV_NFWP_MINB) uk_nfw_poly_kernel(long 
 }
 
 int nfw_poly_records(long long rows, int nm, int nkmax, const double* kmax_d, const double* zs_d, const double* cs_d,
-                     const double* rvir_d, double* rec48, double* prec, cudaStream_t st) {
+                     const double* rvir_d, double* rec, cudaStream_t st) {
   int dev = 0, nsm = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
@@ -443,7 +344,7 @@ int nfw_poly_records(long long rows, int nm, int nkmax, const double* kmax_d, co
   if (e != cudaSuccess) return fail(HMV_E_CUDA, "nfw_poly_records: %s", cudaGetErrorString(e));
   const long long ngroups = (rows + 15) / 16;
   const int grid = (int)((ngroups + 7) / 8 < nsm ? (ngroups + 7) / 8 : nsm);
-  nfw_poly_gemm_kernel<<<grid, 256, NFWP_GEMM_SMEM, st>>>(rows, nm, nkmax, kmax_d, zs_d, cs_d, rvir_d, rec48, prec);
+  nfw_poly_gemm_kernel<<<grid, 256, NFWP_GEMM_SMEM, st>>>(rows, nm, nkmax, kmax_d, zs_d, cs_d, rvir_d, rec);
   return check_launch("nfw_poly_gemm_kernel");
 }
 
@@ -456,19 +357,17 @@ __global__ void sici_test_kernel(int n, const double* __restrict__ x, double* __
 }  // namespace hmv
 using namespace hmv;
 
-static int g_nfw_mode = 0;   // 0: piecewise polynomials (default); 1: Maclaurin series + Si/Ci tail
-
 extern "C" int hmv_set_nfw_mode(int mode) {
-  HMV_REQUIRE(mode == 0 || mode == 1, "hmv_set_nfw_mode: mode must be 0 (piecewise polynomials) or 1 (series + Si/Ci)");
-  g_nfw_mode = mode;
+  HMV_REQUIRE(mode == 0, "hmv_set_nfw_mode: mode %d does not exist; 0 (piecewise polynomials) is the only evaluation "
+              "(the series + Si/Ci path, mode 1, was removed)", mode);
   return HMV_OK;
 }
 
 extern "C" long long hmv_uk_nfw_ws_doubles(int nz, int nm, int nk) {
   if (nz <= 0 || nm <= 0 || nk <= 0) return 0;
-  // per-halo series records and polynomial records, per-chunk min(k) and max(k), padded copies of k and k^2
+  // per-halo records, per-chunk min(k) and max(k), padded copies of k and k^2
   const long long nchunks = (nk + NFW_CH - 1) / NFW_CH;
-  return (long long)nz * nm * (NFW_NREC + NFWP_REC) + 2 * nchunks + 2 * nchunks * NFW_CH + 4;
+  return (long long)nz * nm * NFW_REC + 2 * nchunks + 2 * nchunks * NFW_CH + 4;
 }
 
 extern "C" int hmv_uk_nfw(int nz, int nm, int nk, int ldk, const double* zs_d, const double* ks_d,
@@ -476,35 +375,25 @@ extern "C" int hmv_uk_nfw(int nz, int nm, int nk, int ldk, const double* zs_d, c
                           void* stream) {
   HMV_REQUIRE(nz > 0 && nm > 0 && nk > 0 && ldk >= nk, "hmv_uk_nfw: bad sizes (nz=%d nm=%d nk=%d ldk=%d)", nz, nm, nk, ldk);
   HMV_REQUIRE(zs_d && ks_d && cs_d && rvir_d && ws_d && uk_d, "hmv_uk_nfw: null pointer");
+  // the kernels move 16-byte words: an even row stride and 16-byte aligned rows and workspace
+  HMV_REQUIRE((ldk & 1) == 0 && (((size_t)uk_d | (size_t)ws_d) & 15) == 0,
+              "hmv_uk_nfw: uk_d and ws_d must be 16-byte aligned and ldk even (ldk=%d)", ldk);
   const long long rows = (long long)nz * nm;
   if (rows > 2147483647LL) return fail(HMV_E_LIMIT, "hmv_uk_nfw: %lld halo rows exceed the 2^31-1 grid limit", rows);
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = HMV_OK;
   const int nchunks = (nk + NFW_CH - 1) / NFW_CH;
-  // the polynomial path moves 16-byte words: it needs an even row stride and 16-byte aligned rows and workspace
-  if (g_nfw_mode == 0 && (ldk & 1) == 0 && (((size_t)uk_d | (size_t)ws_d) & 15) == 0) {
-    double* prec = ws_d + rows * NFW_NREC;              // NFW_NREC and NFWP_REC are even: still 16-byte aligned
-    double* ksp = prec + rows * NFWP_REC;
-    double* k2p = ksp + (size_t)nchunks * NFW_CH;
-    double* kcmin = k2p + (size_t)nchunks * NFW_CH;
-    double* kcmx = kcmin + nchunks;
-    nfw_chunk_kernel<<<nchunks, 32, 0, st>>>(nk, ks_d, kcmin, kcmx, ksp, k2p);
-    rc = check_launch("nfw_chunk_kernel");
-    if (rc) return rc;
-    rc = nfw_poly_records(rows, nm, nchunks, kcmx, zs_d, cs_d, rvir_d, ws_d, prec, st);
-    if (rc) return rc;
-    uk_nfw_poly_kernel<<<cdiv(rows, NFW_T / 32), NFW_T, 0, st>>>(rows, nk, ldk, ksp, k2p, ws_d, prec, kcmin, kcmx, uk_d);
-    return check_launch("uk_nfw_poly_kernel");
-  }
-  nfw_record_kernel<<<cdiv(rows, 128), 128, 0, st>>>(nz, nm, zs_d, cs_d, rvir_d, ws_d);
-  rc = check_launch("nfw_record_kernel");
+  double* rec = ws_d;                                    // NFW_REC is even: what follows stays 16-byte aligned
+  double* ksp = rec + rows * NFW_REC;
+  double* k2p = ksp + (size_t)nchunks * NFW_CH;
+  double* kcmin = k2p + (size_t)nchunks * NFW_CH;
+  double* kcmax = kcmin + nchunks;
+  nfw_chunk_kernel<<<nchunks, 32, 0, st>>>(nk, ks_d, kcmin, kcmax, ksp, k2p);
+  int rc = check_launch("nfw_chunk_kernel");
   if (rc) return rc;
-  double* kcmax = ws_d + rows * NFW_NREC;
-  nfw_chunkmax_kernel<<<nchunks, 32, 0, st>>>(nk, ks_d, kcmax);
-  rc = check_launch("nfw_chunkmax_kernel");
+  rc = nfw_poly_records(rows, nm, nchunks, kcmax, zs_d, cs_d, rvir_d, rec, st);
   if (rc) return rc;
-  uk_nfw_kernel<2><<<(unsigned)rows, NFW_T, 0, st>>>(nk, ldk, ks_d, ws_d, kcmax, kmax, uk_d);
-  return check_launch("uk_nfw_kernel<both>");
+  uk_nfw_poly_kernel<<<cdiv(rows, NFW_T / 32), NFW_T, 0, st>>>(rows, nk, ldk, ksp, k2p, rec, kcmin, kcmax, uk_d);
+  return check_launch("uk_nfw_poly_kernel");
 }
 
 // test hook: elementwise Si/Ci of the device routine (x > 0)

@@ -19,7 +19,6 @@
 #include <cstdlib>
 #include <initializer_list>
 #include "common.cuh"
-#include "nfw_device.cuh"
 #include "nfw_poly.cuh"
 
 namespace hmv {
@@ -745,11 +744,11 @@ __global__ void __launch_bounds__(OT_T, OT_MINB) power_one_tab_kernel(const OneT
 // ---------------------------------------------------------------------------------------------------------
 // Spectra-only fusion: the six spectra with the NFW matter profile evaluated IN the reduction instead of being read
 // from a cube.  u_NFW(k|M,z) is a function of s = k r_s c (1+z) given by piecewise polynomials (nfw_poly.cuh,
-// k_nfw.cu), so a per-halo record of FREC doubles -- the halo's NFWP_REC polynomial coefficients, then
+// k_nfw.cu), so a per-halo record of NFW_REC doubles -- the halo's NFWP_REC polynomial coefficients, then
 // {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0} -- replaces an 8*nk-byte cube row: the kernel streams only the electron
 // cube (half the HBM traffic of power_six_kernel and no 32 GB NFW store/reload) and spends the freed time in the FP64
 // pipe on the Horner chains.  Beyond the last polynomial interval (s > 64) u_NFW takes its closed form (Si/Ci).
-// Same ring as power_six_kernel; stage = SIX_R rows x (4 KB of u_e + 64 B coefficients + FREC doubles of NFW record).
+// Same ring as power_six_kernel; stage = SIX_R rows x (4 KB of u_e + 64 B coefficients + NFW_REC doubles of NFW record).
 // k tiles are the slow grid dimension, highest k first: the tiles that reach the closed form are scheduled first.
 // ---------------------------------------------------------------------------------------------------------
 // {min, max} of ks over [b*tile, (b+1)*tile) for each block b (one warp per block)
@@ -765,14 +764,12 @@ __global__ void tile_range_kernel(int nk, int tile, const double* __restrict__ k
   if (lane == 0) { tilek[2 * b] = mn; tilek[2 * b + 1] = mx; }
 }
 
-constexpr int FREC = NFWP_REC + 6;          // per-halo record of the fused kernel: polynomial coefficients, then
-                                            // {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0}
 constexpr int FSX_NST = 6;
-constexpr int FSX_STAGE_DOUBLES = SIX_R * SIX_K + SIX_R * 8 + SIX_R * FREC;
+constexpr int FSX_STAGE_DOUBLES = SIX_R * SIX_K + SIX_R * 8 + SIX_R * NFW_REC;
 
 struct FusedArgs {
   int nm, nk, ldk;
-  const double *ue, *coef, *rec48, *prec;
+  const double *ue, *coef, *rec;
   SixOut out;
 };
 
@@ -831,12 +828,11 @@ __global__ void __launch_bounds__(FSX_CT + 32, 1) power_six_nfw_kernel(const Fus
       const unsigned segb = (unsigned)segk * 8u;
       for (int it = 0; it < nit; ++it, ring.advance(slot)) {
         const int m0 = it * SIX_R, rows = min(SIX_R, a.nm - m0);
-        const RingStage st = ring.acquire<true>(slot, (unsigned)rows * (segb + 64u + FREC * 8u));
+        const RingStage st = ring.acquire<true>(slot, (unsigned)rows * (segb + 64u + NFW_REC * 8u));
         for (int r = 0; r < rows; ++r) {
           bulk_g2s(st.p + r * SIX_K, a.ue + (zrow + m0 + r) * (long long)a.ldk + k0, segb, st.full);
-          double* rr = st.p + SIX_R * SIX_K + SIX_R * 8 + r * FREC;
-          bulk_g2s(rr, a.prec + (zrow + m0 + r) * NFWP_REC, NFWP_REC * 8u, st.full);
-          bulk_g2s(rr + NFWP_REC, a.rec48 + (zrow + m0 + r) * NFW_NREC + 42, 48u, st.full);
+          double* rr = st.p + SIX_R * SIX_K + SIX_R * 8 + r * NFW_REC;
+          bulk_g2s(rr, a.rec + (zrow + m0 + r) * NFW_REC, NFW_REC * 8u, st.full);
         }
         bulk_g2s(st.p + SIX_R * SIX_K, a.coef + (zrow + m0) * 8, (unsigned)rows * 64u, st.full);
       }
@@ -853,9 +849,9 @@ __global__ void __launch_bounds__(FSX_CT + 32, 1) power_six_nfw_kernel(const Fus
     const double* cfs = st + SIX_R * SIX_K;
 #pragma unroll 1
     for (int r = 0; r < rows; r += 2) {
-      const double* r0 = recs + r * FREC;
+      const double* r0 = recs + r * NFW_REC;
       const bool two = r + 1 < rows;
-      const double* r1 = two ? r0 + FREC : r0;
+      const double* r1 = two ? r0 + NFW_REC : r0;
       double um0, um1;
       nfw_poly_pair(T, r0, r1, kk, um0, um1);
       six_fma(acc, six_coef(cfs + r * 8), um0, st[r * SIX_K + min(tid, segk - 1)]);
@@ -1075,7 +1071,7 @@ extern "C" int hmv_power_tab(int nz, int nm, int nk, const double* ms_d, const d
 
 extern "C" long long hmv_power_six_nfw_ws_doubles(int nz, int nm) {
   if (nz <= 0 || nm <= 0) return 0;
-  return (8LL + NFW_NREC + NFWP_REC) * nz * nm + 2LL * nz + 4;   // coefficient records + NFW records + zoff + max(ks)
+  return (8LL + NFW_REC) * nz * nm + 2LL * nz + 4;   // coefficient records + NFW records + zoff + max(ks)
 }
 
 extern "C" int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* zs_d, const double* ms_d,
@@ -1089,9 +1085,8 @@ extern "C" int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* 
   cudaStream_t st = (cudaStream_t)stream;
   const long long cs = (long long)nz * nm;
   double* coef = ws_d;
-  double* rec48 = ws_d + 8 * cs;
-  double* prec = rec48 + NFW_NREC * cs;
-  double* zoff = prec + NFWP_REC * cs;
+  double* rec = ws_d + 8 * cs;
+  double* zoff = rec + NFW_REC * cs;
   double* kmax_dev = zoff + 2 * nz + ((2 * nz) & 1);
   FusedArgs a;
   int rc = six_setup("hmv_power_six_nfw", nz, nm, nk, ldk, {ue_d}, ms_d, ks_d, nzm_d, bh_d, Pzk_d, rho_m0, kstar, Nc_d,
@@ -1100,9 +1095,9 @@ extern "C" int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* 
   tile_range_kernel<<<1, 32, 0, st>>>(nk, nk, ks_d, kmax_dev);          // {min, max} of ks
   rc = check_launch("tile_range_kernel");
   if (rc) return rc;
-  rc = nfw_poly_records(cs, nm, 1, kmax_dev + 1, zs_d, cs_d, rvir_d, rec48, prec, st);
+  rc = nfw_poly_records(cs, nm, 1, kmax_dev + 1, zs_d, cs_d, rvir_d, rec, st);
   if (rc) return rc;
-  a.nm = nm; a.nk = nk; a.ldk = ldk; a.ue = ue_d; a.coef = coef; a.rec48 = rec48; a.prec = prec;
+  a.nm = nm; a.nk = nk; a.ldk = ldk; a.ue = ue_d; a.coef = coef; a.rec = rec;
   const size_t smem = BulkRing::smem_bytes(FSX_NST, FSX_STAGE_DOUBLES);
   rc = smem_opt_in(power_six_nfw_kernel, "power_six_nfw_kernel", smem);
   if (rc) return rc;

@@ -1,12 +1,14 @@
 // nfw_poly.cuh -- device helpers of the piecewise-polynomial NFW evaluation shared by the cube kernel (k_nfw.cu) and
 // the fused spectra kernel (k_power.cu).  See k_nfw.cu for the method.
 #pragma once
-#include "nfw_device.cuh"
+#include "sici.cuh"
 
 namespace hmv {
 #include "nfw_poly_tables.inc"
 
 constexpr int NFWP_REC = NFWP_NI * NFWP_STRIDE;          // polynomial coefficients per halo
+constexpr int NFW_REC = NFWP_REC + 6;                    // per-halo record: the polynomial coefficients, then
+                                                         // {c, a = r_s (1+z), a c, ln(1+c), 1/m_c, 0}
 
 __device__ __forceinline__ int nfwp_interval(double s) {
   const int si = __double2int_rz(fmin(s, 1.0e6));
@@ -32,10 +34,9 @@ __device__ __forceinline__ int nfwp_lookup(const NfwpTables& T, double s) {
   return T.idx[min(__double2int_rz(s), 64)];            // the conversion saturates for huge s
 }
 
-// host: per-halo polynomial records prec[rows][NFWP_REC] and the constants {c, a, a c, ln(1+c), 1/m_c, 0} in slots
-// 42..47 of rec48[rows][48], from ONE tensor-core contraction (k_nfw.cu).  kmax_d: device scalar >= max(ks), or the
-// per-chunk maxima (nkmax entries).
+// host: per-halo records rec[rows][NFW_REC] from ONE tensor-core contraction (k_nfw.cu).  kmax_d: device scalar
+// >= max(ks), or the per-chunk maxima (nkmax entries).
 int nfw_poly_records(long long rows, int nm, int nkmax, const double* kmax_d, const double* zs_d, const double* cs_d,
-                     const double* rvir_d, double* rec48, double* prec, cudaStream_t st);
+                     const double* rvir_d, double* rec, cudaStream_t st);
 
 }  // namespace hmv

@@ -63,14 +63,16 @@ int hmv_mdelta(int nz, int nm, const double* ms_d, const double* cs_d, const dou
                const double* drho2_d, double* m2_d, void* stream);
 
 /* ---- a4: analytic NFW u(k|M,z)  (hmvec.py:346-353) --------------------------------------------------
- * ws_d: workspace of hmv_uk_nfw_ws_doubles() doubles (per-halo series and polynomial coefficients, see k_nfw.cu). */
+ * u is evaluated as per-halo piecewise polynomials in (x c)^2 up to x c = 64 and the closed form's asymptotic branch
+ * beyond; ks need not be sorted.  uk_d and ws_d must be 16-byte aligned and ldk even (HMV_E_ARG otherwise).
+ * ws_d: workspace of hmv_uk_nfw_ws_doubles() doubles (one record of 300 doubles per halo -- its polynomial coefficients
+ * and constants -- and per-256-wavenumber chunk bounds and padded copies of ks and ks^2, see k_nfw.cu). */
 long long hmv_uk_nfw_ws_doubles(int nz, int nm, int nk);
-/* Process-wide choice of the evaluation: 0 (default) = per-halo piecewise polynomials in (x c)^2 up to x c = 64 and the
- * closed form's asymptotic branch beyond; 1 = the earlier Maclaurin series up to x c = 16 + Si/Ci closed form (kept for
- * A/B measurements and as the cross-check of the polynomial tables).  Both agree to ~1e-11 of max|u|. */
+/* The analytic NFW profile has one evaluation, the piecewise polynomials.  Mode 0 selects it and is accepted for ABI
+ * stability; any other mode returns HMV_E_ARG. */
 int hmv_set_nfw_mode(int mode);
 int hmv_uk_nfw(int nz, int nm, int nk, int ldk, const double* zs_d, const double* ks_d,
-               double kmax /* used only by the series + Si/Ci mode (>= max(ks)); the default path reduces ks on the device */, const double* cs_d,
+               double kmax /* ignored: max(ks) is reduced on the device */, const double* cs_d,
                const double* rvir_d, double* ws_d, double* uk_d, void* stream);
 
 /* ---- a6: Battaglia GNFW per-halo shape parameters  (hmvec.py:215-249,278-316,800-802,856-860,918-927)

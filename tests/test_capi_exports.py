@@ -91,6 +91,31 @@ def test_k1_rejects_before_any_launch():
         assert rc == HMV_E_ARG and "16-byte aligned" in capi.last_error(), (what, rc, capi.last_error())
 
 
+def test_k2_rejects_before_any_launch():
+    """The analytic NFW profile has one evaluation, selected by mode 0 alone, and hmv_uk_nfw moves 16-byte words of
+    the cube and the workspace: an odd ldk or a misaligned cube or workspace is refused before the first launch (dummy
+    device pointers, no GPU), never routed to another kernel."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("dummy device pointers must never reach a launch on a GPU")
+    from hmvec_b200 import _capi as capi
+    L = capi.lib
+    assert L.hmv_set_nfw_mode(0) == 0
+    assert L.hmv_set_nfw_mode(1) == HMV_E_ARG
+    ptr = [ctypes.c_void_p(0x10000 + 0x100 * i) for i in range(6)]      # non-null, 16-byte aligned, never dereferenced
+    bad = ctypes.c_void_p(0x20008)                                       # misaligned
+    nz, nm, nk = 2, 40, 30
+    zs, ks, cs, rvir, ws, uk = ptr
+    calls = {
+        "odd ldk": lambda: L.hmv_uk_nfw(nz, nm, nk, 31, zs, ks, 1.0, cs, rvir, ws, uk, None),
+        "misaligned uk": lambda: L.hmv_uk_nfw(nz, nm, nk, 32, zs, ks, 1.0, cs, rvir, ws, bad, None),
+        "misaligned ws": lambda: L.hmv_uk_nfw(nz, nm, nk, 32, zs, ks, 1.0, cs, rvir, bad, uk, None),
+    }
+    for what, call in calls.items():
+        rc = call()
+        assert rc == HMV_E_ARG and "16-byte aligned" in capi.last_error(), (what, rc, capi.last_error())
+
+
 def test_no_cpu_fallback_in_product():
     """The product package must not import the oracle (or the reference) anywhere."""
     pkg = os.path.join(ROOT, "hmvec_b200")

@@ -19,6 +19,9 @@ ABI, so it is known which kernel ran, and the reference is a plain numpy reducti
   and the z tiles), and the whole result against a host W^2 @ sPzk (adds the top-hat window) at a pure rtol: every
   term is non-negative except the Cartwright correction of an even-length Simpson rule.
 * HOD occupations, ngal, b_g and the all-z bisection at nm around the 1024-thread CTA width.
+* K2, the analytic NFW cube (`hmv_uk_nfw`), against `oracle.hmvec_oracle.uk_nfw_analytic`, the reference's Si/Ci
+  closed form in float64 (2.3e-14 absolute from 40-digit mpmath for 0.6 <= c <= 25), at inputs chosen so that every
+  plan of the cube kernel runs (`_k2_plans` restates the kernel's choices and each case asserts the ones it is for).
 
 Largest error-to-bound ratios measured on one B200 (1000 W power limit); the tolerances below keep about 10x headroom
 over them and stay far below the effect of the faults these tests exist for (dropping the last mass row of the
@@ -33,7 +36,8 @@ random inputs moves the ratio to 0.3 - 1):
     sigma^2 against its own W^2 table 5.1e-15 -> rtol 5e-14; sigma^2 against the host window 3.0e-13 -> rtol 3e-12:
     the floor is the top-hat window's cancellation 3 (sin x - x cos x) / x^3 just above the Taylor switch x = 0.01
     (device and numpy sin / cos differ in the last bit, amplified by 1/x^2);
-    HOD occupations 4.2e-13 -> rtol 4e-12 (above the 1e-14 max floor of N_c ~ 0); ngal and b_g 4.2e-16 -> 5e-15.
+    HOD occupations 4.2e-13 -> rtol 4e-12 (above the 1e-14 max floor of N_c ~ 0); ngal and b_g 4.2e-16 -> 5e-15;
+    uk_nfw 3.5e-13 of the row's max|u| -> tau = 4e-12: the polynomials' truncation error, not rounding.
 The whole file runs in about 10 s and allocates under 0.4 GB of device memory.
 
 Also here: NaN in the cube padding columns [nk, ldk) must not reach any output; outputs are written between NaN
@@ -50,6 +54,7 @@ pytestmark = pytest.mark.gpu
 
 TAU_K5 = 7e-14          # power_six / power_pair / power_one / power_six_tab / power_tab
 TAU_NFW = 2e-11         # power_six_nfw against the hmv_uk_nfw cube (two evaluations of u_NFW)
+TAU_K2 = 4e-12          # hmv_uk_nfw against the Si/Ci closed form, as a fraction of the row's max|u|
 TOL_EXPAND = 2e-15      # hmv_profile_expand against np.interp, as a fraction of the row's max|u|
 RTOL_SIGMA2_GEMM = 5e-14
 RTOL_SIGMA2 = 3e-12
@@ -645,3 +650,97 @@ def test_hod_around_cta_width(env, nm):
     torch.cuda.synchronize()
     assert int(iters[0]) == it_want
     assert_close(res.host((zs.size,))[0], l10_want, 1e-12, name="log10mthresh nm=%d" % nm)
+
+
+# ------------------------------------------------------------------------------------------------- K2: the NFW cube
+NFWP_HI = 1.005 * np.array([1, 2, 4, 6, 8, 10, 12, 14, 16, 20, 24, 28, 32, 36, 40, 44, 48, 52, 56, 60, 64.0])
+NFWP_NI, NFW_CH = 21, 256
+
+
+def _nfwp_interval(s):
+    """nfwp_interval of nfw_poly.cuh: the polynomial interval of s = x c (NFWP_NI: beyond s = 64)."""
+    si = np.floor(np.minimum(s, 1e6)).astype(np.int64)
+    return np.where(si < 1, 0, np.where(si < 2, 1, np.where(si < 16, 1 + (si >> 1),
+                                                            np.where(si < 64, 5 + (si >> 2), NFWP_NI))))
+
+
+def _k2_plans(ks, sr, xr):
+    """The plans uk_nfw_poly_kernel takes (k_nfw.cu restated) over all halo rows, s = k sr and x = k xr per row:
+    the leading run below s = 1 (fast), a chunk inside one interval (one), a chunk over several (several) with pairs
+    that straddle an edge or reach s = 64 (redo), whole chunks beyond s = 64 with every x > 4 (far) or some x <= 4
+    (near)."""
+    nch = -(-ks.size // NFW_CH)
+    kp = np.concatenate([ks, np.full(nch * NFW_CH - ks.size, ks[-1])]).reshape(nch, NFW_CH)  # as nfw_chunk_kernel pads
+    kmin, kmax = kp.min(axis=1), kp.max(axis=1)
+    sr, xr = sr.ravel()[:, None], xr.ravel()[:, None]
+    smin, smax = kmin * sr, kmax * sr
+    fast = np.cumprod((smax < NFWP_HI[0]) & (np.arange(nch) < nch - 1), axis=1).astype(bool)
+    beyond = ~fast & (smin >= 64.0)
+    iv = _nfwp_interval(smin)
+    one = ~fast & ~beyond & (smax < NFWP_HI[np.minimum(iv, NFWP_NI - 1)])
+    several = ~fast & ~beyond & ~one
+    pairs = kp.reshape(nch, NFW_CH // 2, 2)
+    plo, phi = pairs.min(axis=2)[None] * sr[..., None], pairs.max(axis=2)[None] * sr[..., None]
+    ivp = _nfwp_interval(plo)
+    redo = several & ((phi >= NFWP_HI[np.minimum(ivp, NFWP_NI - 1)]) | (ivp >= NFWP_NI)).any(axis=2)
+    return {name for name, hit in (("fast", fast), ("one", one), ("several", several), ("redo", redo),
+                                   ("far", beyond & (kmin * xr > 4.0)), ("near", beyond & (kmin * xr <= 4.0)))
+            if hit.any()}
+
+
+def _k2_inputs(case, nsm):
+    """(zs, cs, rvir, ks, plans the case must take).  c spans [0.6, 25] with both ends in every case."""
+    rng = np.random.default_rng(len(case))
+    if case == "sorted":                # every in-row plan, 37 masses: 111 rows, not a multiple of the 8 per CTA;
+        zs, nm = np.array([0.0, 0.7, 3.0]), 37      # c >= 16 at s >= 64 gives whole chunks with x <= 4 (near)
+        ks, plans = np.geomspace(1e-4, 300.0, 4097), {"fast", "one", "several", "redo", "far", "near"}
+    elif case == "shuffled":            # unsorted ks: every chunk spans many intervals, pairs straddle edges
+        zs, nm = np.array([0.3, 2.0]), 21
+        ks, plans = rng.permutation(np.geomspace(1e-3, 100.0, 515)), {"several", "redo"}
+    elif case == "partial":             # nk < 256: one partial chunk, the general loop only
+        zs, nm = np.array([0.5]), 16
+        ks, plans = np.geomspace(1e-2, 5.0, 200), {"one", "several"}
+    elif case == "global":              # 129 chunks > 128: chunk bounds read from global memory, in every plan
+        zs, nm = np.array([0.1]), 5
+        ks, plans = np.geomspace(1e-4, 100.0, 33001), {"fast", "one", "several", "redo", "far"}
+    elif case == "global_shuffled":
+        zs, nm = np.array([1.0]), 5
+        ks, plans = rng.permutation(np.geomspace(1e-4, 100.0, 33001)), {"several", "redo"}
+    else:                               # "gridstride": more rows than nfw_poly_gemm_kernel's grid covers in one
+        zs, nm = np.array([0.2, 1.5]), 64 * nsm + 37        # pass (16 rows x 8 warps x SM count)
+        ks, plans = np.geomspace(1e-3, 30.0, 33), set()
+    nz = zs.size
+    cs = np.stack([rng.permutation(np.linspace(0.6, 25.0, nm)) for _ in range(nz)])
+    rv = np.broadcast_to(np.geomspace(0.05, 3.0, nm), (nz, nm)).copy()
+    return zs, cs, rv, ks, plans
+
+
+@pytest.mark.parametrize("case", ["sorted", "shuffled", "partial", "global", "global_shuffled", "gridstride"])
+def test_k2_uk_nfw_plans(env, case):
+    """hmv_uk_nfw (chunk pre-pass, tensor-core record pre-pass, cube kernel) against the float64 Si/Ci closed form
+    of the same halos, in every plan of the cube kernel; every case has odd nk or padding columns [nk, ldk)."""
+    torch, capi, orc = env
+    nsm = torch.cuda.get_device_properties(0).multi_processor_count
+    zs, cs, rv, ks, plans = _k2_inputs(case, nsm)
+    nz, nm, nk = cs.shape[0], cs.shape[1], ks.size
+    sr = rv * (1.0 + zs[:, None])                   # s = k r_vir (1+z),  x = s / c
+    assert plans <= _k2_plans(ks, sr, sr / cs), case
+    nch = -(-nk // NFW_CH)
+    assert {"partial": nch == 1 and nk < NFW_CH, "global": nch > 128, "global_shuffled": nch > 128,
+            "gridstride": nz * nm > 16 * 8 * nsm and (nz * nm) % 8 != 0}.get(case, True)
+    ldk = _ldk(nk)
+    assert ldk > nk
+    out = Out(torch, 1, nz * nm * ldk)
+    out.poison[GUARD:GUARD + nz * nm * ldk].reshape(nz * nm, ldk)[:, nk:] = True     # NaN padding must survive
+    dz, dk, dc, dr = (_dev(torch, a) for a in (zs, ks, cs, rv))
+    L, p = capi.lib, capi.ptr
+    ws = torch.empty(int(L.hmv_uk_nfw_ws_doubles(nz, nm, nk)), dtype=torch.float64, device="cuda")
+
+    def launch():
+        capi.check(L.hmv_uk_nfw(nz, nm, nk, ldk, p(dz), p(dk), float(ks.max()), p(dc), p(dr), p(ws), out.ptr,
+                                capi.stream()), "hmv_uk_nfw")
+    _twice(torch, launch, (out,))
+    got = out.host((nz, nm, ldk))[0][..., :nk]
+    want = orc.uk_nfw_analytic(ks, zs, cs, rv)
+    bound = np.broadcast_to(np.abs(want).max(axis=-1, keepdims=True), want.shape)       # max|u| of the row (= 1)
+    _assert_bound("uk_nfw", "uk_nfw " + case, got, want, bound, TAU_K2)

@@ -155,24 +155,6 @@ def test_transform_table_mode_and_fused_six():
         assert_close(p2[i].cpu().numpy(), g2[tag], 1e-12, name="P2h_" + tag)
 
 
-def test_nfw_polynomial_and_series_paths_agree(hm):
-    """The two evaluations of the analytic NFW profile (piecewise polynomials with the tensor-core pre-pass, the
-    default; Maclaurin series + Si/Ci) against each other and on an unsorted wavenumber axis."""
-    from hmvec_b200 import _capi as capi
-    zs = np.array([0.0, 0.7, 3.0]); ms = np.geomspace(1e10, 1e16, 37)
-    rng = np.random.default_rng(5)
-    for ks in (np.geomspace(1e-4, 300., 1001), rng.permutation(np.geomspace(1e-3, 100., 515))):
-        cubes = []
-        for mode in (1, 0):
-            capi.check(capi.lib.hmv_set_nfw_mode(mode), "hmv_set_nfw_mode")
-            try:
-                h = hm.HaloModel(zs, ks, ms=ms, accuracy='low')
-                cubes.append(h.uk_profiles['nfw'])
-            finally:
-                capi.lib.hmv_set_nfw_mode(0)
-        assert_close(cubes[1], cubes[0], 1e-9, 2e-11, name="uk_nfw poly vs series")
-
-
 def test_eh98_on_the_device(hm):
     """hmv_eh98_factor (Eisenstein & Hu 1998 on the device, both the oscillating and the no-wiggle form) against the
     host-side factors, which tests/test_host_logic.py pins to the reference's Tk / P_lin_approx."""
