@@ -10,6 +10,8 @@
 //   power_prep_kernel      coefficient records of a tracer pair (hmv_power, hmv_power_tab)
 //   power_pair_kernel      any tracer pair (matter / HOD / pressure), up to four distinct cubes
 //   power_one_kernel       a pair whose two legs read the same single cube and no central-profile cube
+//   power_resp_prep_kernel, power_one_resp_kernel, power_pair_resp_kernel
+//                          the same bodies with the response's records and epilogue (hmv_power_response, DESIGN.md §4.5)
 //   power_six_prep_kernel  coefficient records of the six spectra (hmv_power_six, _six_tab, _six_nfw)
 //   power_six_kernel       {mm, ee, me, gg, gm, ge} in one pass over two cubes
 //   power_six_tab_kernel   the same with the electron profile interpolated from its bin tables
@@ -18,6 +20,7 @@
 //   power_six_nfw_kernel   the six spectra with the NFW profile evaluated in-kernel (spectra-only fusion)
 #include <cstdlib>
 #include <initializer_list>
+#include <math_constants.h>
 #include "common.cuh"
 #include "nfw_poly.cuh"
 
@@ -52,11 +55,13 @@ __device__ __forceinline__ void leg_coeffs(const TracerArgs& t, int z, long long
   }
 }
 
-__global__ void __launch_bounds__(256) power_prep_kernel(int nm, const double* __restrict__ ms,
-                                                          const double* __restrict__ nzm,
-                                                          const double* __restrict__ bh, double rho_m0,
-                                                          TracerArgs A, TracerArgs B, int form,
-                                                          double* __restrict__ coef, double* __restrict__ zoff) {
+// kResp: the records of the response to a long mode (hmv_power_response): c4 = w2, so that the 1-halo sum of the
+// consumers is R1h = sum_m w n b t_A t_B.  Only form 0 occurs there.
+template <bool kResp>
+__device__ __forceinline__ void power_prep_body(int nm, const double* __restrict__ ms, const double* __restrict__ nzm,
+                                                const double* __restrict__ bh, double rho_m0, TracerArgs A,
+                                                TracerArgs B, int form, double* __restrict__ coef,
+                                                double* __restrict__ zoff) {
   __shared__ double red[32];
   const int z = blockIdx.x;
   double cA = 0.0, cB = 0.0, gA = 0.0, gB = 0.0;
@@ -67,8 +72,8 @@ __global__ void __launch_bounds__(256) power_prep_kernel(int nm, const double* _
     double aA, bA, tA0, aB, bB, tB0;
     leg_coeffs(A, z, i, mu, aA, bA, tA0);
     leg_coeffs(B, z, i, mu, aB, bB, tB0);
-    double c4 = w1, c6 = 0.0;
-    if (form == 1) {            // hmvec.py:477-479
+    double c4 = kResp ? w2 : w1, c6 = 0.0;
+    if (!kResp && form == 1) {            // hmvec.py:477-479
       const double ig = 1.0 / A.ngal[z], ig2 = ig * ig;
       c4 = w1 * 2.0 * A.NcNs[i] * ig2;
       c6 = w1 * A.NsNsm1[i] * ig2;
@@ -94,6 +99,22 @@ __global__ void __launch_bounds__(256) power_prep_kernel(int nm, const double* _
   }
 }
 
+__global__ void __launch_bounds__(256) power_prep_kernel(int nm, const double* __restrict__ ms,
+                                                          const double* __restrict__ nzm,
+                                                          const double* __restrict__ bh, double rho_m0,
+                                                          TracerArgs A, TracerArgs B, int form,
+                                                          double* __restrict__ coef, double* __restrict__ zoff) {
+  power_prep_body<false>(nm, ms, nzm, bh, rho_m0, A, B, form, coef, zoff);
+}
+
+__global__ void __launch_bounds__(256) power_resp_prep_kernel(int nm, const double* __restrict__ ms,
+                                                               const double* __restrict__ nzm,
+                                                               const double* __restrict__ bh, double rho_m0,
+                                                               TracerArgs A, TracerArgs B,
+                                                               double* __restrict__ coef, double* __restrict__ zoff) {
+  power_prep_body<true>(nm, ms, nzm, bh, rho_m0, A, B, 0, coef, zoff);
+}
+
 // Generic tracer pair on the same ring as power_six_kernel: up to four distinct cubes (us_A, uc_A, us_B, uc_B,
 // de-duplicated by pointer) are streamed once; a stage holds PR_R rows of every cube plus the rows' 64-byte records.
 constexpr int PR_K = 512, PR_R = 4, PR_CT = 256;
@@ -115,7 +136,42 @@ __device__ __forceinline__ void pair_epilogue(const PairArgs& a, int z, int k, d
   if (a.p2h) a.p2h[o] = a.Pzk[o] * (iA + a.zoff[2 * z]) * (iB + a.zoff[2 * z + 1]);
 }
 
-__global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArgs a) {
+// n_eff = d ln P_lin / d ln k at column k of the row P (nk >= 2), as np.gradient(np.log(P), np.log(ks)): the
+// second-order stencil of a non-uniform grid inside, first-order one-sided differences at both ends.  A P that is not
+// positive at the column or at a neighbour the stencil reads gives NaN.
+__device__ __forceinline__ double n_eff(const double* __restrict__ ks, const double* __restrict__ P, int nk, int k) {
+  const int lo = k > 0 ? k - 1 : 0, hi = k < nk - 1 ? k + 1 : nk - 1;
+  const double Pl = P[lo], Pc = P[k], Ph = P[hi];
+  if (!(Pl > 0.0 && Pc > 0.0 && Ph > 0.0)) return CUDART_NAN;
+  const double xl = log(ks[lo]), xc = log(ks[k]), xh = log(ks[hi]);
+  const double fl = log(Pl), fc = log(Pc), fh = log(Ph);
+  if (k == 0) return (fh - fc) / (xh - xc);
+  if (k == nk - 1) return (fc - fl) / (xc - xl);
+  const double d1 = xc - xl, d2 = xh - xc;
+  return -d2 / (d1 * (d1 + d2)) * fl + (d2 - d1) / (d1 * d2) * fc + d1 / (d2 * (d1 + d2)) * fh;
+}
+
+// The response of one (z, k) to a long-wavelength mode (hmv_power_response): R1h = the 1-halo sum of the response
+// records (c4 = w2, no damping) into p1h, R2h = (47/21 - n_eff/3) P_lin (I_A + b_A - C_A)(I_B + b_B - C_B) into p2h.
+__device__ __forceinline__ void response_epilogue(const PairArgs& a, int z, int k, double p1, double iA, double iB) {
+  const long long o = (long long)z * a.nk + k;
+  if (a.p1h) a.p1h[o] = p1;
+  if (a.p2h) {
+    const double P2h = a.Pzk[o] * (iA + a.zoff[2 * z]) * (iB + a.zoff[2 * z + 1]);
+    a.p2h[o] = (47.0 / 21.0 - n_eff(a.ks, a.Pzk + (long long)z * a.nk, a.nk, k) / 3.0) * P2h;
+  }
+}
+
+// the epilogue of the two streaming bodies: the spectra (hmv_power) or the response (hmv_power_response)
+template <bool kResp>
+__device__ __forceinline__ void pair_out(const PairArgs& a, int z, int k, double p1, double iA, double iB) {
+  if (kResp) response_epilogue(a, z, k, p1, iA, iB);
+  else pair_epilogue(a, z, k, p1, iA, iB);
+}
+
+template <bool kResp>
+__device__ __forceinline__ void power_pair_body(const PairArgs a) {
+  __builtin_assume(threadIdx.x < PR_CT + 32);            // the kernels' launch bounds, which the body does not see
   extern __shared__ __align__(128) unsigned char pair_smem[];
   const BulkRing ring(pair_smem, a.nst, a.ncube * PR_R * PR_K + PR_R * 8, PR_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -180,9 +236,12 @@ __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArg
   for (int e = 0; e < 2; ++e) {
     const int k = k0 + 2 * tid + e;
     if (k >= a.nk) break;
-    pair_epilogue(a, z, k, e ? p1.y : p1.x, e ? iA.y : iA.x, e ? iB.y : iB.x);
+    pair_out<kResp>(a, z, k, e ? p1.y : p1.x, e ? iA.y : iA.x, e ? iB.y : iB.x);
   }
 }
+
+__global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArgs a) { power_pair_body<false>(a); }
+__global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_resp_kernel(const PairArgs a) { power_pair_body<true>(a); }
 
 // Tracer pairs whose two legs read the SAME single cube and have no central-profile cube (mm, ee, yy autos; galaxies x
 // their own satellite profile): t_A = aA + bA u, t_B = aB + bB u.  Same ring as power_pair_kernel, but a thread owns
@@ -192,7 +251,9 @@ __global__ void __launch_bounds__(PR_CT + 32, 1) power_pair_kernel(const PairArg
 constexpr int ONE_K = 1024, ONE_R = 4, ONE_NST = 5, ONE_CT = 256;
 constexpr int ONE_STAGE_DOUBLES = ONE_R * ONE_K + ONE_R * 8;
 
-__global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArgs a) {
+template <bool kResp>
+__device__ __forceinline__ void power_one_body(const PairArgs a) {
+  __builtin_assume(threadIdx.x < ONE_CT + 32);           // the kernels' launch bounds, which the body does not see
   extern __shared__ __align__(128) unsigned char one_smem[];
   const BulkRing ring(one_smem, ONE_NST, ONE_STAGE_DOUBLES, ONE_CT / 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -249,9 +310,12 @@ __global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArg
   for (int e = 0; e < 4; ++e) {
     const int k = k0 + (e >> 1) * 512 + 2 * tid + (e & 1);
     if (k >= a.nk || (e < 2 ? !act0 : !act1)) continue;
-    pair_epilogue(a, z, k, p1[e], iA[e], iB[e]);
+    pair_out<kResp>(a, z, k, p1[e], iA[e], iB[e]);
   }
 }
+
+__global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_kernel(const PairArgs a) { power_one_body<false>(a); }
+__global__ void __launch_bounds__(ONE_CT + 32, 1) power_one_resp_kernel(const PairArgs a) { power_one_body<true>(a); }
 
 // ---------------------------------------------------------------------------------------------------------
 // six spectra {mm, ee, me, gg, gm, ge} in one pass over (u_m, u_e); HOD satellites follow u_m, centrals u_c = 1
@@ -984,6 +1048,53 @@ extern "C" int hmv_power(int nz, int nm, int nk, int ldk, const double* ms_d, co
     if (!p2h_d) return HMV_OK;
   }
   return launch(A->us_d, A->uc_d, B->us_d, B->uc_d, a);
+}
+
+extern "C" int hmv_power_response(int nz, int nm, int nk, int ldk, const double* ms_d, const double* ks_d,
+                                  const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0,
+                                  const double* uA_d, int kindA, const double* uB_d, int kindB, double* ws_d,
+                                  double* r1h_d, double* r2h_d, void* stream) {
+  const char* fn = "hmv_power_response";
+  HMV_REQUIRE(nz >= 1 && nm >= 1 && nk >= 2, "%s: sizes must be >= 1 and nk >= 2 (nz=%d nm=%d nk=%d)", fn, nz, nm, nk);
+  HMV_REQUIRE(ldk >= nk && (ldk & 1) == 0, "%s: ldk must be even and >= nk (ldk=%d nk=%d)", fn, ldk, nk);
+  HMV_REQUIRE(ms_d && ks_d && nzm_d && bh_d && Pzk_d && uA_d && uB_d && ws_d, "%s: null pointer", fn);
+  HMV_REQUIRE(r1h_d || r2h_d, "%s: null pointer (r1h and r2h are both NULL)", fn);
+  HMV_REQUIRE(kindA == 0 || kindA == 2, "%s: cube A: kind %d is neither 0 (matter) nor 2 (pressure)", fn, kindA);
+  HMV_REQUIRE(kindB == 0 || kindB == 2, "%s: cube B: kind %d is neither 0 (matter) nor 2 (pressure)", fn, kindB);
+  HMV_REQUIRE(aligned16(uA_d), "%s: cube A must be 16-byte aligned", fn);
+  HMV_REQUIRE(aligned16(uB_d), "%s: cube B must be 16-byte aligned", fn);
+  HMV_REQUIRE(aligned16(ws_d), "%s: workspace must be 16-byte aligned", fn);
+  if (nz > 65535) return fail(HMV_E_LIMIT, "%s: nz=%d exceeds 65535 (grid y of the streaming kernel)", fn, nz);
+  cudaStream_t st = (cudaStream_t)stream;
+  double* coef = ws_d;
+  double* zoff = ws_d + 8LL * nz * nm;
+  TracerArgs ta, tb;
+  ta.kind = kindA; tb.kind = kindB;
+  ta.Nc = ta.Ns = ta.NcNs = ta.NsNsm1 = ta.ngal = ta.bias = nullptr;
+  tb.Nc = tb.Ns = tb.NcNs = tb.NsNsm1 = tb.ngal = tb.bias = nullptr;
+  PairArgs a;
+  a.nm = nm; a.nk = nk; a.ldk = ldk; a.form = 0;
+  a.coef = coef; a.zoff = zoff; a.ks = ks_d; a.Pzk = Pzk_d; a.kstar = 0.0;
+  a.p1h = r1h_d; a.p2h = r2h_d;
+  a.cube[0] = uA_d; a.cube[1] = uB_d; a.cube[2] = a.cube[3] = nullptr;
+  a.rusA = 0; a.rusB = uB_d == uA_d ? 0 : 1; a.rucA = a.rucB = -1;
+  a.ncube = a.rusB + 1;
+  const int stage_doubles = a.ncube * PR_R * PR_K + PR_R * 8;
+  a.nst = a.ncube == 1 ? ONE_NST : (int)((200 * 1024) / (stage_doubles * sizeof(double)));
+  if (a.nst > 6) a.nst = 6;
+  const size_t smem = a.ncube == 1 ? BulkRing::smem_bytes(ONE_NST, ONE_STAGE_DOUBLES) : BulkRing::smem_bytes(a.nst, stage_doubles);
+  int rc = a.ncube == 1 ? smem_opt_in(power_one_resp_kernel, "power_one_resp_kernel", smem)
+                        : smem_opt_in(power_pair_resp_kernel, "power_pair_resp_kernel", smem);
+  if (rc) return rc;
+  power_resp_prep_kernel<<<nz, 256, 0, st>>>(nm, ms_d, nzm_d, bh_d, rho_m0, ta, tb, coef, zoff);
+  rc = check_launch("power_resp_prep_kernel");
+  if (rc) return rc;
+  if (a.ncube == 1) {             // one cube: power_one's body (t = a + b u folded into the records)
+    power_one_resp_kernel<<<dim3(cdiv(ldk, ONE_K), nz), ONE_CT + 32, smem, st>>>(a);
+    return check_launch("power_one_resp_kernel");
+  }
+  power_pair_resp_kernel<<<dim3(cdiv(ldk, PR_K), nz), PR_CT + 32, smem, st>>>(a);
+  return check_launch("power_pair_resp_kernel");
 }
 
 extern "C" int hmv_power_six(int nz, int nm, int nk, int ldk, const double* ms_d, const double* ks_d,

@@ -9,6 +9,7 @@
 // P2[K][l'] = t_C t_D at k2, and sigma2_gemm_kernel<MT, A K-major> forms C = P1^T P2 on the tensor pipe -- over all of
 // K with a fixed-order split-k reduction for the covariance, batched over z (K = m, one batch item per split index)
 // for the trispectrum.  A last kernel sums the splits in a fixed order and drops the padding column.
+// The super-sample covariance (DESIGN.md §4.5) reuses the projection with K = z; sigma_b^2 of a disc is here too.
 #include "common.cuh"
 #include "gemm_f64.cuh"
 
@@ -103,19 +104,19 @@ struct TrispecPlan {
   int nbatch;           // 1 (covariance) or nz (trispectrum)
 };
 
-static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2) {
+// output rows per CTA, padded widths and K = nz * rows_z of the contraction of an n1 x n2 result
+static TrispecPlan base_plan(int nz, int rows_z, int n1, int n2) {
   TrispecPlan p;
   p.mt = n1 <= 32 ? 4 : n1 <= 64 ? 8 : n1 <= 128 ? 16 : 26;
-  p.nmp = nm + (nm & 1);
+  p.nmp = rows_z;
   p.ld1 = n1 + (n1 & 1);
   p.ld2 = n2 + (n2 & 1);
   p.K = (long long)nz * p.nmp;
-  if (!proj) {                       // one batch item per redshift: its K range is its nmp mass rows
-    p.kchunk = p.nmp;
-    p.nsplit = 1;
-    p.nbatch = nz;
-    return p;
-  }
+  return p;
+}
+
+// The projection's split of K: fills kchunk, nsplit and nbatch = 1 of a plan whose mt, ld1, ld2 and K are set.
+static TrispecPlan split_k(TrispecPlan p, int n1) {
   // Split K so that the grid is about sixteen waves of resident CTAs (148 SMs; MT = 26 runs one CTA per SM): the last
   // wave is then a small fraction of the run.  CTAs are issued tile-fastest, so the resident ones walk the same K range
   // together and every panel row comes from HBM about once, the other tiles finding it in L2.  At least eight k
@@ -131,6 +132,17 @@ static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2) {
   p.nsplit = cdiv(p.K, p.kchunk);
   p.nbatch = 1;
   return p;
+}
+
+static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2) {
+  TrispecPlan p = base_plan(nz, nm + (nm & 1), n1, n2);
+  if (!proj) {                       // one batch item per redshift: its K range is its nmp mass rows
+    p.kchunk = p.nmp;
+    p.nsplit = 1;
+    p.nbatch = nz;
+    return p;
+  }
+  return split_k(p, n1);
 }
 
 static long long trispec_ws(const TrispecPlan& p, int n1) {
@@ -153,6 +165,25 @@ static cudaError_t trispec_gemm(const TrispecPlan& p, int n1, const double* P1, 
   sigma2_gemm_kernel<MT, true><<<grid, SG_T, smem, st>>>(n1, p.ld2, (int)p.K, p.kchunk, P1, P2, part,
                                                          (long long)n1 * p.ld2, p.ld1);
   return cudaSuccess;
+}
+
+// C = P1^T P2 of a plan's panels: the contraction into the split-k partial sums, then their fixed-order reduction into
+// out [nbatch][n1][n2] without the padding column
+static int trispec_contract(const char* who, const TrispecPlan& p, int n1, int n2, const double* P1, const double* P2,
+                            double* part, double* out_d, cudaStream_t st) {
+  cudaError_t e;
+  switch (p.mt) {
+    case 4: e = trispec_gemm<4>(p, n1, P1, P2, part, st); break;
+    case 8: e = trispec_gemm<8>(p, n1, P1, P2, part, st); break;
+    case 16: e = trispec_gemm<16>(p, n1, P1, P2, part, st); break;
+    default: e = trispec_gemm<26>(p, n1, P1, P2, part, st); break;
+  }
+  if (e != cudaSuccess) return fail(HMV_E_CUDA, "%s: sigma2_gemm_kernel smem opt-in: %s", who, cudaGetErrorString(e));
+  int rc = check_launch("sigma2_gemm_kernel<A K-major>");
+  if (rc) return rc;
+  const long long n = (long long)p.nbatch * n1 * n2;
+  trispec_reduce_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, p.nsplit, n1, n2, p.ld2, part, out_d);
+  return check_launch("trispec_reduce_kernel");
 }
 
 static int trispec_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
@@ -187,20 +218,74 @@ static int trispec_run(const char* who, bool proj, int nz, int nm, int nk, int l
                                             p.ld2, q2_d, zs_d, proj ? chis_d : nullptr, pref_d, P1, P2);
   int rc = check_launch("trispec_panel_kernel");
   if (rc) return rc;
-  cudaError_t e;
-  switch (p.mt) {
-    case 4: e = trispec_gemm<4>(p, n1, P1, P2, part, st); break;
-    case 8: e = trispec_gemm<8>(p, n1, P1, P2, part, st); break;
-    case 16: e = trispec_gemm<16>(p, n1, P1, P2, part, st); break;
-    default: e = trispec_gemm<26>(p, n1, P1, P2, part, st); break;
-  }
-  if (e != cudaSuccess) return fail(HMV_E_CUDA, "%s: sigma2_gemm_kernel smem opt-in: %s", who, cudaGetErrorString(e));
-  rc = check_launch("sigma2_gemm_kernel<A K-major>");
-  if (rc) return rc;
-  const long long n = (long long)p.nbatch * n1 * n2;
-  trispec_reduce_kernel<<<cdiv(n, 256), 256, 0, st>>>(n, p.nsplit, n1, n2, p.ld2, part, out_d);
-  return check_launch("trispec_reduce_kernel");
+  return trispec_contract(who, p, n1, n2, P1, P2, part, out_d, st);
 }
+
+
+// ---- super-sample covariance (DESIGN.md §4.5) -------------------------------------------------------------------------
+//   sigma_b^2(z)        = sum_j kw_j P[z][j] W(k_j R_z)^2,  W(x) = 2 J1(x)/x, kw_j = s_j k_j/(2 pi) from the caller
+//   Cov^{AB,CD}(l,l')   = sum_z zeta_z pref_z R^{AB}((l+1/2)/chi_z, z) R^{CD}((l'+1/2)/chi_z, z)
+// with pref = H^3 W_A W_B W_C W_D sigma_b^2/chi^4 from the caller and R linear in k on ks, clamped to its ends.  The
+// covariance is the trispectrum's contraction with K = z: one panel row per redshift.
+
+// 2 J1(x)/x, the Fourier transform of a disc; its Taylor series near x = 0 (error below 1e-16 for |x| < 1e-2)
+__device__ __forceinline__ double disc_window(double x) {
+  if (fabs(x) < 1e-2) {
+    const double x2 = x * x;
+    return fma(x2, fma(x2, 1.0 / 192.0, -1.0 / 8.0), 1.0);
+  }
+  return 2.0 * j1(x) / x;
+}
+
+// one CTA per redshift; a fixed-order block reduction, so repeated calls give identical results
+__global__ void __launch_bounds__(256) sigma_b2_kernel(int nks, const double* __restrict__ ks,
+                                                       const double* __restrict__ kw, const double* __restrict__ P,
+                                                       const double* __restrict__ R, double* __restrict__ out) {
+  __shared__ double red[32];
+  const int z = blockIdx.x;
+  const double Rz = R[z];
+  const double* Pz = P + (long long)z * nks;
+  double s = 0.0;
+  for (int j = threadIdx.x; j < nks; j += blockDim.x) {
+    const double W = disc_window(ks[j] * Rz);
+    s = fma(kw[j] * Pz[j], W * W, s);
+  }
+  s = block_sum(s, red);
+  if (threadIdx.x == 0) out[z] = s;
+}
+
+// P1[z][l] = zeta_z pref_z R^{AB}(z, (l+1/2)/chi_z), P2[z][l'] = R^{CD}(z, (l'+1/2)/chi_z); columns in [n, ld) are zero.
+// One thread per column and redshift: one interval search each.
+__global__ void __launch_bounds__(TP_T) ssc_panel_kernel(int nz, int nk, const double* __restrict__ ks,
+                                                         const double* __restrict__ rAB, const double* __restrict__ rCD,
+                                                         int n1, int ld1, const double* __restrict__ l1, int n2,
+                                                         int ld2, const double* __restrict__ l2,
+                                                         const double* __restrict__ zs, const double* __restrict__ chis,
+                                                         const double* __restrict__ pref, double* __restrict__ P1,
+                                                         double* __restrict__ P2) {
+  const int z = blockIdx.y, l = blockIdx.x * TP_T + threadIdx.x;
+  const double inv_chi = 1.0 / chis[z];
+  int j;
+  double f;
+  if (l < ld1) {
+    double v = 0.0;
+    if (l < n1) {
+      k_locate(ks, nk, (l1[l] + 0.5) * inv_chi, j, f);
+      v = pref[z] * (nz > 1 ? trapz_weight(zs, z, nz) : 1.0) * k_lerp(rAB + (long long)z * nk, j, f);
+    }
+    P1[(long long)z * ld1 + l] = v;
+  }
+  if (l < ld2) {
+    double v = 0.0;
+    if (l < n2) {
+      k_locate(ks, nk, (l2[l] + 0.5) * inv_chi, j, f);
+      v = k_lerp(rCD + (long long)z * nk, j, f);
+    }
+    P2[(long long)z * ld2 + l] = v;
+  }
+}
+
+static TrispecPlan ssc_plan(int nz, int n1, int n2) { return split_k(base_plan(nz, 1, n1, n2), n1); }
 
 }  // namespace hmv
 
@@ -228,4 +313,40 @@ extern "C" int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d
                              const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream) {
   return trispec_run("hmv_cl_cov_1h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, u_h, kind_h, nl1, ells1_d, nl2,
                      ells2_d, zs_d, chis_d, pref_d, ws_d, out_d, stream);
+}
+
+extern "C" int hmv_sigma_b2(int nz, int nks, const double* ks_d, const double* kw_d, const double* P_d,
+                            const double* R_d, double* out_d, void* stream) {
+  HMV_REQUIRE(nz >= 1 && nks >= 1, "hmv_sigma_b2: sizes must be >= 1 (nz=%d nks=%d)", nz, nks);
+  HMV_REQUIRE(ks_d && kw_d && P_d && R_d && out_d, "hmv_sigma_b2: null pointer");
+  sigma_b2_kernel<<<nz, 256, 0, (cudaStream_t)stream>>>(nks, ks_d, kw_d, P_d, R_d, out_d);
+  return check_launch("sigma_b2_kernel");
+}
+
+extern "C" long long hmv_cl_cov_ssc_ws_doubles(int nz, int nl1, int nl2) {
+  if (nz <= 0 || nl1 <= 0 || nl2 <= 0) return 0;
+  return trispec_ws(ssc_plan(nz, nl1, nl2), nl1);
+}
+
+extern "C" int hmv_cl_cov_ssc(int nz, int nk, const double* ks_d, const double* rAB_d, const double* rCD_d, int nl1,
+                              const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                              const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream) {
+  const char* who = "hmv_cl_cov_ssc";
+  HMV_REQUIRE(nz >= 1 && nk >= 2 && nl1 >= 1 && nl2 >= 1,
+              "%s: sizes must be >= 1 and nk >= 2 (nz=%d nk=%d n1=%d n2=%d)", who, nz, nk, nl1, nl2);
+  HMV_REQUIRE(ks_d && rAB_d && rCD_d && ells1_d && ells2_d && ws_d && out_d, "%s: null pointer", who);
+  HMV_REQUIRE(zs_d && chis_d && pref_d, "%s: null pointer (zs, chis or pref)", who);
+  HMV_REQUIRE(((size_t)ws_d & 15) == 0, "%s: workspace must be 16-byte aligned", who);
+  if (nz > 65535) return fail(HMV_E_LIMIT, "%s: nz=%d exceeds 65535 (grid y of the panel kernel)", who, nz);
+  const TrispecPlan p = ssc_plan(nz, nl1, nl2);
+  double* P1 = ws_d;
+  double* P2 = P1 + p.K * p.ld1;
+  double* part = P2 + p.K * p.ld2;
+  cudaStream_t st = (cudaStream_t)stream;
+  dim3 pg(cdiv(p.ld1 > p.ld2 ? p.ld1 : p.ld2, TP_T), nz);
+  ssc_panel_kernel<<<pg, TP_T, 0, st>>>(nz, nk, ks_d, rAB_d, rCD_d, nl1, p.ld1, ells1_d, nl2, p.ld2, ells2_d, zs_d,
+                                        chis_d, pref_d, P1, P2);
+  const int rc = check_launch("ssc_panel_kernel");
+  if (rc) return rc;
+  return trispec_contract(who, p, nl1, nl2, P1, P2, part, out_d, st);
 }

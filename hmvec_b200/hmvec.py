@@ -911,8 +911,9 @@ class HaloModel(Cosmology):
         return {t: h1[i] for i, t in enumerate(tags)}, {t: h2[i] for i, t in enumerate(tags)}
 
     # ------------------------------------------------------------------ 1-halo trispectrum and C_l covariance
-    def _trispec_legs(self, names):
-        """Device cubes and kinds of four profile tracers: matter profile first, then pressure profile.  A table-backed
+    def _trispec_legs(self, names, what="1-halo trispectrum",
+                      hod_why="needs occupation moments up to fourth order, which the HOD does not define"):
+        """Device cubes and kinds of profile tracers: matter profile first, then pressure profile.  A table-backed
         profile is expanded to its cube (DeviceCubes.device)."""
         cubes, kinds = [], []
         for n in names:
@@ -923,12 +924,11 @@ class HaloModel(Cosmology):
                 cubes.append(self.pk_profiles.device(n))
                 kinds.append(_KIND_PRESSURE)
             elif n in self.hods:
-                raise ValueError("%r is an HOD: its 1-halo trispectrum needs occupation moments up to fourth order, "
-                                 "which the HOD does not define" % (n,))
+                raise ValueError("%r is an HOD: its %s %s" % (n, what, hod_why))
             else:
                 raise ValueError("no matter or pressure profile named %r" % (n,))
         if not np.all(np.diff(self._ks64) > 0):
-            raise ValueError("the model's ks must be strictly increasing for the trispectrum's interpolation")
+            raise ValueError("the model's ks must be strictly increasing for the %s's interpolation" % what)
         return cubes, kinds
 
     @staticmethod
@@ -986,9 +986,23 @@ class HaloModel(Cosmology):
         name4 = name3 if name4 is None else name4
         l1 = self._positive(ells, "ells")
         l2 = l1 if ells2 is None else self._positive(ells2, "ells2")
+        fsky = self._fsky(fsky)
+        W = self._window_product(windows)
+        chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
+        H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
+        pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
+        extra = (self._zs_d, self._dev(chis), self._dev(pref))
+        return self._trispec_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+
+    @staticmethod
+    def _fsky(fsky):
         fsky = float(fsky)
         if not (0.0 < fsky <= 1.0):
             raise ValueError("fsky must lie in (0, 1]")
+        return fsky
+
+    def _window_product(self, windows):
+        """W_A W_B W_C W_D on self.zs; each window is a scalar or an [nz] array."""
         if len(windows) != 4:
             raise ValueError("windows must hold four entries (A, B, C, D)")
         W = np.ones(self._nz)
@@ -997,11 +1011,119 @@ class HaloModel(Cosmology):
             if w.ndim > 1 or (w.ndim == 1 and w.size != self._nz):
                 raise ValueError("each window must be a scalar or an array of length nz=%d" % self._nz)
             W = W * w
+        return W
+
+    # ------------------------------------------------------------------ super-sample covariance (DESIGN.md §4.5)
+    def _response_legs(self, names):
+        cubes, kinds = self._trispec_legs(names, "response", "needs the number-density term -(b_A + b_B) P, which is "
+                                                             "not part of the response of profile tracers")
+        if self._nk < 2:
+            raise ValueError("the response needs at least two wavenumbers (n_eff)")
+        return cubes, kinds
+
+    def _response_device(self, cubes, kinds):
+        """R1h + R2h of a pair of profile legs as a device tensor [nz, nk] (hmv_power_response)."""
+        nz, nm = self._nz, self._nm
+        ws = self._workspace('power', capi.lib.hmv_power_ws_doubles(nz, nm))
+        r1, r2 = self._empty(nz, self._nk), self._empty(nz, self._nk)
+        capi.check(capi.lib.hmv_power_response(nz, nm, self._nk, self._ldk, capi.ptr(self._ms_d), capi.ptr(self._ks_d),
+                                               capi.ptr(self._nzm_d), capi.ptr(self._bh_d), capi.ptr(self._Pzk_d),
+                                               self._rho_m0, capi.ptr(cubes[0]), kinds[0], capi.ptr(cubes[1]), kinds[1],
+                                               capi.ptr(ws), capi.ptr(r1), capi.ptr(r2), capi.stream()),
+                   "hmv_power_response")
+        capi.check(capi.lib.hmv_sum2(r1.numel(), capi.ptr(r1), capi.ptr(r2), capi.ptr(r1), capi.stream()), "hmv_sum2")
+        return r1
+
+    def get_power_response(self, name="nfw", name2=None):
+        """Response of P^{AB}(k, z) to a long-wavelength density mode, dP/d delta_b on self.ks, [nz, nk]:
+
+            R1h = sum_M w_M n(z,M) b(z,M) t_A(k) t_B(k)                (no 1-halo damping)
+            R2h = [47/21 - n_eff(z,k)/3] P2h^{AB}(k, z),   n_eff = d ln P_lin / d ln k
+
+        (Takada & Hu 2013, PRD 87, 123504).  No counterpart in the reference.  t as in get_trispectrum_1halo: (M/rho_m0) u
+        for a matter profile, u for a pressure profile; P2h is get_power_2halo's.  n_eff follows
+        np.gradient(np.log(Pzk), np.log(ks), axis=1); a P_lin that is not positive at a column or a neighbour gives NaN
+        there.  HODs raise ValueError.  On a z-sharded model: this rank's slab."""
+        name2 = name if name2 is None else name2
+        cubes, kinds = self._response_legs((name, name2))
+        return self._host(self._response_device(cubes, kinds))
+
+    def _sigma_b2_grid(self, fsky):
+        """Disc radius R_z = chi(z) theta_s (cos theta_s = 1 - 2 fsky), the k grid geomspace(k_b, sigma2_kmax,
+        sigma2_numks) with k_b = min(sigma2_kmin, 1e-3 / max_z R_z), and its weights simpson * k / (2 pi)."""
+        from .cosmology import simpson_weights
+        chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
+        R = chis * np.arccos(1.0 - 2.0 * fsky)
+        kb = float(self.p['sigma2_kmin'])
+        if R.max() > 0:
+            kb = min(kb, 1e-3 / R.max())
+        kg = np.geomspace(kb, self.p['sigma2_kmax'], int(self.p['sigma2_numks']))
+        return R, kg, simpson_weights(kg) * kg / (2.0 * np.pi)
+
+    def get_sigma_b2(self, fsky):
+        """Variance of the background density mode over a disc of area 4 pi fsky, flat sky, [nz]:
+
+            sigma_b^2(z) = 1/(2 pi) int dk k P_lin(k, z) [2 J1(k R_z) / (k R_z)]^2,   R_z = chi(z) theta_s
+
+        Simpson on geomspace(k_b, sigma2_kmax, sigma2_numks), k_b = min(sigma2_kmin, 1e-3 / max_z R_z); P_lin from the
+        producer of sPzk (accuracy 'low': EH98 on the device; otherwise P_lin / P_lin_slow).  The model's sPzk, sigma2
+        and mass function are not touched.  On a z-sharded model: this rank's slab (k_b from the slab's redshifts)."""
+        fsky = self._fsky(fsky)
+        R, kg, kw = self._sigma_b2_grid(fsky)
+        if self.accuracy == 'low':
+            P_d = self._plin_device(kg, self.zs)
+        elif self.accuracy == 'high':
+            P_d = self._dev(np.asarray(self.P_lin_slow(kg, self.zs, kmax=self.p['sigma2_kmax']), dtype=np.float64))
+        else:
+            P_d = self._dev(np.asarray(self.P_lin(kg, self.zs), dtype=np.float64))
+        out = self._empty(self._nz)
+        kg_d, kw_d, R_d = self._dev(kg), self._dev(kw), self._dev(R)
+        capi.check(capi.lib.hmv_sigma_b2(self._nz, kg.size, capi.ptr(kg_d), capi.ptr(kw_d), capi.ptr(P_d),
+                                         capi.ptr(R_d), capi.ptr(out), capi.stream()), "hmv_sigma_b2")
+        return self._host(out)
+
+    def get_cl_cov_ssc(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
+                       ells2=None, sigma_b2=None):
+        """Super-sample covariance Cov_SSC(C_l^{AB}, C_l'^{CD}), [len(ells), len(ells2)]:
+
+            sum_z zeta_z H^3 W_A W_B W_C W_D sigma_b^2(z) / chi^4 R^{AB}((l+1/2)/chi, z) R^{CD}((l'+1/2)/chi, z)
+
+        (Takada & Hu 2013; Li, Hu & Takada 2014), with R from get_power_response interpolated linearly in k on `ks` (k
+        clamped to the grid's ends), sigma_b^2 from get_sigma_b2(fsky) and the window convention of get_cl_cov_1halo.
+        fsky enters only through sigma_b^2.  sigma_b2: an optional [nz] array (e.g. from a mask's power spectrum) that
+        replaces the disc.  Names, windows, ells2 and the defaults behave as in get_cl_cov_1halo; HODs raise ValueError.
+        Not available on a z-sharded model (the z sum would need a cross-rank reduction)."""
+        if self._zcomm is not None:
+            raise NotImplementedError("get_cl_cov_ssc on a z-sharded model: the z sum spans the ranks")
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        l1 = self._positive(ells, "ells")
+        l2 = l1 if ells2 is None else self._positive(ells2, "ells2")
+        fsky = self._fsky(fsky)
+        W = self._window_product(windows)
+        if sigma_b2 is not None:
+            sb2 = np.array(sigma_b2, dtype=np.float64).reshape(-1)
+            if sb2.size != self._nz or not np.all(np.isfinite(sb2)) or np.any(sb2 < 0):
+                raise ValueError("sigma_b2 must hold nz=%d finite non-negative values" % self._nz)
+        legAB = self._response_legs((name, name2))
+        legCD = self._response_legs((name3, name4))
+        if sigma_b2 is None:
+            sb2 = self.get_sigma_b2(fsky)
         chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
         H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
-        pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
-        extra = (self._zs_d, self._dev(chis), self._dev(pref))
-        return self._trispec_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+        pref = H ** 3 * W * sb2 / chis ** 4
+        rAB = self._response_device(*legAB)
+        rCD = rAB if (name3, name4) == (name, name2) else self._response_device(*legCD)
+        nz = self._nz
+        ws = self._workspace('ssc', capi.lib.hmv_cl_cov_ssc_ws_doubles(nz, l1.size, l2.size))
+        out = self._empty(l1.size, l2.size)
+        l1_d, l2_d, chis_d, pref_d = self._dev(l1), self._dev(l2), self._dev(chis), self._dev(pref)
+        capi.check(capi.lib.hmv_cl_cov_ssc(nz, self._nk, capi.ptr(self._ks_d), capi.ptr(rAB), capi.ptr(rCD), l1.size,
+                                           capi.ptr(l1_d), l2.size, capi.ptr(l2_d), capi.ptr(self._zs_d),
+                                           capi.ptr(chis_d), capi.ptr(pref_d), capi.ptr(ws), capi.ptr(out),
+                                           capi.stream()), "hmv_cl_cov_ssc")
+        return self._host(out)
 
 
     # ------------------------------------------------------------------ cluster-lensing helper

@@ -312,6 +312,35 @@ int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const dou
                   const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d, double* ws_d,
                   double* out_d, void* stream);
 
+/* ---- super-sample covariance of C_l (matter and pressure profiles) ---------------------------------------------------
+ * No counterpart in the reference.  Takada & Hu 2013, PRD 87, 123504; Li, Hu & Takada 2014, PRD 89, 083519.  Legs t_X
+ * and kinds as in hmv_trispec_1h (0: matter, a = M/rho_m0; 2: pressure, a = 1); w_m the trapezoid weight on ms.
+ * hmv_power_response: the response of P^{AB}(k,z) to a long-wavelength mode, on ks (strictly increasing, nk >= 2):
+ *   r1h[z][k] = sum_m w_m n(z,m) b(z,m) t_A(z,m,k) t_B(z,m,k)                 (no 1-halo damping)
+ *   r2h[z][k] = [47/21 - n_eff(z,k)/3] P2h^{AB}(z,k)
+ * P2h is hmv_power's 2-halo term, P_lin (I_A + b_A - C_A)(I_B + b_B - C_B) (pressure: b = 0, no consistency term);
+ * n_eff = d ln P_lin/d ln k as np.gradient(log Pzk, log ks, axis=1): second-order non-uniform stencil inside,
+ * one-sided at the ends.  A Pzk that is not positive at a column or at a neighbour the stencil reads gives NaN there.
+ * One pass over the cube (uA_d == uB_d) or the two cubes, as hmv_power's power_one / power_pair.  r1h_d or r2h_d may
+ * be NULL, not both; ws_d: hmv_power_ws_doubles(nz, nm) doubles.  Cubes and ws_d 16-byte aligned, ldk even (HMV_E_ARG);
+ * nz <= 65535 (HMV_E_LIMIT).  Every check is made before the first launch.
+ * hmv_sigma_b2: out[z] = sum_j kw[j] P[z][j] (2 J1(ks[j] R[z]) / (ks[j] R[z]))^2, P [nz][nks]: the variance of the
+ *   background mode over a disc of radius R (flat sky) when kw = Simpson weight * k / (2 pi).  x = 0 gives W = 1.
+ * hmv_cl_cov_ssc: Cov^{AB,CD}(l,l') = sum_z zeta_z pref[z] R^{AB}((l+1/2)/chi[z], z) R^{CD}((l'+1/2)/chi[z], z),
+ *   rAB/rCD [nz][nk] (R1h + R2h), linear in k on ks with k clamped to its ends, zeta_z the trapezoid weight on zs (1 when
+ *   nz == 1), pref[z] = H^3 W_A W_B W_C W_D sigma_b^2 / chi^4 from the caller.  out_d [nl1][nl2]; ws_d:
+ *   hmv_cl_cov_ssc_ws_doubles() doubles, 16-byte aligned; nz <= 65535.  The contraction of hmv_cl_cov_1h with one K
+ *   row per redshift; repeated calls give identical results. */
+int hmv_power_response(int nz, int nm, int nk, int ldk, const double* ms_d, const double* ks_d, const double* nzm_d,
+                       const double* bh_d, const double* Pzk_d, double rho_m0, const double* uA_d, int kindA,
+                       const double* uB_d, int kindB, double* ws_d, double* r1h_d, double* r2h_d, void* stream);
+int hmv_sigma_b2(int nz, int nks, const double* ks_d, const double* kw_d, const double* P_d, const double* R_d,
+                 double* out_d, void* stream);
+long long hmv_cl_cov_ssc_ws_doubles(int nz, int nl1, int nl2);
+int hmv_cl_cov_ssc(int nz, int nk, const double* ks_d, const double* rAB_d, const double* rCD_d, int nl1,
+                   const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d, const double* chis_d,
+                   const double* pref_d, double* ws_d, double* out_d, void* stream);
+
 /* ---- f2: kSZ consumer -- the short-wavelength integral of the velocity-reconstruction noise
  * (ksz.py:299-336, Nvv_core_integral):  out[b] = trapz_kS( kS Pge[b,kS]^2 / (Pgg_tot[b,kS] C_tot(chi* kS)) ) with
  * non-finite integrand values set to zero (ksz.py:98-100).  b = 0..nb-1 runs over the (mu,kL) plane when the spectra
