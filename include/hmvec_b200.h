@@ -120,7 +120,10 @@ int hmv_profile_transform_samples(int nz, int nm, int nk, int ldk, const double*
  * hmv_profile_tables runs the evaluation + sine sums only and leaves, per halo, the normalised bins u_j (j <= the bin
  * count the k range needs) in tab_d[z][nmp][JS] (nmp = nm rounded up to 16, JS = hmv_profile_table_stride(nxs)) followed
  * by {k -> bin factor r_s(1+z)/kt_1, u_1, bin count, 0} per halo; hmv_profile_expand interpolates such tables onto ks
- * (fft.py:97-115) and writes the cube.  tables + expand == hmv_profile_transform bit for bit.  Consumers that only
+ * (fft.py:97-115) and writes the cube.  tables + expand == hmv_profile_transform bit for bit.  hmv_profile_expand
+ * recomputes the bin count from its own ks and kmax and does not read the one stored with the table: it must be
+ * called with the ks and kmax the tables were built with (or a range that needs no more bins), since a wider k range
+ * would interpolate from bins that were never written.  Consumers that only
  * need sums over M (hmv_power_six_tab, hmv_power_tab) interpolate from the tables themselves: the 8*nk-byte row of
  * every halo is then neither written nor re-read. */
 long long hmv_profile_table_stride(int nxs);
