@@ -994,6 +994,80 @@ class HaloModel(Cosmology):
         extra = (self._zs_d, self._dev(chis), self._dev(pref))
         return self._trispec_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
 
+    # ------------------------------------------------------------------ 2-halo trispectrum and C_l covariance
+    # Workspace budget of one 2-halo call, in doubles (8 GiB): the largest number of redshifts per pass that fits
+    _TRISPEC_2H_WS_BUDGET = 1 << 30
+
+    def _trispec2h_call(self, fn, names, q1, q2, extra, out_shape):
+        cubes, kinds = self._trispec_legs(names, "2-halo trispectrum",
+                                          "needs occupation moments up to third order, which the HOD does not define")
+        nz, nm = self._nz, self._nm
+        u_h = (C.c_void_p * 4)(*[c.data_ptr() for c in cubes])
+        k_h = (C.c_int * 4)(*kinds)
+        size = getattr(capi.lib, fn + '_ws_doubles')
+        lo, hi = 1, nz                   # the workspace grows with zchunk: the largest zchunk within the budget
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            if size(nz, nm, self._nk, q1.size, q2.size, u_h, k_h, mid) <= self._TRISPEC_2H_WS_BUDGET:
+                lo = mid
+            else:
+                hi = mid - 1
+        ws = self._workspace('trispec', size(nz, nm, self._nk, q1.size, q2.size, u_h, k_h, lo))
+        out = self._empty(*out_shape)
+        q1_d, q2_d = self._dev(q1), self._dev(q2)
+        capi.check(getattr(capi.lib, fn)(nz, nm, self._nk, self._ldk, capi.ptr(self._ks_d), capi.ptr(self._ms_d),
+                                         capi.ptr(self._nzm_d), capi.ptr(self._bh_d), capi.ptr(self._Pzk_d),
+                                         self._rho_m0, u_h, k_h, q1.size, capi.ptr(q1_d), q2.size, capi.ptr(q2_d),
+                                         *[capi.ptr(e) for e in extra], lo, capi.ptr(ws), capi.ptr(out), capi.stream()),
+                   fn)
+        return self._host(out)
+
+    def get_trispectrum_2halo(self, ks1, ks2=None, name="nfw", name2=None, name3=None, name4=None):
+        """2-halo trispectrum of T(k1, -k1, k2, -k2) averaged over the angle between k1 and k2, [nz, nk1, nk2]:
+
+            P(k1) [I1~A(k1) I3^{BCD}(k1,k2,k2) + I1~B(k1) I3^{ACD}(k1,k2,k2)]
+          + P(k2) [I1~C(k2) I3^{ABD}(k1,k1,k2) + I1~D(k2) I3^{ABC}(k1,k1,k2)]
+          + Pbar(k1,k2) [I2^{AC}(k1,k2) I2^{BD}(k1,k2) + I2^{AD}(k1,k2) I2^{BC}(k1,k2)]
+
+        No counterpart in the reference (Cooray & Hu 2001, ApJ 554, 56).  I2^{XY} = sum_M w_M n b t_X t_Y, I3^{XYZ} =
+        sum_M w_M n b t_X t_Y t_Z, I1~X = sum_M w_M n b t_X + b_X - C_X with the consistency terms of get_power_2halo
+        (matter: b = 1, C = sum_M w_M n b M/rho_m0; pressure: 0, 0), so that P I1~A I1~B is get_power_2halo's P2h.  P is
+        Pzk interpolated linearly in k on `ks` and held at its end values outside; Pbar(k1,k2) = (1/(2 k1 k2))
+        int_{|k1-k2|}^{k1+k2} q P(q) dq, in closed form.  The (AB)(CD) pairing carries P(0) and is dropped; I2 and I3
+        carry no consistency term; no 1-halo damping.  Legs t, names, defaults and k handling as get_trispectrum_1halo;
+        HODs raise ValueError.  The redshifts run in passes whose workspace fits _TRISPEC_2H_WS_BUDGET doubles; the
+        result does not depend on the pass size."""
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        k1 = self._positive(ks1, "ks1")
+        k2 = k1 if ks2 is None else self._positive(ks2, "ks2")
+        return self._trispec2h_call('hmv_trispec_2h', (name, name2, name3, name4), k1, k2, (),
+                                    (self._nz, k1.size, k2.size))
+
+    def get_cl_cov_2halo(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
+                         ells2=None):
+        """Non-Gaussian 2-halo Limber covariance Cov(C_l^{AB}, C_l'^{CD}), [len(ells), len(ells2)]:
+
+            1/(4 pi fsky) sum_z zeta_z H^3 W_A W_B W_C W_D / chi^6 T2h^{ABCD}((l+1/2)/chi, (l'+1/2)/chi; z)
+
+        with T2h from get_trispectrum_2halo and the projection, windows, names and defaults of get_cl_cov_1halo.  Not
+        available on a z-sharded model (the z sum would need a cross-rank reduction)."""
+        if self._zcomm is not None:
+            raise NotImplementedError("get_cl_cov_2halo on a z-sharded model: the z sum spans the ranks")
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        l1 = self._positive(ells, "ells")
+        l2 = l1 if ells2 is None else self._positive(ells2, "ells2")
+        fsky = self._fsky(fsky)
+        W = self._window_product(windows)
+        chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
+        H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
+        pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
+        extra = (self._zs_d, self._dev(chis), self._dev(pref))
+        return self._trispec2h_call('hmv_cl_cov_2h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+
     @staticmethod
     def _fsky(fsky):
         fsky = float(fsky)

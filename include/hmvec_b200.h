@@ -315,6 +315,37 @@ int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const dou
                   const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d, double* ws_d,
                   double* out_d, void* stream);
 
+/* ---- 2-halo trispectrum and its non-Gaussian Limber covariance of C_l (DESIGN.md §4.6) ----------------------------
+ * No counterpart in the reference.  Cooray & Hu 2001, ApJ 554, 56; Cooray & Sheth 2002, Phys. Rep. 372, 1, §6.2.  Legs,
+ * kinds, ks and the projection as in hmv_trispec_1h / hmv_cl_cov_1h; w^ = w_m n(z,m) b(z,m) (bh_d [nz][nm]).  For
+ * T(k1,-k1,k2,-k2) averaged over the angle between k1 and k2, legs A, B at k1 and C, D at k2:
+ *   I2^{XY}(k,k')      = sum_m w^ t_X(k) t_Y(k')          I3^{XYZ}(k,k',k'') = sum_m w^ t_X(k) t_Y(k') t_Z(k'')
+ *   I1~X(k)            = sum_m w^ t_X(k) + b_X - C_X       (matter b = 1, C = sum_m w^ M/rho_m0; pressure 0, 0)
+ *   P(k)               = Pzk[z] linear in k on ks, held at the end values outside
+ *   Pbar(k1,k2)        = (1/(2 k1 k2)) int_{|k1-k2|}^{k1+k2} q P(q) dq        (closed form; P piecewise linear)
+ *   T2h(k1,k2;z)       = P(k1) [I1~A I3^{BCD} + I1~B I3^{ACD}] + P(k2) [I1~C I3^{ABD} + I1~D I3^{ABC}]
+ *                      + Pbar [I2^{AC} I2^{BD} + I2^{AD} I2^{BC}]
+ *   Cov2h(l,l')        = sum_z zeta_z pref[z] T2h((l+1/2)/chi[z], (l'+1/2)/chi[z]; z),  pref as in hmv_cl_cov_1h
+ * The (AB)(CD) pairing carries P_lin(0) and is dropped; I2 and I3 carry no consistency term; no 1-halo damping.
+ * zchunk (1 <= zchunk <= nz) redshifts per pass bound the workspace; the result is bit-identical for every zchunk and
+ * for repeated calls.  Legs coincide when they have the same cube pointer and kind: 8 contracted blocks when neither
+ * side coincides, 5 when A == B or C == D, 3 when both.  The workspace functions take the legs for that reason and nk
+ * for the per-redshift Pbar prefix table; they return 0 on invalid sizes or zchunk.  Argument checks, codes and
+ * messages as hmv_trispec_1h, plus bh_d / Pzk_d non-null and the zchunk range, all before the first launch.
+ * hmv_trispec_2h: out_d [nz][nk1][nk2].  hmv_cl_cov_2h: out_d [nl1][nl2]. */
+long long hmv_trispec_2h_ws_doubles(int nz, int nm, int nk, int nk1, int nk2, const double* const* u_h,
+                                    const int* kind_h, int zchunk);
+int hmv_trispec_2h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                   const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                   int nk1, const double* k1_d, int nk2, const double* k2_d, int zchunk, double* ws_d, double* out_d,
+                   void* stream);
+long long hmv_cl_cov_2h_ws_doubles(int nz, int nm, int nk, int nl1, int nl2, const double* const* u_h,
+                                   const int* kind_h, int zchunk);
+int hmv_cl_cov_2h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                  const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                  int nl1, const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                  const double* chis_d, const double* pref_d, int zchunk, double* ws_d, double* out_d, void* stream);
+
 /* ---- super-sample covariance of C_l (matter and pressure profiles) ---------------------------------------------------
  * No counterpart in the reference.  Takada & Hu 2013, PRD 87, 123504; Li, Hu & Takada 2014, PRD 89, 083519.  Legs t_X
  * and kinds as in hmv_trispec_1h (0: matter, a = M/rho_m0; 2: pressure, a = 1); w_m the trapezoid weight on ms.

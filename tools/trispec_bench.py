@@ -1,4 +1,5 @@
-"""Time the non-Gaussian (1-halo) C_l covariance, hmv_cl_cov_1h, on the LARGE grid and on a 25-redshift slab.
+"""Time the non-Gaussian C_l covariances on the LARGE grid: the 1-halo term (hmv_cl_cov_1h, also on a 25-redshift slab)
+and the 2-halo term (hmv_cl_cov_2h).
 
 Cases: C_kk x C_kk (NFW, lensing window of a source at z = 2.5) and C_yy x C_yy (Battaglia pressure) at
 ells = geomspace(10, 1e4, nl) on zs = linspace(0.01, 3, nz), ms = geomspace(2e10, 1e17, nm), ks = geomspace(1e-4, 100,
@@ -9,7 +10,10 @@ nk) (bench.py's grid), and C_kk on the slab zs[:25].  For each case it reports, 
   * flop = 2 n1 n2 nz nm, the contraction's TFLOP/s and its ratio to hmv_bench_dmma measured in the same run;
   * a check of a seeded sample of (l, l') entries against a float64 host reduction over the same cubes;
 
-with the card's name and power limit read in the same run.  Prints one JSON document (and writes it to --out).
+with the card's name and power limit read in the same run.  2-halo cases: C_kk and C_yy autos (3 contracted blocks)
+and the C_ky x C_ky cross (NFW, y, NFW, y: 8 blocks), zchunk as HaloModel.get_cl_cov_2halo picks it; flop = 2 nz nm
+n1 n2 per block; the split into prep, panel, contraction and assembly kernels; a seeded sample of entries against a
+float64 host evaluation (long-double Pbar prefix).  Prints one JSON document (and writes it to --out).
 
     python tools/trispec_bench.py [--nz 200 --nm 2000 --nk 10000 --nl 1000 --reps 10 --out FILE]
 """
@@ -99,6 +103,105 @@ class Case(object):
         return worst
 
 
+class Case2h(object):
+    """The ABI call of one 2-halo covariance, with every input resident on the device."""
+
+    def __init__(self, h, names, windows, ells):
+        from hmvec_b200 import _capi as capi
+        self.capi, self.h, self.names, self.ells = capi, h, names, ells
+        self.cubes, self.kinds = h._trispec_legs(names)
+        zs = h.zs
+        self.chis = np.asarray(h.comoving_radial_distance(zs), dtype=np.float64)
+        H = np.asarray(h.h_of_z(zs), dtype=np.float64)
+        W = np.prod([np.broadcast_to(np.asarray(w, dtype=np.float64), zs.shape) for w in windows], axis=0)
+        self.pref = H ** 3 * W / self.chis ** 6 / (4 * np.pi)
+        self.d = {k: h._dev(v) for k, v in dict(ells=ells, chis=self.chis, pref=self.pref).items()}
+        n = ells.size
+        self.u_h = (C.c_void_p * 4)(*[c.data_ptr() for c in self.cubes])
+        self.k_h = (C.c_int * 4)(*self.kinds)
+        size = lambda zc: capi.lib.hmv_cl_cov_2h_ws_doubles(h._nz, h._nm, h._nk, n, n, self.u_h, self.k_h, zc)
+        self.zchunk = max([zc for zc in range(1, h._nz + 1) if size(zc) <= h._TRISPEC_2H_WS_BUDGET] or [1])
+        self.ws = h._empty(int(size(self.zchunk)))
+        self.out = h._empty(n, n)
+        self.blocks = (1 if self.u_h[0] == self.u_h[1] and self.kinds[0] == self.kinds[1] else 2)
+        nc = (1 if self.u_h[2] == self.u_h[3] and self.kinds[2] == self.kinds[3] else 2)
+        self.blocks = self.blocks * nc + self.blocks + nc
+
+    def launch(self):
+        h, p, d, n = self.h, self.capi.ptr, self.d, self.ells.size
+        self.capi.check(self.capi.lib.hmv_cl_cov_2h(h._nz, h._nm, h._nk, h._ldk, p(h._ks_d), p(h._ms_d), p(h._nzm_d),
+                                                    p(h._bh_d), p(h._Pzk_d), h._rho_m0, self.u_h, self.k_h, n,
+                                                    p(d["ells"]), n, p(d["ells"]), p(h._zs_d), p(d["chis"]),
+                                                    p(d["pref"]), self.zchunk, p(self.ws), p(self.out),
+                                                    self.capi.stream()), "hmv_cl_cov_2h")
+
+    def check_sample(self, rng, npairs=6):
+        """Max |got - want| / sum|terms| over seeded (l, l') entries: T2h per redshift from the cube columns the entries
+        need (gathered on the device), I2, I3, I1~ and P by float64 host sums, Pbar from a long-double prefix."""
+        import torch
+        h = self.h
+        got = self.out.cpu().numpy()
+        ks, ms, nzm, bh, Pzk = h._ks64, h.ms, h.nzm, h.bh, h.Pzk
+        wm = 0.5 * (ms[np.minimum(np.arange(ms.size) + 1, ms.size - 1)] - ms[np.maximum(np.arange(ms.size) - 1, 0)])
+        zs = h.zs
+        zw = 0.5 * (zs[np.minimum(np.arange(zs.size) + 1, zs.size - 1)] - zs[np.maximum(np.arange(zs.size) - 1, 0)])
+        w = wm[None, :] * nzm * bh
+        cons = 1.0 - (w * ms[None, :] / h._rho_m0).sum(1)
+        zi = torch.arange(zs.size, device=self.cubes[0].device)
+        kl = ks.astype(np.longdouble)
+
+        def leg(c, ell):                   # t(z, m) at k = (l + 1/2)/chi_z, linear in k, clamped
+            k = np.clip((ell + 0.5) / self.chis, ks[0], ks[-1])
+            j = np.clip(np.searchsorted(ks, k, side="right") - 1, 0, ks.size - 2)
+            f = (k - ks[j]) / (ks[j + 1] - ks[j])
+            jd = torch.as_tensor(j, device=self.cubes[c].device)
+            u0, u1 = self.cubes[c][zi, :, jd].cpu().numpy(), self.cubes[c][zi, :, jd + 1].cpu().numpy()
+            a = ms / h._rho_m0 if self.kinds[c] == 0 else np.ones(ms.size)
+            return a[None, :] * (u0 + f[:, None] * (u1 - u0))
+
+        def F(z, x):                       # int_0^x q P dq, P linear on ks and held at its ends, long double
+            P = Pzk[z].astype(np.longdouble)
+            S = np.concatenate([[0], np.cumsum((kl[1:] - kl[:-1]) * (kl[:-1] * (2 * P[:-1] + P[1:]) +
+                                                                      kl[1:] * (P[:-1] + 2 * P[1:])) / 6)])
+            x = np.longdouble(x)
+            if x < kl[0]:
+                return P[0] * x * x / 2
+            base = P[0] * kl[0] ** 2 / 2
+            if x >= kl[-1]:
+                return base + S[-1] + P[-1] * (x * x - kl[-1] ** 2) / 2
+            r = min(max(np.searchsorted(kl, x, side="right") - 1, 0), ks.size - 2)
+            px = P[r] + (x - kl[r]) / (kl[r + 1] - kl[r]) * (P[r + 1] - P[r])
+            return base + S[r] + (x - kl[r]) * (kl[r] * (2 * P[r] + px) + x * (P[r] + 2 * px)) / 6
+
+        worst = 0.0
+        for _ in range(npairs):
+            i, j = rng.integers(0, self.ells.size, 2)
+            tA, tB = leg(0, self.ells[i]), leg(1, self.ells[i])
+            tC, tD = leg(2, self.ells[j]), leg(3, self.ells[j])
+            want = bound = 0.0
+            for z in range(zs.size):
+                k1, k2 = (self.ells[i] + 0.5) / self.chis[z], (self.ells[j] + 0.5) / self.chis[z]
+                k1l, k2l = np.longdouble(k1), np.longdouble(k2)
+                pb = float((F(z, k1l + k2l) - F(z, abs(k1l - k2l))) / (2 * k1l * k2l))
+                P1, P2 = np.interp(k1, ks, Pzk[z]), np.interp(k2, ks, Pzk[z])
+                W, Wa = w[z], np.abs(w[z])
+                zo = [cons[z] if k == 0 else 0.0 for k in self.kinds]
+                t = (tA[z], tB[z], tC[z], tD[z])
+                vals = []
+                for s, (Ww, f) in enumerate(((W, lambda x: x), (Wa, np.abs))):
+                    I1 = [np.sum(Ww * f(t[q])) + f(zo[q]) for q in range(4)]
+                    I3 = lambda x, y, u: np.sum(Ww * f(t[x] * t[y] * t[u]))
+                    I2 = lambda x, y: np.sum(Ww * f(t[x] * t[y]))
+                    v = f(P1) * (I1[0] * I3(1, 2, 3) + I1[1] * I3(0, 2, 3)) \
+                        + f(P2) * (I1[2] * I3(0, 1, 3) + I1[3] * I3(0, 1, 2)) \
+                        + f(pb) * (I2(0, 2) * I2(1, 3) + I2(0, 3) * I2(1, 2))
+                    vals.append(v)
+                want += zw[z] * self.pref[z] * vals[0]
+                bound += abs(zw[z] * self.pref[z]) * abs(vals[1])
+            worst = max(worst, abs(got[i, j] - want) / bound if bound > 0 else abs(got[i, j] - want))
+        return worst
+
+
 def time_case(case, reps, dmma_tflops):
     import torch
     from torch.profiler import ProfilerActivity, profile
@@ -118,24 +221,32 @@ def time_case(case, reps, dmma_tflops):
             case.launch()
         torch.cuda.synchronize()
     per = {}
+    names = (("trispec2h_prep_kernel", "prep"), ("trispec2h_panel_kernel", "panel"), ("trispec_panel_kernel", "panel"),
+             ("sigma2_gemm_kernel", "contraction"), ("trispec_reduce_kernel", "reduce"),
+             ("trispec2h_assemble_kernel", "assemble"))
     for ev in prof.key_averages():
-        key = "panel" if "trispec_panel_kernel" in ev.key else "contraction" if "sigma2_gemm_kernel" in ev.key else \
-            "reduce" if "trispec_reduce_kernel" in ev.key else None
+        key = next((k for n, k in names if n in ev.key), None)
         if key:
             t = getattr(ev, "device_time_total", None)
             if t is None:
                 t = ev.cuda_time_total
             per[key] = per.get(key, 0.0) + t / 1e3 / nprof
     h, n = case.h, case.ells.size
-    flop = 2.0 * n * n * h._nz * h._nm
+    blocks = getattr(case, "blocks", 1)
+    flop = 2.0 * n * n * h._nz * h._nm * blocks
     K, ld = h._nz * (h._nm + h._nm % 2), n + n % 2
     res = {"nz": h._nz, "nm": h._nm, "nk": h._nk, "nl": n, "call_ms": total_ms, "reps": reps,
            "panel_ms": per.get("panel"), "contraction_ms": per.get("contraction"), "reduce_ms": per.get("reduce"),
-           "flop": flop, "panel_bytes_written": 2.0 * K * ld * 8}
+           "flop": flop, "blocks": blocks}
+    if blocks == 1:
+        res["panel_bytes_written"] = 2.0 * K * ld * 8
+    else:
+        res.update(prep_ms=per.get("prep"), assemble_ms=per.get("assemble"), zchunk=case.zchunk,
+                   names=list(case.names))
     if per.get("contraction"):
         res["contraction_tflops"] = flop / (per["contraction"] * 1e-3) / 1e12
         res["contraction_over_dmma"] = res["contraction_tflops"] / dmma_tflops
-    if per.get("panel"):
+    if per.get("panel") and "panel_bytes_written" in res:
         res["panel_write_gbs"] = res["panel_bytes_written"] / (per["panel"] * 1e-3) / 1e9
     res["call_tflops"] = flop / (total_ms * 1e-3) / 1e12
     return res
@@ -176,6 +287,14 @@ def main():
         results[tag] = time_case(c, a.reps, dmma)
         results[tag]["sample_max_err_over_bound"] = c.check_sample(rng)
         del c
+        torch.cuda.empty_cache()
+    for tag, names, win in (("large_kk_2h", ("nfw",) * 4, (Wk,) * 4), ("large_yy_2h", ("y",) * 4, (1.,) * 4),
+                            ("large_ky_ky_2h", ("nfw", "y", "nfw", "y"), (Wk, 1., Wk, 1.))):
+        c = Case2h(h, names, win, ells)
+        results[tag] = time_case(c, a.reps, dmma)
+        results[tag]["sample_max_err_over_bound"] = c.check_sample(rng)
+        del c
+        h._ws.clear()
         torch.cuda.empty_cache()
     del h
     torch.cuda.empty_cache()
