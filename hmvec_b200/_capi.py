@@ -94,6 +94,18 @@ _SIGS = {
     "hmv_cl_cov_2h_ws_doubles": (_ll, [_i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_i), _i]),
     "hmv_cl_cov_2h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p,
                            _p, _p, _i, _p, _p, _p]),
+    "hmv_trispec_3h_ws_doubles": (_ll, [_i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_i), _i]),
+    "hmv_trispec_3h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _i,
+                            _p, _p, _p]),
+    "hmv_cl_cov_3h_ws_doubles": (_ll, [_i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_i), _i]),
+    "hmv_cl_cov_3h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p,
+                           _p, _p, _i, _p, _p, _p]),
+    "hmv_trispec_4h_ws_doubles": (_ll, [_i, _i, _i, _i]),
+    "hmv_trispec_4h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p,
+                            _p, _p]),
+    "hmv_cl_cov_4h_ws_doubles": (_ll, [_i, _i, _i, _i]),
+    "hmv_cl_cov_4h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p,
+                           _p, _p, _p, _p, _p]),
     "hmv_power_response": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, _p, _i, _p, _i, _p, _p, _p, _p]),
     "hmv_sigma_b2": (_i, [_i, _i, _p, _p, _p, _p, _p, _p]),
     "hmv_cl_cov_ssc_ws_doubles": (_ll, [_i, _i, _i]),

@@ -12,6 +12,8 @@
 // The super-sample covariance (DESIGN.md §4.5) reuses the projection with K = z; sigma_b^2 of a disc is here too.
 // The 2-halo trispectrum and its covariance (DESIGN.md §4.6) run the trispectrum's batched product three times per pass
 // of redshifts and combine the blocks per (z, k1, k2) with P_lin and its angle average; see the section below.
+// The 3- and 4-halo trispectra (DESIGN.md §4.7) add the angle-averaged tree-level bispectrum and trispectrum: exact
+// window moments of P_lin per (z, k1, k2), the 2-halo I2 product for the 3-halo term.
 #include "common.cuh"
 #include "gemm_f64.cuh"
 
@@ -556,6 +558,517 @@ static int trispec2h_run(const char* who, bool proj, int nz, int nm, int nk, int
   return HMV_OK;
 }
 
+// ---- 3- and 4-halo trispectra (DESIGN.md §4.7) ------------------------------------------------------------------------
+//   T3h^{ABCD}(k1,k2;z) = Bbar [I2^{AC} I1~B I1~D + I2^{AD} I1~B I1~C + I2^{BC} I1~A I1~D + I2^{BD} I1~A I1~C]
+//   T4h^{ABCD}(k1,k2;z) = I1~A I1~B I1~C I1~D Tbar
+//   Bbar = (34/21) P1 P2 + 2 <G P(q)>,   Tbar = 12 P1 P2^2 F3bar(k2/k1) + 12 P1^2 P2 F3bar(k1/k2) + 8 <G^2 P(q)>
+// with I1~, I2 as in the 2-halo section, P1 = P(k1), P2 = P(k2), q = |k1 + k2| and, for x = q^2 and d = k1^2 - k2^2,
+//   G = P1 F2(-k1, k1+k2) + P2 F2(-k2, k1+k2) = g1 x + g0 + gm / x,
+//   g1 = -5/28 (P1/k1^2 + P2/k2^2),  g0 = 13/28 (P1 + P2) - 3d/28 (P1/k1^2 - P2/k2^2),
+//   gm = -d/4 (P1 - P2) + d^2/14 (P1/k1^2 + P2/k2^2).
+// <f> = (1/(2 k1 k2)) int_{|k1-k2|}^{k1+k2} q f(q) dq, so <G P> and <G^2 P> are sums of gn M_n with the window moments
+// M_n = int q^n P(q) dq, n = -3, -1, 1, 3, 5: exact for P linear on each interval of ks and held at its end values.
+
+// double-double accumulation of the moment tables: a window's moment is a difference of two table entries, and a
+// double table would lose (window / whole range) of it
+struct DD {
+  double hi, lo;
+};
+
+__device__ __forceinline__ DD dd_add(DD a, double b) {
+  const double s = a.hi + b, bb = s - a.hi, e = ((a.hi - (s - bb)) + (b - bb)) + a.lo, h = s + e;
+  return {h, e - (h - s)};
+}
+
+__device__ __forceinline__ DD dd_add(DD a, DD b) {
+  const double s = a.hi + b.hi, bb = s - a.hi, e = ((a.hi - (s - bb)) + (b.hi - bb)) + (a.lo + b.lo), h = s + e;
+  return {h, e - (h - s)};
+}
+
+// a - b rounded to double
+__device__ __forceinline__ double dd_diff(DD a, DD b) {
+  const double s = a.hi - b.hi, bb = s - a.hi, e = (a.hi - (s - bb)) + (-b.hi - bb);
+  return s + (e + (a.lo - b.lo));
+}
+
+constexpr int PT_NMOM = 5;   // moments q^-3, q^-1, q^1, q^3, q^5
+
+// int_{x0}^{x1} q^n P(q) dq, n = -3, -1, 1, 3, 5, for P linear from p0 at x0 to p1 at x1; h = x1 - x0 formed by the
+// caller.  The negative powers in closed forms without cancellation (x0 = 0 gives 0: their coefficients vanish there);
+// the positive ones by 4-node Gauss-Legendre, exact for these polynomials of degree <= 6.
+__device__ __forceinline__ void qmom_piece(double x0, double x1, double h, double p0, double p1, double m[PT_NMOM]) {
+  if (x0 > 0.0) {
+    const double y = h / x0, L = log1p(y);
+    m[0] = h * (p0 * (x1 / x0) + p1) / (2.0 * x0 * x1 * x1);
+    m[1] = p0 * L + (p1 - p0) * (1.0 - L / y);
+  } else {
+    m[0] = m[1] = 0.0;
+  }
+  const double t[4] = {0.06943184420297371, 0.33000947820757187, 0.66999052179242813, 0.93056815579702629};
+  const double w[4] = {0.17392742256872693, 0.32607257743127307, 0.32607257743127307, 0.17392742256872693};
+  m[2] = m[3] = m[4] = 0.0;
+  for (int i = 0; i < 4; ++i) {
+    const double q = fma(h, t[i], x0), q2 = q * q, v = h * w[i] * q * fma(t[i], p1 - p0, p0);
+    m[2] += v;
+    m[3] = fma(v, q2, m[3]);
+    m[4] = fma(v * q2, q2, m[4]);
+  }
+}
+
+// One CTA per chunk redshift: tab[zl][n][j] (double-double) = int_{ks[0]}^{ks[j]} q^n P for n = 1, 3, 5 and
+// int_{ks[j]}^{ks[nk-1]} q^n P for n = -3, -1 (each accumulated from the end where it is small, so that a difference is
+// dominated by its own window).  Each thread sums a contiguous run of intervals, thread 0 scans the run totals: a fixed
+// order, so every chunking gives the same bits.
+__global__ void __launch_bounds__(256) trispec_pt_moments_kernel(int z0, int nk, const double* __restrict__ ks,
+                                                                 const double* __restrict__ Pzk,
+                                                                 DD* __restrict__ tab) {
+  __shared__ DD red[256][PT_NMOM];
+  const int zl = blockIdx.x, z = z0 + zl, t = threadIdx.x;
+  const double* P = Pzk + (long long)z * nk;
+  DD* T = tab + (long long)zl * PT_NMOM * nk;
+  const int per = (nk - 1 + blockDim.x - 1) / blockDim.x, j0 = min(nk - 1, t * per), j1 = min(nk - 1, j0 + per);
+  DD run[PT_NMOM];
+  double m[PT_NMOM];
+  for (int n = 0; n < PT_NMOM; ++n) run[n] = {0.0, 0.0};
+  for (int j = j0; j < j1; ++j) {
+    qmom_piece(ks[j], ks[j + 1], ks[j + 1] - ks[j], P[j], P[j + 1], m);
+    for (int n = 0; n < PT_NMOM; ++n) run[n] = dd_add(run[n], m[n]);
+  }
+  for (int n = 0; n < PT_NMOM; ++n) red[t][n] = run[n];
+  __syncthreads();
+  if (t == 0) {   // exclusive scans: forward for the positive powers, backward for the negative ones
+    for (int n = 0; n < PT_NMOM; ++n) {
+      DD s = {0.0, 0.0};
+      for (int i = 0; i < (int)blockDim.x; ++i) {
+        const int q = n < 2 ? (int)blockDim.x - 1 - i : i;
+        const DD v = red[q][n];
+        red[q][n] = s;
+        s = dd_add(s, v);
+      }
+      T[(long long)n * nk + (n < 2 ? nk - 1 : 0)] = {0.0, 0.0};
+    }
+  }
+  __syncthreads();
+  for (int n = 0; n < PT_NMOM; ++n) run[n] = red[t][n];
+  for (int j = j0; j < j1; ++j) {
+    qmom_piece(ks[j], ks[j + 1], ks[j + 1] - ks[j], P[j], P[j + 1], m);
+    for (int n = 2; n < PT_NMOM; ++n) {
+      run[n] = dd_add(run[n], m[n]);
+      T[(long long)n * nk + j + 1] = run[n];
+    }
+  }
+  for (int j = j1 - 1; j >= j0; --j) {
+    qmom_piece(ks[j], ks[j + 1], ks[j + 1] - ks[j], P[j], P[j + 1], m);
+    for (int n = 0; n < 2; ++n) {
+      run[n] = dd_add(run[n], m[n]);
+      T[(long long)n * nk + j] = run[n];
+    }
+  }
+}
+
+// Ratios max(k1,k2)/min(k1,k2) >= PT_R0 take the local branch of pt_averages (below).  The Laurent sums' terms grow
+// like r^2 times <G^2 P>, and Tbar is a further r^2 below its two leading pieces (12 P_lo^2 P_hi F3bar(lo/hi) ->
+// -(2/3) r^2 P_lo^2 P_hi and 8 <G^2 P> -> +(2/3) r^2 P_lo^2 P_hi), so there the Laurent route would lose eps r^4 of
+// Tbar; below PT_R0 that is <~1e-9.  The local branch costs 8 evaluations per interval its window crosses, so PT_R0 is
+// as large as that loss allows.  The decision uses the caller's q values, so the F3 table and the assembly agree.
+constexpr double PT_R0 = 100.0;
+
+__device__ __forceinline__ bool pt_local(double x1, double x2) { return fmax(x1, x2) >= PT_R0 * fmin(x1, x2); }
+
+// The local branch, in t = q - hi on the window t in [-lo, lo] (r = hi/lo >= PT_R0).  With A = -(1/2) r mu P_lo, the
+// large part of P_lo F2(-k_lo, s), and R = G - A (bounded):
+//   <G P>   = <A (P(q) - P_hi) + R P(q)>                       (<A> P_hi = 0)
+//   <D>     = <G^2 P> - (r^2/12) P_lo^2 P_hi = <A^2 (P(q) - P_hi) + (2A + R) R P(q)>
+// and the caller's Tbar = 12 P1 P2 (P2 F12 + P1 F21) + 8 <D> holds with the table entry of the small ratio x = lo/hi
+// taken as F3bar(x) + 1/(18 x^2) (f3bar's tail): the two -(2/3) r^2 P_lo^2 P_hi pieces cancel in closed form.  Every
+// factor is formed from local differences: mu r = (t (2 hi + t) - lo^2)/(2 lo^2); P(q) - P_hi from node differences
+// and slopes times local lengths.  Each piece of the window between nodes takes 8-node Gauss-Legendre: the integrand
+// is a polynomial of degree <= 6 in t plus a rational part whose poles (q = 0) lie r half-widths away, so the rule's
+// error is below (2 r)^-16 of the terms.  Pointwise terms are O(r) times the result: the error is a few eps r.
+__device__ __noinline__ void pt_averages_local(const double* __restrict__ ks, const double* __restrict__ P, int nk,
+                                               double k1, double k2, double P1, double P2, double& gp, double& g2p) {
+  const double x[4] = {0.1834346424956498, 0.5255324099163290, 0.7966664774136267, 0.9602898564975363};
+  const double w[4] = {0.3626837833783620, 0.3137066458778873, 0.2223810344533745, 0.1012285362903763};
+  const double lo = fmin(k1, k2), hi = fmax(k1, k2), Plo = k1 <= k2 ? P1 : P2, Phi = k1 <= k2 ? P2 : P1;
+  int ra, rb, m;
+  plin_at(ks, P, nk, hi - lo, ra);
+  plin_at(ks, P, nk, hi + lo, rb);
+  plin_at(ks, P, nk, hi, m);
+  const double sm = (m < 0 || m >= nk - 1) ? 0.0 : (P[m + 1] - P[m]) / (ks[m + 1] - ks[m]);
+  const double lo2 = lo * lo;
+  double sg = 0.0, sd = 0.0;
+  for (int j = ra; j <= rb; ++j) {
+    const bool held = j < 0 || j >= nk - 1;
+    const double sj = held ? 0.0 : (P[j + 1] - P[j]) / (ks[j + 1] - ks[j]);
+    const double t0 = j == ra ? -lo : ks[j] - hi, t1 = j == rb ? lo : ks[j + 1] - hi;
+    const double hw = 0.5 * (t1 - t0), c = t0 + hw;
+    // P(q) - P_hi = base + sj * (t - tj): from the node next to hi, so that no term is larger than the window needs
+    double base = 0.0, tj = 0.0;
+    if (j > m) {
+      base = sm * (ks[m + 1] - hi) + (P[j] - P[m + 1]);
+      tj = ks[j] - hi;
+    } else if (j < m) {
+      base = (P[j + 1] - P[m]) - sm * (hi - ks[m]);
+      tj = ks[j + 1] - hi;
+    }
+    for (int g = 0; g < 8; ++g) {
+      const double t = fma(hw, g < 4 ? -x[3 - g] : x[g - 4], c), wt = hw * w[g < 4 ? 3 - g : g - 4];
+      const double dP = base + sj * (t - tj), Pq = Phi + dP;
+      const double u = t * (2.0 * hi + t), q = hi + t, q2 = q * q;
+      const double A = -0.25 * (u - lo2) / lo2 * Plo;
+      const double v = (u + lo2) / (2.0 * lo), ww = hi + t + (t * t - lo2) / (2.0 * hi);
+      const double R = Plo * (3.0 / 14.0 - 0.5 * lo * v / q2 + (2.0 / 7.0) * v * v / q2) +
+                       Phi * (5.0 / 7.0 - 0.5 * ww / hi - 0.5 * hi * ww / q2 + (2.0 / 7.0) * ww * ww / q2);
+      const double f = wt * q;
+      sg = fma(f, A * dP + R * Pq, sg);
+      sd = fma(f, A * A * dP + (2.0 * A + R) * R * Pq, sd);
+    }
+  }
+  const double inv = 1.0 / (2.0 * lo * hi);
+  gp = sg * inv;
+  g2p = sd * inv;
+}
+
+// <G P> and <G^2 P> at (k1, k2) from one redshift's P and moment table; local (pt_local of the caller's q): the local
+// branch, whose g2p is <D>.  Window [a, b] = [|k1-k2|, k1+k2]: ends in one region give one piece; otherwise an end
+// piece on each side (widths formed as in pbar) and, over whole intervals between them, a difference of table entries.
+__device__ __forceinline__ void pt_averages(const double* __restrict__ ks, const double* __restrict__ P,
+                                            const DD* __restrict__ T, int nk, double k1, double k2, double P1,
+                                            double P2, bool local, double& gp, double& g2p) {
+  if (local) {
+    pt_averages_local(ks, P, nk, k1, k2, P1, P2, gp, g2p);
+    return;
+  }
+  const double lo = fmin(k1, k2), hi = fmax(k1, k2), a = hi - lo, b = hi + lo;
+  int ra, rb;
+  const double pa = plin_at(ks, P, nk, a, ra), pb = plin_at(ks, P, nk, b, rb);
+  double M[PT_NMOM], m[PT_NMOM];
+  if (ra == rb) {
+    qmom_piece(a, b, 2.0 * lo, pa, pb, M);
+  } else {
+    const double xa = ks[ra + 1], xb = ks[rb];
+    qmom_piece(a, xa, (xa - hi) + lo, pa, P[ra + 1], M);
+    qmom_piece(xb, b, (hi - xb) + lo, P[rb], pb, m);
+    for (int n = 0; n < PT_NMOM; ++n) M[n] += m[n];
+    if (rb > ra + 1)
+      for (int n = 0; n < PT_NMOM; ++n)
+        M[n] += n < 2 ? dd_diff(T[(long long)n * nk + ra + 1], T[(long long)n * nk + rb])
+                      : dd_diff(T[(long long)n * nk + rb], T[(long long)n * nk + ra + 1]);
+  }
+  const double d = (k1 - k2) * (k1 + k2), r1 = P1 / (k1 * k1), r2 = P2 / (k2 * k2);
+  const double g1 = (-5.0 / 28.0) * (r1 + r2);
+  const double g0 = (13.0 / 28.0) * (P1 + P2) - (3.0 / 28.0) * d * (r1 - r2);
+  const double gm = -0.25 * d * (P1 - P2) + (d * d / 14.0) * (r1 + r2);
+  const double inv = 1.0 / (2.0 * k1 * k2);
+  gp = (g1 * M[3] + g0 * M[2] + gm * M[1]) * inv;
+  g2p = (g1 * g1 * M[4] + 2.0 * g1 * g0 * M[3] + (g0 * g0 + 2.0 * g1 * gm) * M[2] + 2.0 * g0 * gm * M[1] +
+         gm * gm * M[0]) * inv;
+}
+
+// F3bar(r) = <F3_sym(k, q, -q)> over the angle, r = q/k:
+//   [12/r^2 - 158 + 100 r^2 - 42 r^4 + (3/r^3)(r^2-1)^3 (7r^2+2) ln|(1+r)/(1-r)|] / (3024 r^2).
+// The closed form cancels for small and large r: series in r^2 below 0.4 and in 1/r^2 above 2.5 (26 terms each, exact
+// rationals rounded once, truncation below 1e-20); -11/378 at r = 1.  tail (r < 0.4 only): F3bar(r) + 1/(18 r^2), the
+// small-r series without its leading term (see pt_averages_local).
+__device__ double f3bar(double r, bool tail) {
+  constexpr double cs[26] = {
+      -0.05555555555555555, 0.061375661375661375, -0.042630385487528344, 0.00655076845553036,
+      0.000760438855676951, 0.00021354307068592783, 8.38667505334172e-05, 3.975690250200054e-05,
+      2.130652285451047e-05, 1.2456624575156199e-05, 7.773259316439517e-06, 5.103490671630971e-06,
+      3.4900532521396275e-06, 2.467901851543364e-06, 1.7946309316753127e-06, 1.3364096913719952e-06,
+      1.0157257186584305e-06, 7.8582630624582e-07, 6.175121382494654e-07, 4.919865547043248e-07,
+      3.9682399296693115e-07, 3.2361537371936314e-07, 2.665494674200016e-07, 2.2153424371892526e-07,
+      1.856390527643294e-07, 1.567325245090209e-07};
+  constexpr double cl[26] = {
+      -0.032275132275132276, 0.006349206349206349, -0.0025195263290501385, -0.0003939622987242035,
+      -0.0001289715575429861, -5.567624615243663e-05, -2.8149047756890894e-05, -1.580806534366906e-05,
+      -9.57648016471546e-06, -6.145351606190404e-06, -4.126746045481503e-06, -2.875065894934407e-06,
+      -2.0649791002709783e-06, -1.521683261458535e-06, -1.146173436372423e-06, -8.798426793730217e-07,
+      -6.866684127132244e-07, -5.437793456226636e-07, -4.3623737003527943e-07, -3.540397349651057e-07,
+      -2.9033872860683223e-07, -2.40352959565456e-07, -2.0068396195714407e-07, -1.6887706154407393e-07,
+      -1.4313317314164382e-07, -1.2211599375569742e-07};
+  if (r < 0.4 || r > 2.5) {   // F = sum cs[k] r^(2k-2)  or  sum cl[k] r^(-2k-2)
+    const double y = r < 0.4 ? r * r : 1.0 / (r * r);
+    const double* c = r < 0.4 ? cs : cl;
+    double s = c[25];
+    for (int k = 24; k >= (tail ? 1 : 0); --k) s = fma(s, y, c[k]);
+    return tail ? s : r < 0.4 ? s / y : s * y;
+  }
+  if (r == 1.0) return -11.0 / 378.0;
+  const double r2 = r * r, L = 2.0 * atanh(r < 1.0 ? r : 1.0 / r), u = r2 - 1.0;
+  return (12.0 / r2 - 158.0 + r2 * (100.0 - 42.0 * r2) + (3.0 / (r2 * r)) * (u * u * u) * (7.0 * r2 + 2.0) * L) /
+         (3024.0 * r2);
+}
+
+// F3[0][i][j] = F3bar(k2/k1), F3[1][i][j] = F3bar(k1/k2): the ratio is the same at every redshift, (l'+1/2)/(l+1/2) in
+// projection.  Where pt_local holds, the entry of the small ratio is f3bar's tail (see pt_averages_local).
+__global__ void __launch_bounds__(256) trispec4h_f3_kernel(int n1, int n2, const double* __restrict__ q1,
+                                                           const double* __restrict__ q2, int proj,
+                                                           double* __restrict__ F3) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x, n = (long long)n1 * n2;
+  if (e >= n) return;
+  const int i = (int)(e / n2), j = (int)(e - (long long)i * n2);
+  const double s = proj ? 0.5 : 0.0, x1 = q1[i] + s, x2 = q2[j] + s;
+  const bool local = pt_local(x1, x2);
+  F3[e] = f3bar(x2 / x1, local && x2 < x1);
+  F3[n + e] = f3bar(x1 / x2, local && x1 < x2);
+}
+
+// One thread per chunk redshift blockIdx.y, side blockIdx.z (0: k1 legs A, B; 1: k2 legs C, D) and column: P(k) into
+// Pk[zl][l] and I1~ of the side's distinct legs into I1[zl][leg][ld] by a mass sum in increasing m.
+__global__ void __launch_bounds__(TP_T) trispec_pt_side_kernel(int z0, int nm, int nk, int ldk,
+                                                               const double* __restrict__ ks,
+                                                               const double* __restrict__ ms,
+                                                               const double* __restrict__ nzm,
+                                                               const double* __restrict__ bh,
+                                                               const double* __restrict__ Pzk, double rho_m0,
+                                                               const Legs2h L, int n1, int ld1,
+                                                               const double* __restrict__ q1, int n2, int ld2,
+                                                               const double* __restrict__ q2,
+                                                               const double* __restrict__ chis, double* __restrict__ Pk1,
+                                                               double* __restrict__ Pk2, double* __restrict__ I1a,
+                                                               double* __restrict__ I1c) {
+  const int zl = blockIdx.y, z = z0 + zl, side = blockIdx.z, l = blockIdx.x * TP_T + threadIdx.x;
+  const int n = side ? n2 : n1, ld = side ? ld2 : ld1, X = 2 * side, nleg = side ? L.nC1 : L.nA1;
+  if (l >= n) return;
+  const double q = side ? q2[l] : q1[l], inv_chi = chis ? 1.0 / chis[z] : 0.0;
+  int j;
+  double f;
+  k_locate(ks, nk, chis ? (q + 0.5) * inv_chi : q, j, f);
+  (side ? Pk2 : Pk1)[(long long)zl * n + l] = k_lerp(Pzk + (long long)z * nk, j, f);
+  double c = 0.0, s0 = 0.0, s1 = 0.0;
+  for (int m = 0; m < nm; ++m) {
+    const long long i = (long long)z * nm + m, row = i * ldk;
+    const double a = ms[m] / rho_m0, w = trapz_weight(ms, m, nm) * nzm[i] * bh[i];
+    c = fma(w, a, c);
+    s0 = fma(w, (L.matter[X] ? a : 1.0) * k_lerp(L.u[X] + row, j, f), s0);
+    if (nleg == 2) s1 = fma(w, (L.matter[X + 1] ? a : 1.0) * k_lerp(L.u[X + 1] + row, j, f), s1);
+  }
+  double* I1 = (side ? I1c : I1a) + (long long)zl * 2 * ld;
+  I1[l] = s0 + (L.matter[X] ? 1.0 - c : 0.0);
+  if (nleg == 2) I1[ld + l] = s1 + (L.matter[X + 1] ? 1.0 - c : 0.0);
+}
+
+// The side vectors of a pass of zc redshifts: Pk1 [zc][n1p], Pk2 [zc][n2p], I1a [zc][2][n1p], I1c [zc][2][n2p] and the
+// moment table [zc][5][nk] in double-double
+struct PtSides {
+  double *Pk1, *Pk2, *I1a, *I1c;
+  DD* tab;
+};
+
+static long long pt_sides_doubles(int zc, int nk, int n1, int n2) {
+  return (long long)zc * (3LL * (n1 + (n1 & 1)) + 3LL * (n2 + (n2 & 1)) + 2LL * PT_NMOM * nk);
+}
+
+static PtSides pt_sides(double* ws, int zc, int nk, int n1, int n2) {
+  PtSides s;
+  const long long n1p = n1 + (n1 & 1), n2p = n2 + (n2 & 1);
+  s.Pk1 = ws;
+  s.Pk2 = s.Pk1 + zc * n1p;
+  s.I1a = s.Pk2 + zc * n2p;
+  s.I1c = s.I1a + 2LL * zc * n1p;
+  s.tab = reinterpret_cast<DD*>(s.I1c + 2LL * zc * n2p);
+  return s;
+}
+
+static int pt_sides_run(int z0, int zn, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                        const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0, const Legs2h& L,
+                        int n1, const double* q1_d, int n2, const double* q2_d, const double* chis_d,
+                        const PtSides& s, cudaStream_t st) {
+  trispec_pt_moments_kernel<<<zn, 256, 0, st>>>(z0, nk, ks_d, Pzk_d, s.tab);
+  int rc = check_launch("trispec_pt_moments_kernel");
+  if (rc) return rc;
+  dim3 g(cdiv(n1 > n2 ? n1 : n2, TP_T), zn, 2);
+  trispec_pt_side_kernel<<<g, TP_T, 0, st>>>(z0, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, L, n1,
+                                             n1 + (n1 & 1), q1_d, n2, n2 + (n2 & 1), q2_d, chis_d, s.Pk1, s.Pk2,
+                                             s.I1a, s.I1c);
+  return check_launch("trispec_pt_side_kernel");
+}
+
+// One thread per output element (i, j): the chunk's redshifts in increasing z (3D: T3h into out[z][i][j]; projection:
+// zeta_z pref_z T3h added onto the previous chunk's value, onto zero when first == 1).
+__global__ void __launch_bounds__(256) trispec3h_assemble_kernel(int z0, int zc, int nz, int nk,
+                                                                 const double* __restrict__ ks,
+                                                                 const double* __restrict__ Pzk, const Plan2h p, const double* __restrict__ q1,
+                                                                 const double* __restrict__ q2,
+                                                                 const double* __restrict__ zs,
+                                                                 const double* __restrict__ chis,
+                                                                 const double* __restrict__ pref,
+                                                                 const double* __restrict__ O22, const PtSides s,
+                                                                 int first, double* __restrict__ out) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x, n = (long long)p.n1 * p.n2;
+  if (e >= n) return;
+  const int i = (int)(e / p.n2), j = (int)(e - (long long)i * p.n2);
+  const long long w22 = p.m2s(), s22 = p.m1s() * w22;
+  const long long rB = (p.nA1 == 2 ? p.n1p : 0), cD = (p.nC1 == 2 ? p.n2p : 0);   // B and D rows/columns, also in I1
+  const bool local = chis ? pt_local(q1[i] + 0.5, q2[j] + 0.5) : pt_local(q1[i], q2[j]);
+  double acc = (chis && !first) ? out[e] : 0.0;
+  for (int zl = 0; zl < zc; ++zl) {
+    const int z = z0 + zl;
+    const double* o22 = O22 + zl * s22;
+    const double* Ia = s.I1a + 2LL * zl * p.n1p;
+    const double* Ic = s.I1c + 2LL * zl * p.n2p;
+    const double I1A = Ia[i], I1B = Ia[rB + i], I1C = Ic[j], I1D = Ic[cD + j];
+    const double I2AC = o22[i * w22 + j], I2AD = o22[i * w22 + cD + j];
+    const double I2BC = o22[(rB + i) * w22 + j], I2BD = o22[(rB + i) * w22 + cD + j];
+    const double inv_chi = chis ? 1.0 / chis[z] : 0.0;
+    const double k1 = chis ? (q1[i] + 0.5) * inv_chi : q1[i], k2 = chis ? (q2[j] + 0.5) * inv_chi : q2[j];
+    const double P1 = s.Pk1[(long long)zl * p.n1 + i], P2 = s.Pk2[(long long)zl * p.n2 + j];
+    double gp, g2p;
+    pt_averages(ks, Pzk + (long long)z * nk, s.tab + (long long)zl * PT_NMOM * nk, nk, k1, k2, P1, P2, local, gp,
+                g2p);
+    const double B = (34.0 / 21.0) * P1 * P2 + 2.0 * gp;
+    const double T = B * (I2AC * I1B * I1D + I2AD * I1B * I1C + I2BC * I1A * I1D + I2BD * I1A * I1C);
+    if (chis) acc += pref[z] * (nz > 1 ? trapz_weight(zs, z, nz) : 1.0) * T;
+    else out[(long long)z * n + e] = T;
+  }
+  if (chis) out[e] = acc;
+}
+
+// One thread per output element (i, j), all redshifts in increasing z
+__global__ void __launch_bounds__(256) trispec4h_assemble_kernel(int nz, int nk, int n1, int n2,
+                                                                 const double* __restrict__ ks,
+                                                                 const double* __restrict__ Pzk, const Legs2h L,
+                                                                 const double* __restrict__ q1,
+                                                                 const double* __restrict__ q2,
+                                                                 const double* __restrict__ zs,
+                                                                 const double* __restrict__ chis,
+                                                                 const double* __restrict__ pref, const PtSides s,
+                                                                 const double* __restrict__ F3,
+                                                                 double* __restrict__ out) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x, n = (long long)n1 * n2;
+  if (e >= n) return;
+  const int i = (int)(e / n2), j = (int)(e - (long long)i * n2);
+  const long long n1p = n1 + (n1 & 1), n2p = n2 + (n2 & 1);
+  const long long bB = (L.nA1 == 2 ? n1p : 0), bD = (L.nC1 == 2 ? n2p : 0);
+  const double F12 = F3[e], F21 = F3[n + e];
+  const bool local = chis ? pt_local(q1[i] + 0.5, q2[j] + 0.5) : pt_local(q1[i], q2[j]);
+  double acc = 0.0;
+  for (int z = 0; z < nz; ++z) {
+    const double* Ia = s.I1a + 2LL * z * n1p;
+    const double* Ic = s.I1c + 2LL * z * n2p;
+    const double inv_chi = chis ? 1.0 / chis[z] : 0.0;
+    const double k1 = chis ? (q1[i] + 0.5) * inv_chi : q1[i], k2 = chis ? (q2[j] + 0.5) * inv_chi : q2[j];
+    const double P1 = s.Pk1[(long long)z * n1 + i], P2 = s.Pk2[(long long)z * n2 + j];
+    double gp, g2p;
+    pt_averages(ks, Pzk + (long long)z * nk, s.tab + (long long)z * PT_NMOM * nk, nk, k1, k2, P1, P2, local, gp,
+                g2p);
+    const double Tb = 12.0 * P1 * P2 * (P2 * F12 + P1 * F21) + 8.0 * g2p;
+    const double T = Ia[i] * Ia[bB + i] * Ic[j] * Ic[bD + j] * Tb;
+    if (chis) acc += pref[z] * (nz > 1 ? trapz_weight(zs, z, nz) : 1.0) * T;
+    else out[(long long)z * n + e] = T;
+  }
+  if (chis) out[e] = acc;
+}
+
+// The checks shared by the 3- and 4-halo entry points (those of the 2-halo ones without zchunk); fills L
+static int trispec_pt_check(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                            const double* ms_d, const double* nzm_d, const double* bh_d, const double* Pzk_d,
+                            const double* const* u_h, const int* kind_h, int n1, const double* q1_d, int n2,
+                            const double* q2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                            const double* ws_d, const double* out_d, Legs2h& L) {
+  TrispecLegs L4;
+  const int chk = trispec_check(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, u_h, kind_h, n1, q1_d, n2, q2_d, zs_d,
+                                chis_d, pref_d, ws_d, out_d, L4);
+  if (chk) return chk;
+  for (int i = 0; i < 4; ++i) {
+    L.u[i] = L4.u[i];
+    L.matter[i] = L4.matter[i];
+  }
+  HMV_REQUIRE(bh_d && Pzk_d, "%s: null pointer (bh or Pzk)", who);
+  distinct_2h(u_h, kind_h, L.nA1, L.nC1);
+  return HMV_OK;
+}
+
+// 3-halo workspace: the 2-halo panels P1s P1p P2s P2p and the I2 block O22 of a pass, then its side vectors
+static long long trispec3h_ws(const Plan2h& p) {
+  return (long long)p.zc * (p.nmp * (p.m1s() + p.n1q + p.m2s() + p.n2q) + p.m1s() * p.m2s()) +
+         pt_sides_doubles(p.zc, p.nk, p.n1, p.n2);
+}
+
+static long long trispec3h_ws_doubles(int nz, int nm, int nk, int n1, int n2, const double* const* u_h,
+                                      const int* kind_h, int zchunk) {
+  if (nz <= 0 || nm <= 0 || nk < 2 || n1 <= 0 || n2 <= 0 || !u_h || !kind_h || zchunk < 1 || zchunk > nz) return 0;
+  int nA1, nC1;
+  distinct_2h(u_h, kind_h, nA1, nC1);
+  return trispec3h_ws(plan_2h(nm, nk, n1, n2, nA1, nC1, zchunk));
+}
+
+static int trispec3h_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                         const double* ms_d, const double* nzm_d, const double* bh_d, const double* Pzk_d,
+                         double rho_m0, const double* const* u_h, const int* kind_h, int n1, const double* q1_d, int n2,
+                         const double* q2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                         int zchunk, double* ws_d, double* out_d, void* stream) {
+  Legs2h L;
+  const int chk = trispec_pt_check(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, u_h, kind_h, n1, q1_d,
+                                   n2, q2_d, zs_d, chis_d, pref_d, ws_d, out_d, L);
+  if (chk) return chk;
+  HMV_REQUIRE(zchunk >= 1 && zchunk <= nz, "%s: zchunk must lie in [1, nz] (zchunk=%d nz=%d)", who, zchunk, nz);
+  const Plan2h full = plan_2h(nm, nk, n1, n2, L.nA1, L.nC1, zchunk);
+  const long long zc = zchunk;
+  double* P1s = ws_d;
+  double* P1p = P1s + zc * full.nmp * full.m1s();
+  double* P2s = P1p + zc * full.nmp * full.n1q;
+  double* P2p = P2s + zc * full.nmp * full.m2s();
+  double* O22 = P2p + zc * full.nmp * full.n2q;
+  const PtSides s = pt_sides(O22 + zc * full.m1s() * full.m2s(), zchunk, nk, n1, n2);
+  cudaStream_t st = (cudaStream_t)stream;
+  const double* chis = proj ? chis_d : nullptr;
+  const long long nout = (long long)n1 * n2;
+  for (int z0 = 0; z0 < nz; z0 += zchunk) {
+    const int zn = min(zchunk, nz - z0);
+    Plan2h p = full;
+    p.zc = zn;
+    int rc = pt_sides_run(z0, zn, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, L, n1, q1_d, n2, q2_d, chis, s,
+                          st);
+    if (rc) return rc;
+    // The 2-halo panel kernel, unchanged: of its outputs only P1s and P2s are read here.  Its P(k1), P(k2) go to the
+    // side kernel's Pk1, Pk2, rewriting them with the same bits (the same k_locate and k_lerp); P1p and P2p are unused.
+    dim3 pg(cdiv(p.n1q > p.n2q ? p.n1q : p.n2q, TP_T), zn, cdiv(p.nmp, TP_MROWS));
+    trispec2h_panel_kernel<<<pg, TP_T, 0, st>>>(z0, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, L, p, q1_d,
+                                                q2_d, chis, P1s, P1p, P2s, P2p, s.Pk1, s.Pk2);
+    rc = check_launch("trispec2h_panel_kernel");
+    if (rc) return rc;
+    rc = trispec_product(who, trispec_plan(false, zn, nm, (int)p.m1s(), (int)p.m2s()), (int)p.m1s(), P1s, P2s, O22,
+                         st);
+    if (rc) return rc;
+    trispec3h_assemble_kernel<<<cdiv(nout, 256), 256, 0, st>>>(z0, zn, nz, nk, ks_d, Pzk_d, p, q1_d, q2_d, zs_d, chis,
+                                                               pref_d, O22, s, z0 == 0, out_d);
+    rc = check_launch("trispec3h_assemble_kernel");
+    if (rc) return rc;
+  }
+  return HMV_OK;
+}
+
+static long long trispec4h_ws_doubles(int nz, int nk, int n1, int n2) {
+  if (nz <= 0 || nk < 2 || n1 <= 0 || n2 <= 0) return 0;
+  return pt_sides_doubles(nz, nk, n1, n2) + 2LL * n1 * n2;
+}
+
+static int trispec4h_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                         const double* ms_d, const double* nzm_d, const double* bh_d, const double* Pzk_d,
+                         double rho_m0, const double* const* u_h, const int* kind_h, int n1, const double* q1_d, int n2,
+                         const double* q2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                         double* ws_d, double* out_d, void* stream) {
+  Legs2h L;
+  const int chk = trispec_pt_check(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, u_h, kind_h, n1, q1_d,
+                                   n2, q2_d, zs_d, chis_d, pref_d, ws_d, out_d, L);
+  if (chk) return chk;
+  const PtSides s = pt_sides(ws_d, nz, nk, n1, n2);
+  double* F3 = ws_d + pt_sides_doubles(nz, nk, n1, n2);
+  cudaStream_t st = (cudaStream_t)stream;
+  const double* chis = proj ? chis_d : nullptr;
+  const long long nout = (long long)n1 * n2;
+  int rc = pt_sides_run(0, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, L, n1, q1_d, n2, q2_d, chis, s,
+                        st);
+  if (rc) return rc;
+  trispec4h_f3_kernel<<<cdiv(nout, 256), 256, 0, st>>>(n1, n2, q1_d, q2_d, proj, F3);
+  rc = check_launch("trispec4h_f3_kernel");
+  if (rc) return rc;
+  trispec4h_assemble_kernel<<<cdiv(nout, 256), 256, 0, st>>>(nz, nk, n1, n2, ks_d, Pzk_d, L, q1_d, q2_d, zs_d, chis,
+                                                             pref_d, s, F3, out_d);
+  return check_launch("trispec4h_assemble_kernel");
+}
 
 // ---- super-sample covariance (DESIGN.md §4.5) -------------------------------------------------------------------------
 //   sigma_b^2(z)        = sum_j kw_j P[z][j] W(k_j R_z)^2,  W(x) = 2 J1(x)/x, kw_j = s_j k_j/(2 pi) from the caller
@@ -675,6 +1188,58 @@ extern "C" int hmv_cl_cov_2h(int nz, int nm, int nk, int ldk, const double* ks_d
                              int zchunk, double* ws_d, double* out_d, void* stream) {
   return trispec2h_run("hmv_cl_cov_2h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, u_h, kind_h,
                        nl1, ells1_d, nl2, ells2_d, zs_d, chis_d, pref_d, zchunk, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_trispec_3h_ws_doubles(int nz, int nm, int nk, int nk1, int nk2, const double* const* u_h,
+                                                const int* kind_h, int zchunk) {
+  return trispec3h_ws_doubles(nz, nm, nk, nk1, nk2, u_h, kind_h, zchunk);
+}
+
+extern "C" int hmv_trispec_3h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                              const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0,
+                              const double* const* u_h, const int* kind_h, int nk1, const double* k1_d, int nk2,
+                              const double* k2_d, int zchunk, double* ws_d, double* out_d, void* stream) {
+  return trispec3h_run("hmv_trispec_3h", false, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, u_h, kind_h,
+                       nk1, k1_d, nk2, k2_d, nullptr, nullptr, nullptr, zchunk, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_cl_cov_3h_ws_doubles(int nz, int nm, int nk, int nl1, int nl2, const double* const* u_h,
+                                               const int* kind_h, int zchunk) {
+  return trispec3h_ws_doubles(nz, nm, nk, nl1, nl2, u_h, kind_h, zchunk);
+}
+
+extern "C" int hmv_cl_cov_3h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                             const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0,
+                             const double* const* u_h, const int* kind_h, int nl1, const double* ells1_d, int nl2,
+                             const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                             int zchunk, double* ws_d, double* out_d, void* stream) {
+  return trispec3h_run("hmv_cl_cov_3h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, u_h, kind_h,
+                       nl1, ells1_d, nl2, ells2_d, zs_d, chis_d, pref_d, zchunk, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_trispec_4h_ws_doubles(int nz, int nk, int nk1, int nk2) {
+  return trispec4h_ws_doubles(nz, nk, nk1, nk2);
+}
+
+extern "C" int hmv_trispec_4h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                              const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0,
+                              const double* const* u_h, const int* kind_h, int nk1, const double* k1_d, int nk2,
+                              const double* k2_d, double* ws_d, double* out_d, void* stream) {
+  return trispec4h_run("hmv_trispec_4h", false, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, u_h, kind_h,
+                       nk1, k1_d, nk2, k2_d, nullptr, nullptr, nullptr, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_cl_cov_4h_ws_doubles(int nz, int nk, int nl1, int nl2) {
+  return trispec4h_ws_doubles(nz, nk, nl1, nl2);
+}
+
+extern "C" int hmv_cl_cov_4h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                             const double* nzm_d, const double* bh_d, const double* Pzk_d, double rho_m0,
+                             const double* const* u_h, const int* kind_h, int nl1, const double* ells1_d, int nl2,
+                             const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                             double* ws_d, double* out_d, void* stream) {
+  return trispec4h_run("hmv_cl_cov_4h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, bh_d, Pzk_d, rho_m0, u_h, kind_h,
+                       nl1, ells1_d, nl2, ells2_d, zs_d, chis_d, pref_d, ws_d, out_d, stream);
 }
 
 extern "C" int hmv_sigma_b2(int nz, int nks, const double* ks_d, const double* kw_d, const double* P_d,

@@ -998,9 +998,11 @@ class HaloModel(Cosmology):
     # Workspace budget of one 2-halo call, in doubles (8 GiB): the largest number of redshifts per pass that fits
     _TRISPEC_2H_WS_BUDGET = 1 << 30
 
-    def _trispec2h_call(self, fn, names, q1, q2, extra, out_shape):
-        cubes, kinds = self._trispec_legs(names, "2-halo trispectrum",
-                                          "needs occupation moments up to third order, which the HOD does not define")
+    def _trispec2h_call(self, fn, names, q1, q2, extra, out_shape, what="2-halo trispectrum",
+                        hod_why="needs occupation moments up to third order, which the HOD does not define",
+                        budget=None):
+        budget = self._TRISPEC_2H_WS_BUDGET if budget is None else budget
+        cubes, kinds = self._trispec_legs(names, what, hod_why)
         nz, nm = self._nz, self._nm
         u_h = (C.c_void_p * 4)(*[c.data_ptr() for c in cubes])
         k_h = (C.c_int * 4)(*kinds)
@@ -1008,7 +1010,7 @@ class HaloModel(Cosmology):
         lo, hi = 1, nz                   # the workspace grows with zchunk: the largest zchunk within the budget
         while lo < hi:
             mid = (lo + hi + 1) // 2
-            if size(nz, nm, self._nk, q1.size, q2.size, u_h, k_h, mid) <= self._TRISPEC_2H_WS_BUDGET:
+            if size(nz, nm, self._nk, q1.size, q2.size, u_h, k_h, mid) <= budget:
                 lo = mid
             else:
                 hi = mid - 1
@@ -1067,6 +1069,98 @@ class HaloModel(Cosmology):
         pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
         extra = (self._zs_d, self._dev(chis), self._dev(pref))
         return self._trispec2h_call('hmv_cl_cov_2h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+
+    # ------------------------------------------------------------------ 3- and 4-halo trispectra and C_l covariance
+    # Workspace budget of one 3-halo call, in doubles (8 GiB): the largest number of redshifts per pass that fits
+    _TRISPEC_3H_WS_BUDGET = 1 << 30
+    _PT_HOD_WHY = "is not implemented for HOD tracers (matter and pressure profiles only)"
+
+    def _trispec4h_call(self, fn, names, q1, q2, extra, out_shape):
+        cubes, kinds = self._trispec_legs(names, "4-halo trispectrum", self._PT_HOD_WHY)
+        nz, nm = self._nz, self._nm
+        ws = self._workspace('trispec', getattr(capi.lib, fn + '_ws_doubles')(nz, self._nk, q1.size, q2.size))
+        out = self._empty(*out_shape)
+        q1_d, q2_d = self._dev(q1), self._dev(q2)
+        u_h = (C.c_void_p * 4)(*[c.data_ptr() for c in cubes])
+        capi.check(getattr(capi.lib, fn)(nz, nm, self._nk, self._ldk, capi.ptr(self._ks_d), capi.ptr(self._ms_d),
+                                         capi.ptr(self._nzm_d), capi.ptr(self._bh_d), capi.ptr(self._Pzk_d),
+                                         self._rho_m0, u_h, (C.c_int * 4)(*kinds), q1.size, capi.ptr(q1_d), q2.size,
+                                         capi.ptr(q2_d), *[capi.ptr(e) for e in extra], capi.ptr(ws), capi.ptr(out),
+                                         capi.stream()),
+                   fn)
+        return self._host(out)
+
+    def _pt_args(self, ks1, ks2, name, name2, name3, name4):
+        name2 = name if name2 is None else name2
+        name3 = name if name3 is None else name3
+        name4 = name3 if name4 is None else name4
+        k1 = self._positive(ks1, "ks1")
+        k2 = k1 if ks2 is None else self._positive(ks2, "ks2")
+        return (name, name2, name3, name4), k1, k2
+
+    def _pt_cov_args(self, what, ells, name, name2, name3, name4, windows, fsky, ells2):
+        if self._zcomm is not None:
+            raise NotImplementedError("%s on a z-sharded model: the z sum spans the ranks" % what)
+        names, l1, l2 = self._pt_args(ells, ells2, name, name2, name3, name4)
+        fsky = self._fsky(fsky)
+        W = self._window_product(windows)
+        chis = np.asarray(self.comoving_radial_distance(self.zs), dtype=np.float64).reshape(-1)
+        H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
+        pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
+        return names, l1, l2, (self._zs_d, self._dev(chis), self._dev(pref))
+
+    def get_trispectrum_3halo(self, ks1, ks2=None, name="nfw", name2=None, name3=None, name4=None):
+        """3-halo trispectrum of T(k1, -k1, k2, -k2) averaged over mu = k1^.k2^, [nz, nk1, nk2]:
+
+            Bbar(k1,k2) [I2^{AC} I1~B I1~D + I2^{AD} I1~B I1~C + I2^{BC} I1~A I1~D + I2^{BD} I1~A I1~C]
+            Bbar = (34/21) P(k1) P(k2) + 2 <G P(|k1+k2|)>,  G = P(k1) F2(-k1, k1+k2) + P(k2) F2(-k2, k1+k2)
+
+        No counterpart in the reference (Cooray & Hu 2001, ApJ 554, 56).  Bbar is the angle-averaged tree-level
+        bispectrum with the pairings that carry P(0) dropped; <.> = (1/2) int dmu, exact for P linear on `ks` (held at
+        its end values outside).  I2 and I1~ as in get_trispectrum_2halo (I2 carries no consistency term).  Legs,
+        names, defaults and k handling as get_trispectrum_2halo; HODs raise ValueError.  The redshifts run in passes
+        whose workspace fits _TRISPEC_3H_WS_BUDGET doubles; the result does not depend on the pass size."""
+        names, k1, k2 = self._pt_args(ks1, ks2, name, name2, name3, name4)
+        return self._trispec2h_call('hmv_trispec_3h', names, k1, k2, (), (self._nz, k1.size, k2.size),
+                                    "3-halo trispectrum", self._PT_HOD_WHY, self._TRISPEC_3H_WS_BUDGET)
+
+    def get_cl_cov_3halo(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
+                         ells2=None):
+        """Non-Gaussian 3-halo Limber covariance Cov(C_l^{AB}, C_l'^{CD}), [len(ells), len(ells2)]:
+
+            1/(4 pi fsky) sum_z zeta_z H^3 W_A W_B W_C W_D / chi^6 T3h^{ABCD}((l+1/2)/chi, (l'+1/2)/chi; z)
+
+        with T3h from get_trispectrum_3halo and the projection, windows, names and defaults of get_cl_cov_1halo.  Not
+        available on a z-sharded model (the z sum would need a cross-rank reduction)."""
+        names, l1, l2, extra = self._pt_cov_args("get_cl_cov_3halo", ells, name, name2, name3, name4, windows, fsky,
+                                                 ells2)
+        return self._trispec2h_call('hmv_cl_cov_3h', names, l1, l2, extra, (l1.size, l2.size), "3-halo trispectrum",
+                                    self._PT_HOD_WHY, self._TRISPEC_3H_WS_BUDGET)
+
+    def get_trispectrum_4halo(self, ks1, ks2=None, name="nfw", name2=None, name3=None, name4=None):
+        """4-halo trispectrum of T(k1, -k1, k2, -k2) averaged over mu = k1^.k2^, [nz, nk1, nk2]:
+
+            I1~A(k1) I1~B(k1) I1~C(k2) I1~D(k2) Tbar(k1,k2)
+            Tbar = 12 P1 P2^2 F3bar(k2/k1) + 12 P1^2 P2 F3bar(k1/k2) + 8 <G^2 P(|k1+k2|)>
+
+        No counterpart in the reference (Cooray & Hu 2001, ApJ 554, 56).  Tbar is the angle-averaged tree-level
+        trispectrum with the pairings that carry P(0) dropped; F3bar(r) = <F3_sym(k, q, -q)>, r = q/k; G and <.> as in
+        get_trispectrum_3halo; I1~ as in get_trispectrum_2halo.  Legs, names, defaults and k handling as
+        get_trispectrum_2halo; HODs raise ValueError."""
+        names, k1, k2 = self._pt_args(ks1, ks2, name, name2, name3, name4)
+        return self._trispec4h_call('hmv_trispec_4h', names, k1, k2, (), (self._nz, k1.size, k2.size))
+
+    def get_cl_cov_4halo(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
+                         ells2=None):
+        """Non-Gaussian 4-halo Limber covariance Cov(C_l^{AB}, C_l'^{CD}), [len(ells), len(ells2)]:
+
+            1/(4 pi fsky) sum_z zeta_z H^3 W_A W_B W_C W_D / chi^6 T4h^{ABCD}((l+1/2)/chi, (l'+1/2)/chi; z)
+
+        with T4h from get_trispectrum_4halo and the projection, windows, names and defaults of get_cl_cov_1halo.  Not
+        available on a z-sharded model (the z sum would need a cross-rank reduction)."""
+        names, l1, l2, extra = self._pt_cov_args("get_cl_cov_4halo", ells, name, name2, name3, name4, windows, fsky,
+                                                 ells2)
+        return self._trispec4h_call('hmv_cl_cov_4h', names, l1, l2, extra, (l1.size, l2.size))
 
     @staticmethod
     def _fsky(fsky):

@@ -346,6 +346,46 @@ int hmv_cl_cov_2h(int nz, int nm, int nk, int ldk, const double* ks_d, const dou
                   int nl1, const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
                   const double* chis_d, const double* pref_d, int zchunk, double* ws_d, double* out_d, void* stream);
 
+/* ---- 3- and 4-halo trispectra and their non-Gaussian Limber covariance of C_l (DESIGN.md §4.7) ----------------------
+ * No counterpart in the reference.  Cooray & Hu 2001, ApJ 554, 56; Takada & Jain 2009, MNRAS 395, 2065.  Legs, kinds,
+ * w^, I1~X, I2^{XY}, P and the projection as in hmv_trispec_2h / hmv_cl_cov_2h; P1 = P(k1), P2 = P(k2).  For
+ * T(k1,-k1,k2,-k2) averaged over mu = k1^.k2^ (<.> = (1/2) int_{-1}^{1} dmu), q = |k1 + k2|:
+ *   G(mu)        = P1 F2(-k1, k1+k2) + P2 F2(-k2, k1+k2),  F2 the symmetric second-order PT kernel
+ *   F3bar(r)     = <F3_sym(k, q', -q')>, r = q'/k (the P13 kernel divided by 3024 r^2)
+ *   Bbar(k1,k2)  = (34/21) P1 P2 + 2 <G P(q)>
+ *   Tbar(k1,k2)  = 12 P1 P2^2 F3bar(k2/k1) + 12 P1^2 P2 F3bar(k1/k2) + 8 <G^2 P(q)>
+ *   T3h(k1,k2;z) = Bbar [I2^{AC} I1~B I1~D + I2^{AD} I1~B I1~C + I2^{BC} I1~A I1~D + I2^{BD} I1~A I1~C]
+ *   T4h(k1,k2;z) = I1~A I1~B I1~C I1~D Tbar
+ * Terms carrying P(0) are dropped.  <G P> and <G^2 P> are exact for P piecewise linear (per-redshift moment tables of
+ * int q^n P dq, n = -3, -1, 1, 3, 5); ks must be positive and k1, k2 > 0.  hmv_*_3h: zchunk and the workspace as in
+ * hmv_trispec_2h, with 1, 2 or 4 contracted I2 blocks (A == B and C == D, one of them, neither).  hmv_*_4h: one pass,
+ * no contraction; the workspace depends on the sizes only.  The workspace functions return 0 on invalid sizes or
+ * zchunk.  Argument checks, codes and messages as hmv_trispec_2h, all before the first launch; the result is
+ * bit-identical for every zchunk and for repeated calls.  hmv_trispec_3h/4h: out_d [nz][nk1][nk2];
+ * hmv_cl_cov_3h/4h: out_d [nl1][nl2]. */
+long long hmv_trispec_3h_ws_doubles(int nz, int nm, int nk, int nk1, int nk2, const double* const* u_h,
+                                    const int* kind_h, int zchunk);
+int hmv_trispec_3h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                   const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                   int nk1, const double* k1_d, int nk2, const double* k2_d, int zchunk, double* ws_d, double* out_d,
+                   void* stream);
+long long hmv_cl_cov_3h_ws_doubles(int nz, int nm, int nk, int nl1, int nl2, const double* const* u_h,
+                                   const int* kind_h, int zchunk);
+int hmv_cl_cov_3h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                  const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                  int nl1, const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                  const double* chis_d, const double* pref_d, int zchunk, double* ws_d, double* out_d, void* stream);
+long long hmv_trispec_4h_ws_doubles(int nz, int nk, int nk1, int nk2);
+int hmv_trispec_4h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                   const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                   int nk1, const double* k1_d, int nk2, const double* k2_d, double* ws_d, double* out_d,
+                   void* stream);
+long long hmv_cl_cov_4h_ws_doubles(int nz, int nk, int nl1, int nl2);
+int hmv_cl_cov_4h(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d, const double* nzm_d,
+                  const double* bh_d, const double* Pzk_d, double rho_m0, const double* const* u_h, const int* kind_h,
+                  int nl1, const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                  const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream);
+
 /* ---- super-sample covariance of C_l (matter and pressure profiles) ---------------------------------------------------
  * No counterpart in the reference.  Takada & Hu 2013, PRD 87, 123504; Li, Hu & Takada 2014, PRD 89, 083519.  Legs t_X
  * and kinds as in hmv_trispec_1h (0: matter, a = M/rho_m0; 2: pressure, a = 1); w_m the trapezoid weight on ms.
