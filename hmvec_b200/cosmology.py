@@ -472,14 +472,28 @@ def _upload_many(arrays, device):
     return [d[o:o + a.size] for a, o in zip(arrays, offs)]
 
 
+def _sort_order(x, name):
+    """None when x is strictly increasing, else the permutation that sorts it; repeated values are an error."""
+    if np.all(np.diff(x) > 0):
+        return None
+    order = np.argsort(x, kind="stable")
+    if not np.all(np.diff(x[order]) > 0):
+        raise ValueError("limber_integral: %s must not hold repeated values" % name)
+    return order
+
+
 def limber_integral(ells, zs, ks, Pzks, gzs, Wz1s, Wz2s, hzs, chis, device=None):
     r"""C(ell) = \int dz (H(z)/c) W1(z) W2(z) P(z, k=(ell+1/2)/chi) / chi^2   (cosmology.py:867-904) on the device.
 
-    Pzks may be a numpy array [npzs,nk] or a CUDA tensor of that shape (kept on the device after an all-gather)."""
-    device = torch.device(device) if device is not None else _default_device()
+    Pzks may be a numpy array [npzs,nk] or a CUDA tensor of that shape (kept on the device after an all-gather).
+    ks and zs may come in any order (a HaloModel on shuffled ks hands out spectra in that order): the kernel looks
+    them up by binary search, so they are sorted here and the table's columns and rows permuted to match, as the
+    reference's interp2d does.  The window redshifts gzs are integrated over in the order given."""
     ells = np.asarray(ells, dtype=np.float64).reshape(-1)
     zs = np.asarray(zs, dtype=np.float64).reshape(-1)
     ks = np.asarray(ks, dtype=np.float64).reshape(-1)
+    kord, zord = _sort_order(ks, "ks"), _sort_order(zs, "zs")
+    device = torch.device(device) if device is not None else _default_device()
     gzs = np.asarray(gzs, dtype=np.float64).reshape(-1)
     hzs = np.array(hzs, dtype=np.float64).reshape(-1)
     chis = np.array(chis, dtype=np.float64).reshape(-1)
@@ -498,6 +512,14 @@ def limber_integral(ells, zs, ks, Pzks, gzs, Wz1s, Wz2s, hzs, chis, device=None)
         P_d.copy_(h, non_blocking=h.is_pinned())
     if P_d.dim() != 2 or P_d.shape[0] != zs.size or P_d.shape[1] != ks.size:
         raise ValueError("Pzks must have shape (zs.size, ks.size)")
+    if kord is not None or zord is not None:
+        # one gather on the device puts the table in the sorted (z, k) order
+        zi = np.arange(zs.size) if zord is None else zord
+        ki = np.arange(ks.size) if kord is None else kord
+        idx = torch.from_numpy((zi[:, None] * ks.size + ki[None, :]).reshape(-1)).to(device)
+        capi.count_h2d(idx.numel() * 8)
+        P_d = P_d.reshape(-1).index_select(0, idx).view(zs.size, ks.size)
+        zs, ks = zs[zi], ks[ki]
     out = torch.empty(ells.size, dtype=torch.float64, device=device)
     # keep every temporary alive until the launch has been issued (the caching allocator may otherwise recycle it)
     ells_d, zs_d, ks_d, gzs_d, pref_d, chis_d = _upload_many((ells, zs, ks, gzs, pref, chis), device)

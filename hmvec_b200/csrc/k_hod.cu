@@ -185,7 +185,8 @@ __global__ void hod_bisect_pick_kernel(int nz, const double* __restrict__ ys,
 static int hod_smem(int nm, size_t* bytes) {
   *bytes = ((size_t)NTAB + 2 * (size_t)nm + 32) * sizeof(double);
   if (*bytes > 200 * 1024)
-    return fail(HMV_E_LIMIT, "HOD kernels stage 2*nm doubles in shared memory: nm=%d too large (max ~10000)", nm);
+    return fail(HMV_E_LIMIT, "HOD kernels stage %d + 2*nm + 32 doubles (at most 200 KiB) in shared memory: nm=%d too "
+                "large (max 10784)", NTAB, nm);
   return HMV_OK;
 }
 

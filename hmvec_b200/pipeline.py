@@ -92,6 +92,12 @@ class GridSix(object):
         tsz_tables (default): the Compton-y profile stays in the transform's bin tables (hmv_profile_tables) and P_yy is
         reduced straight from them (hmv_power_tab) -- its 32 GB cube is never written or read (measured 3.0 vs 4.6 ms on
         a 64-z slab); False materialises the cube (hmv_profile_transform + hmv_power) as every other consumer needs."""
+        if "ells" in inp:
+            # hmv_limber_multi binary-searches ks and the table's redshifts; sorting them here would cost a gather of
+            # the packed table every step, so a Limber grid must come sorted
+            for name, x in (("ks", inp["ks"]), ("zs", inp["zs"] if nz_total_zs is None else nz_total_zs)):
+                if not np.all(np.diff(np.asarray(x, dtype=np.float64).reshape(-1)) > 0):
+                    raise ValueError("GridSix with ells: %s must be strictly increasing" % name)
         if not torch.cuda.is_available():
             raise RuntimeError("hmvec_b200 needs a CUDA device (B200, sm_100a): there is no CPU fallback.")
         self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())

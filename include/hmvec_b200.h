@@ -231,13 +231,17 @@ int hmv_power_six_nfw(int nz, int nm, int nk, int ldk, const double* zs_d, const
 /* ---- a16: Limber integral  (cosmology.py:867-904) ---------------------------------------------------
  * C_l = trapz_gz( pref[gz] * P(k=(l+1/2)/chi[gz], gz) )  (ngz>1) or pref*P (ngz==1); P by bilinear
  * interpolation in linear (k,z) with out-of-range coordinates clamped to the table edge. pref = H W1 W2/chi^2.
- * P2_d: optional second [nzp][ldp] table added to P_d at lookup (P = P1h + P2h without a temporary), or NULL. */
+ * P2_d: optional second [nzp][ldp] table added to P_d at lookup (P = P1h + P2h without a temporary), or NULL.
+ * ks_d [nk] and the table's redshifts zs_d [nzp] must be strictly increasing (both are binary-searched; unsorted axes
+ * give wrong C_l without an error).  The window redshifts gzs_d may come in either order: the trapezoid follows them,
+ * so a decreasing gzs gives -C_l, as numpy.trapz does. */
 int hmv_limber(int nl, const double* ells_d, int nzp, int nk, int ldp, const double* zs_d, const double* ks_d,
                const double* P_d, const double* P2_d, int ngz, const double* gzs_d, const double* pref_d,
                const double* chis_d, double* cl_d, void* stream);
 
 /* The same for up to HMV_LIMBER_MAXJOBS projections of tables that share the (zs, ks) grid and the multipoles, in one
- * launch (C_kk, C_kg, C_yy of one step: cosmology.py:536-597).  jobs_h: HOST array; fields as in hmv_limber. */
+ * launch (C_kk, C_kg, C_yy of one step: cosmology.py:536-597).  jobs_h: HOST array; fields as in hmv_limber, and
+ * ks_d and zs_d strictly increasing as there. */
 #define HMV_LIMBER_MAXJOBS 4
 typedef struct hmv_limber_job {
   const double* P_d;     /* [nzp][ldp] table */
