@@ -88,6 +88,11 @@ _SIGS = {
     "hmv_cl_cov_1h_ws_doubles": (_ll, [_i, _i, _i, _i]),
     "hmv_cl_cov_1h": (_i, [_i, _i, _i, _i, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _p, _p, _p,
                            _p, _p, _p]),
+    "hmv_trispec_1h_tracers_ws_doubles": (_ll, [_i, _i, _i, _i, C.POINTER(Tracer)]),
+    "hmv_trispec_1h_tracers": (_i, [_i, _i, _i, _i, _p, _p, _p, _d, C.POINTER(Tracer), _i, _p, _i, _p, _p, _p, _p]),
+    "hmv_cl_cov_1h_tracers_ws_doubles": (_ll, [_i, _i, _i, _i, C.POINTER(Tracer)]),
+    "hmv_cl_cov_1h_tracers": (_i, [_i, _i, _i, _i, _p, _p, _p, _d, C.POINTER(Tracer), _i, _p, _i, _p, _p, _p, _p, _p,
+                                   _p, _p]),
     "hmv_trispec_2h_ws_doubles": (_ll, [_i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_i), _i]),
     "hmv_trispec_2h": (_i, [_i, _i, _i, _i, _p, _p, _p, _p, _p, _d, C.POINTER(_p), C.POINTER(_i), _i, _p, _i, _p, _i,
                             _p, _p, _p]),

@@ -8,7 +8,8 @@
 // Both are one FP64 contraction over K = (z, m): a panel kernel writes P1[K][l] = w_m n (zeta pref) t_A t_B at k1 and
 // P2[K][l'] = t_C t_D at k2, and sigma2_gemm_kernel<MT, A K-major> forms C = P1^T P2 on the tensor pipe -- over all of
 // K with a fixed-order split-k reduction for the covariance, batched over z (K = m, one batch item per split index)
-// for the trispectrum.  A last kernel sums the splits in a fixed order and drops the padding column.
+// for the trispectrum.  A last kernel sums the splits in a fixed order and drops the padding column.  Galaxy (HOD) legs
+// of the 1-halo term (DESIGN.md §4.8) have their own panel kernel and feed the same contraction.
 // The super-sample covariance (DESIGN.md §4.5) reuses the projection with K = z; sigma_b^2 of a disc is here too.
 // The 2-halo trispectrum and its covariance (DESIGN.md §4.6) run the trispectrum's batched product three times per pass
 // of redshifts and combine the blocks per (z, k1, k2) with P_lin and its angle average; see the section below.
@@ -102,7 +103,7 @@ __global__ void trispec_reduce_kernel(long long n, int ns, int n1, int n2, int l
 // ---- launch plan: a function of the shapes only, so that the workspace size and the launch agree ----------------------
 struct TrispecPlan {
   int mt;               // 8*mt output rows per CTA
-  int nmp, ld1, ld2;    // mass rows and panel widths, padded to even
+  int nmp, ld1, ld2;    // rows per redshift (nseg segments of the even-padded mass rows) and panel widths, padded to even
   long long K;          // nz * nmp
   int kchunk, nsplit;   // K range of one split index, split indices per batch item
   int nbatch;           // 1 (covariance) or nz (trispectrum)
@@ -138,9 +139,10 @@ static TrispecPlan split_k(TrispecPlan p, int n1) {
   return p;
 }
 
-static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2) {
-  TrispecPlan p = base_plan(nz, nm + (nm & 1), n1, n2);
-  if (!proj) {                       // one batch item per redshift: its K range is its nmp mass rows
+// nseg: segments of mass rows per redshift (2 for the split galaxy pair of the tracer panels, else 1)
+static TrispecPlan trispec_plan(bool proj, int nz, int nm, int n1, int n2, int nseg = 1) {
+  TrispecPlan p = base_plan(nz, nseg * (nm + (nm & 1)), n1, n2);
+  if (!proj) {                       // one batch item per redshift: its K range is its nmp rows
     p.kchunk = p.nmp;
     p.nsplit = 1;
     p.nbatch = nz;
@@ -153,9 +155,9 @@ static long long trispec_ws(const TrispecPlan& p, int n1) {
   return p.K * (p.ld1 + p.ld2) + (long long)p.nbatch * p.nsplit * n1 * p.ld2;
 }
 
-static long long trispec_ws_doubles(bool proj, int nz, int nm, int n1, int n2) {
+static long long trispec_ws_doubles(bool proj, int nz, int nm, int n1, int n2, int nseg = 1) {
   if (nz <= 0 || nm <= 0 || n1 <= 0 || n2 <= 0) return 0;
-  return trispec_ws(trispec_plan(proj, nz, nm, n1, n2), n1);
+  return trispec_ws(trispec_plan(proj, nz, nm, n1, n2, nseg), n1);
 }
 
 template <int MT>
@@ -196,30 +198,48 @@ static int trispec_contract(const char* who, const TrispecPlan& p, int n1, int n
   return check_launch("trispec_reduce_kernel");
 }
 
-// The argument checks of every trispectrum entry point (1- and 2-halo), made before any launch; fills L.
+// The size, pointer and limit checks shared by every trispectrum entry point, made before any launch.  check_legs() runs
+// between the pointer and the limit checks and sets nseg, the segments of mass rows per redshift that K counts.
+template <class LegCheck>
+static int trispec_check_args(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                              const double* ms_d, const double* nzm_d, bool legs, int n1, const double* q1_d, int n2,
+                              const double* q2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                              const double* ws_d, const double* out_d, int& nseg, LegCheck check_legs) {
+  HMV_REQUIRE(nz >= 1 && nm >= 1 && nk >= 2 && n1 >= 1 && n2 >= 1,
+              "%s: sizes must be >= 1 and nk >= 2 (nz=%d nm=%d nk=%d n1=%d n2=%d)", who, nz, nm, nk, n1, n2);
+  HMV_REQUIRE(ldk >= nk && (ldk & 1) == 0, "%s: ldk must be even and >= nk (ldk=%d nk=%d)", who, ldk, nk);
+  HMV_REQUIRE(ks_d && ms_d && nzm_d && legs && q1_d && q2_d && ws_d && out_d, "%s: null pointer", who);
+  HMV_REQUIRE(!proj || (zs_d && chis_d && pref_d), "%s: null pointer (zs, chis or pref)", who);
+  nseg = 1;
+  const int rc = check_legs();
+  if (rc) return rc;
+  HMV_REQUIRE(((size_t)ws_d & 15) == 0, "%s: workspace must be 16-byte aligned", who);
+  if (nz > 65535) return fail(HMV_E_LIMIT, "%s: nz=%d exceeds 65535 (grid y of the panel kernel)", who, nz);
+  const long long K = (long long)nz * nseg * (nm + (nm & 1));
+  if (K > (1LL << 30))
+    return fail(HMV_E_LIMIT, "%s: nz * nm%s = %lld exceeds 2^30 (32-bit k index of the contraction)", who,
+                nseg > 1 ? " * segments" : "", K);
+  return HMV_OK;
+}
+
+// The argument checks of every profile-leg trispectrum entry point (1- to 4-halo), made before any launch; fills L.
 static int trispec_check(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
                          const double* ms_d, const double* nzm_d, const double* const* u_h, const int* kind_h, int n1,
                          const double* q1_d, int n2, const double* q2_d, const double* zs_d, const double* chis_d,
                          const double* pref_d, const double* ws_d, const double* out_d, TrispecLegs& L) {
-  HMV_REQUIRE(nz >= 1 && nm >= 1 && nk >= 2 && n1 >= 1 && n2 >= 1,
-              "%s: sizes must be >= 1 and nk >= 2 (nz=%d nm=%d nk=%d n1=%d n2=%d)", who, nz, nm, nk, n1, n2);
-  HMV_REQUIRE(ldk >= nk && (ldk & 1) == 0, "%s: ldk must be even and >= nk (ldk=%d nk=%d)", who, ldk, nk);
-  HMV_REQUIRE(ks_d && ms_d && nzm_d && u_h && kind_h && q1_d && q2_d && ws_d && out_d, "%s: null pointer", who);
-  HMV_REQUIRE(!proj || (zs_d && chis_d && pref_d), "%s: null pointer (zs, chis or pref)", who);
-  for (int i = 0; i < 4; ++i) {
-    HMV_REQUIRE(u_h[i], "%s: null pointer (cube %d)", who, i);
-    HMV_REQUIRE(kind_h[i] == 0 || kind_h[i] == 2, "%s: cube %d: kind %d is neither 0 (matter) nor 2 (pressure)", who, i,
-                kind_h[i]);
-    HMV_REQUIRE(((size_t)u_h[i] & 15) == 0, "%s: cube %d must be 16-byte aligned", who, i);
-    L.u[i] = u_h[i];
-    L.matter[i] = kind_h[i] == 0;
-  }
-  HMV_REQUIRE(((size_t)ws_d & 15) == 0, "%s: workspace must be 16-byte aligned", who);
-  if (nz > 65535) return fail(HMV_E_LIMIT, "%s: nz=%d exceeds 65535 (grid y of the panel kernel)", who, nz);
-  const long long K = (long long)nz * (nm + (nm & 1));
-  if (K > (1LL << 30))
-    return fail(HMV_E_LIMIT, "%s: nz * nm = %lld exceeds 2^30 (32-bit k index of the contraction)", who, K);
-  return HMV_OK;
+  int nseg;
+  return trispec_check_args(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, u_h && kind_h, n1, q1_d, n2, q2_d, zs_d,
+                            chis_d, pref_d, ws_d, out_d, nseg, [&]() -> int {
+    for (int i = 0; i < 4; ++i) {
+      HMV_REQUIRE(u_h[i], "%s: null pointer (cube %d)", who, i);
+      HMV_REQUIRE(kind_h[i] == 0 || kind_h[i] == 2, "%s: cube %d: kind %d is neither 0 (matter) nor 2 (pressure)", who,
+                  i, kind_h[i]);
+      HMV_REQUIRE(((size_t)u_h[i] & 15) == 0, "%s: cube %d must be 16-byte aligned", who, i);
+      L.u[i] = u_h[i];
+      L.matter[i] = kind_h[i] == 0;
+    }
+    return HMV_OK;
+  });
 }
 
 static int trispec_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
@@ -243,7 +263,210 @@ static int trispec_run(const char* who, bool proj, int nz, int nm, int nk, int l
   return trispec_contract(who, p, n1, n2, P1, P2, part, out_d, st);
 }
 
-// ---- 2-halo trispectrum (DESIGN.md §4.6) -------------------------------------------------------------------------------
+// ---- 1-halo trispectrum with galaxy (HOD) legs (DESIGN.md §4.8) ------------------------------------------------------
+// A galaxy leg is t_g = (Nc u_c + Ns u_s)/ngal (u_c = 1 without a central profile), hmv_power's HOD leg.  Two galaxy
+// legs in one halo take the pair moment without self-pairs,
+//   <g g>(k, k') = [NsNsm1 u_s(k) u_s(k') + NcNs (u_c(k) u_s(k') + u_s(k) u_c(k'))] / ngal^2,
+// so that with both on one side the panel column is w n <g g>(k, k) (hmv_power's form-1 integrand) and the panels stay
+// rank-1.  With one on each side (legs g X at k1, g Y at k2) <g g>(k1, k2) has rank 2 and each redshift gets two
+// segments of mass rows, K = (z, segment, m):
+//   segment 0:  P1 = w n u_s t_X / ngal^2 (k1)           P2 = (NsNsm1 u_s + NcNs u_c) t_Y (k2)
+//   segment 1:  P1 = w n NcNs u_c t_X / ngal^2 (k1)      P2 = u_s t_Y (k2)
+// Three or four galaxy legs need higher occupation moments than the HOD defines and are refused.
+struct TracerLegs {
+  const double* us[4];
+  const double* uc[4];                            // kind 1: central profile or null (u_c = 1)
+  int kind[4];
+  const double *Nc, *Ns, *NcNs, *NsNsm1, *ngal;   // the one HOD of the kind-1 legs
+  int pair1, pair2;                               // 1: both legs of side 1 (A, B) / side 2 (C, D) are galaxies
+  int g1, g2;                                     // split pair: the galaxy leg of side 1 (0, 1) and side 2 (2, 3); else -1
+};
+
+// u_s and u_c of leg x at (row, j, f)
+__device__ __forceinline__ void hod_profiles(const TracerLegs& L, int x, long long row, int j, double f, double& us,
+                                             double& uc) {
+  us = k_lerp(L.us[x] + row, j, f);
+  uc = L.uc[x] ? k_lerp(L.uc[x] + row, j, f) : 1.0;
+}
+
+// t_x at (row, j, f) of mass element i: a u_s (kind 0 a = M/rho_m0, kind 2 a = 1) or (Nc u_c + Ns u_s)/ngal
+__device__ __forceinline__ double tracer_leg(const TracerLegs& L, int x, long long i, long long row, int j, double f,
+                                             double a, double ig) {
+  if (L.kind[x] == 1) {
+    double us, uc;
+    hod_profiles(L, x, row, j, f, us, uc);
+    return (L.Nc[i] * uc + L.Ns[i] * us) * ig;
+  }
+  return (L.kind[x] == 0 ? a : 1.0) * k_lerp(L.us[x] + row, j, f);
+}
+
+// t_x t_{x+1} of one side, or the pair moment <g g>(k, k) = u_s (2 NcNs u_c + NsNsm1 u_s)/ngal^2 when both are galaxies
+__device__ __forceinline__ double tracer_side(const TracerLegs& L, int x, int pair, long long i, long long row, int j,
+                                              double f, double a, double ig) {
+  if (pair) {
+    double us, uc;
+    hod_profiles(L, x, row, j, f, us, uc);
+    return us * (2.0 * L.NcNs[i] * uc + L.NsNsm1[i] * us) * (ig * ig);
+  }
+  return tracer_leg(L, x, i, row, j, f, a, ig) * tracer_leg(L, x + 1, i, row, j, f, a, ig);
+}
+
+// trispec_panel_kernel for tracer legs: the same grid, columns and padding, with nseg (1 or 2) segments of nmp rows per
+// redshift; the split pair (L.g1 >= 0) writes both segments of a mass row from one pair of interval searches.
+__global__ void __launch_bounds__(TP_T) trispec_tracer_panel_kernel(int nz, int nm, int nmp, int nseg, int nk, int ldk,
+                                                                    const double* __restrict__ ks,
+                                                                    const double* __restrict__ ms,
+                                                                    const double* __restrict__ nzm, double rho_m0,
+                                                                    const TracerLegs L, int n1, int ld1,
+                                                                    const double* __restrict__ q1, int n2, int ld2,
+                                                                    const double* __restrict__ q2,
+                                                                    const double* __restrict__ zs,
+                                                                    const double* __restrict__ chis,
+                                                                    const double* __restrict__ pref,
+                                                                    double* __restrict__ P1, double* __restrict__ P2) {
+  const int z = blockIdx.y, l = blockIdx.x * TP_T + threadIdx.x;
+  const int m0 = blockIdx.z * TP_MROWS, m1 = min(nmp, m0 + TP_MROWS);
+  HMV_DEV_ASSERT(z < nz && (nmp == nm || nmp == nm + 1) && nseg == (L.g1 >= 0 ? 2 : 1));
+  const bool c1 = l < n1, c2 = l < n2;
+  double zfac = 1.0, inv_chi = 0.0;
+  if (chis) {
+    zfac = pref[z] * (nz > 1 ? trapz_weight(zs, z, nz) : 1.0);
+    inv_chi = 1.0 / chis[z];
+  }
+  const double ig = L.ngal ? 1.0 / L.ngal[z] : 1.0;
+  int j1 = 0, j2 = 0;
+  double f1 = 0.0, f2 = 0.0;
+  if (c1) k_locate(ks, nk, chis ? (q1[l] + 0.5) * inv_chi : q1[l], j1, f1);
+  if (c2) k_locate(ks, nk, chis ? (q2[l] + 0.5) * inv_chi : q2[l], j2, f2);
+  for (int m = m0; m < m1; ++m) {
+    double v10 = 0.0, v11 = 0.0, v20 = 0.0, v21 = 0.0;   // panel values of segments 0 and 1
+    if (m < nm) {
+      const long long i = (long long)z * nm + m, row = i * ldk;
+      const double a = ms[m] / rho_m0;
+      if (c1) {
+        const double wn = trapz_weight(ms, m, nm) * nzm[i] * zfac;
+        if (L.g1 >= 0) {
+          double us, uc;
+          hod_profiles(L, L.g1, row, j1, f1, us, uc);
+          const double wx = wn * (ig * ig) * tracer_leg(L, 1 - L.g1, i, row, j1, f1, a, ig);
+          v10 = wx * us;
+          v11 = wx * L.NcNs[i] * uc;
+        } else {
+          v10 = wn * tracer_side(L, 0, L.pair1, i, row, j1, f1, a, ig);
+        }
+      }
+      if (c2) {
+        if (L.g2 >= 0) {
+          double us, uc;
+          hod_profiles(L, L.g2, row, j2, f2, us, uc);
+          const double ty = tracer_leg(L, 5 - L.g2, i, row, j2, f2, a, ig);
+          v20 = (L.NsNsm1[i] * us + L.NcNs[i] * uc) * ty;
+          v21 = us * ty;
+        } else {
+          v20 = tracer_side(L, 2, L.pair2, i, row, j2, f2, a, ig);
+        }
+      }
+    }
+    const long long K = (long long)z * nseg * nmp + m;
+    if (l < ld1) P1[K * ld1 + l] = v10;
+    if (l < ld2) P2[K * ld2 + l] = v20;
+    if (nseg == 2) {
+      if (l < ld1) P1[(K + nmp) * ld1 + l] = v11;
+      if (l < ld2) P2[(K + nmp) * ld2 + l] = v21;
+    }
+  }
+}
+
+// segments per redshift of a leg set: 2 for one galaxy leg on each side, else 1
+static int tracer_nseg(const hmv_tracer* legs_h) {
+  const bool g1 = legs_h[0].kind == 1 || legs_h[1].kind == 1, g2 = legs_h[2].kind == 1 || legs_h[3].kind == 1;
+  const int ng = (legs_h[0].kind == 1) + (legs_h[1].kind == 1) + (legs_h[2].kind == 1) + (legs_h[3].kind == 1);
+  return ng == 2 && g1 && g2 ? 2 : 1;
+}
+
+static long long tracer_ws_doubles(bool proj, int nz, int nm, int n1, int n2, const hmv_tracer* legs_h) {
+  if (!legs_h) return 0;
+  return trispec_ws_doubles(proj, nz, nm, n1, n2, tracer_nseg(legs_h));
+}
+
+// Checks of the tracer entry points, before any launch: fills L and nseg, ng = the number of galaxy legs.
+static int tracer_check(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                        const double* ms_d, const double* nzm_d, const hmv_tracer* legs_h, int n1, const double* q1_d,
+                        int n2, const double* q2_d, const double* zs_d, const double* chis_d, const double* pref_d,
+                        const double* ws_d, const double* out_d, TracerLegs& L, int& nseg, int& ng) {
+  return trispec_check_args(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, legs_h != nullptr, n1, q1_d, n2, q2_d, zs_d,
+                            chis_d, pref_d, ws_d, out_d, nseg, [&]() -> int {
+    const hmv_tracer* g = nullptr;
+    ng = 0;
+    L.Nc = L.Ns = L.NcNs = L.NsNsm1 = L.ngal = nullptr;
+    for (int i = 0; i < 4; ++i) {
+      const hmv_tracer& t = legs_h[i];
+      HMV_REQUIRE(t.us_d, "%s: null pointer (cube %d)", who, i);
+      HMV_REQUIRE(t.kind >= 0 && t.kind <= 2, "%s: leg %d: kind %d is not 0 (matter), 1 (HOD) or 2 (pressure)", who,
+                  i, t.kind);
+      HMV_REQUIRE(((size_t)t.us_d & 15) == 0 && ((size_t)t.uc_d & 15) == 0, "%s: cube %d must be 16-byte aligned",
+                  who, i);
+      HMV_REQUIRE(!t.bias_d, "%s: leg %d: bias_d has no meaning in the 1-halo trispectrum; pass NULL", who, i);
+      L.us[i] = t.us_d;
+      L.uc[i] = t.kind == 1 ? t.uc_d : nullptr;
+      L.kind[i] = t.kind;
+      if (t.kind != 1) continue;
+      HMV_REQUIRE(t.Nc_d && t.Ns_d && t.NcNs_d && t.NsNsm1_d && t.ngal_d, "%s: HOD leg %d lacks occupation arrays", who,
+                  i);
+      if (g) {
+        HMV_REQUIRE(t.us_d == g->us_d && t.uc_d == g->uc_d && t.Nc_d == g->Nc_d && t.Ns_d == g->Ns_d &&
+                        t.NcNs_d == g->NcNs_d && t.NsNsm1_d == g->NsNsm1_d && t.ngal_d == g->ngal_d,
+                    "%s: HOD legs %d and %d differ: the joint occupation of two HODs is not defined", who,
+                    (int)(g - legs_h), i);
+      } else {
+        g = &t;
+        L.Nc = t.Nc_d; L.Ns = t.Ns_d; L.NcNs = t.NcNs_d; L.NsNsm1 = t.NsNsm1_d; L.ngal = t.ngal_d;
+      }
+      ++ng;
+    }
+    HMV_REQUIRE(ng <= 2, "%s: %d HOD legs need occupation moments of order %d, which the HOD does not define", who, ng,
+                ng);
+    L.pair1 = L.kind[0] == 1 && L.kind[1] == 1;
+    L.pair2 = L.kind[2] == 1 && L.kind[3] == 1;
+    nseg = tracer_nseg(legs_h);
+    L.g1 = nseg == 2 ? (L.kind[0] == 1 ? 0 : 1) : -1;
+    L.g2 = nseg == 2 ? (L.kind[2] == 1 ? 2 : 3) : -1;
+    return HMV_OK;
+  });
+}
+
+// Profile legs only: trispec_run, so that the result is the profile entry point's to the bit.
+static int tracer_run(const char* who, bool proj, int nz, int nm, int nk, int ldk, const double* ks_d,
+                      const double* ms_d, const double* nzm_d, double rho_m0, const hmv_tracer* legs_h, int n1,
+                      const double* q1_d, int n2, const double* q2_d, const double* zs_d, const double* chis_d,
+                      const double* pref_d, double* ws_d, double* out_d, void* stream) {
+  TracerLegs L;
+  int nseg = 1, ng = 0;
+  const int chk = tracer_check(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, legs_h, n1, q1_d, n2, q2_d, zs_d, chis_d,
+                               pref_d, ws_d, out_d, L, nseg, ng);
+  if (chk) return chk;
+  if (ng == 0) {
+    const double* u_h[4] = {legs_h[0].us_d, legs_h[1].us_d, legs_h[2].us_d, legs_h[3].us_d};
+    const int kind_h[4] = {legs_h[0].kind, legs_h[1].kind, legs_h[2].kind, legs_h[3].kind};
+    return trispec_run(who, proj, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, u_h, kind_h, n1, q1_d, n2, q2_d, zs_d,
+                       chis_d, pref_d, ws_d, out_d, stream);
+  }
+  const TrispecPlan p = trispec_plan(proj, nz, nm, n1, n2, nseg);
+  const int nmp = nm + (nm & 1);
+  double* P1 = ws_d;
+  double* P2 = P1 + p.K * p.ld1;
+  double* part = P2 + p.K * p.ld2;
+  cudaStream_t st = (cudaStream_t)stream;
+  dim3 pg(cdiv(p.ld1 > p.ld2 ? p.ld1 : p.ld2, TP_T), nz, cdiv(nmp, TP_MROWS));
+  trispec_tracer_panel_kernel<<<pg, TP_T, 0, st>>>(nz, nm, nmp, nseg, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, L, n1,
+                                                   p.ld1, q1_d, n2, p.ld2, q2_d, zs_d, proj ? chis_d : nullptr, pref_d,
+                                                   P1, P2);
+  int rc = check_launch("trispec_tracer_panel_kernel");
+  if (rc) return rc;
+  return trispec_contract(who, p, n1, n2, P1, P2, part, out_d, st);
+}
+
+// ---- 2-halo trispectrum (DESIGN.md §4.6)-------------------------------------------------------------------------------
 //   T2h^{ABCD}(k1,k2;z) = P(k1) [I1~A(k1) I3^{BCD}(k1,k2,k2) + I1~B(k1) I3^{ACD}(k1,k2,k2)]
 //                       + P(k2) [I1~C(k2) I3^{ABD}(k1,k1,k2) + I1~D(k2) I3^{ABC}(k1,k1,k2)]
 //                       + Pbar(k1,k2) [I2^{AC}(k1,k2) I2^{BD}(k1,k2) + I2^{AD}(k1,k2) I2^{BC}(k1,k2)]
@@ -1161,6 +1384,31 @@ extern "C" int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d
                              const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream) {
   return trispec_run("hmv_cl_cov_1h", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, u_h, kind_h, nl1, ells1_d, nl2,
                      ells2_d, zs_d, chis_d, pref_d, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_trispec_1h_tracers_ws_doubles(int nz, int nm, int nk1, int nk2, const hmv_tracer* legs_h) {
+  return tracer_ws_doubles(false, nz, nm, nk1, nk2, legs_h);
+}
+
+extern "C" int hmv_trispec_1h_tracers(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                                      const double* nzm_d, double rho_m0, const hmv_tracer* legs_h, int nk1,
+                                      const double* k1_d, int nk2, const double* k2_d, double* ws_d, double* out_d,
+                                      void* stream) {
+  return tracer_run("hmv_trispec_1h_tracers", false, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, legs_h, nk1, k1_d,
+                    nk2, k2_d, nullptr, nullptr, nullptr, ws_d, out_d, stream);
+}
+
+extern "C" long long hmv_cl_cov_1h_tracers_ws_doubles(int nz, int nm, int nl1, int nl2, const hmv_tracer* legs_h) {
+  return tracer_ws_doubles(true, nz, nm, nl1, nl2, legs_h);
+}
+
+extern "C" int hmv_cl_cov_1h_tracers(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                                     const double* nzm_d, double rho_m0, const hmv_tracer* legs_h, int nl1,
+                                     const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                                     const double* chis_d, const double* pref_d, double* ws_d, double* out_d,
+                                     void* stream) {
+  return tracer_run("hmv_cl_cov_1h_tracers", true, nz, nm, nk, ldk, ks_d, ms_d, nzm_d, rho_m0, legs_h, nl1, ells1_d,
+                    nl2, ells2_d, zs_d, chis_d, pref_d, ws_d, out_d, stream);
 }
 
 extern "C" long long hmv_trispec_2h_ws_doubles(int nz, int nm, int nk, int nk1, int nk2, const double* const* u_h,

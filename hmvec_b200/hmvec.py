@@ -951,6 +951,44 @@ class HaloModel(Cosmology):
                                          capi.ptr(ws), capi.ptr(out), capi.stream()), fn)
         return self._host(out)
 
+    def _trispec1h_call(self, fn, names, q1, q2, extra, out_shape):
+        """The 1-halo term of four legs resolved as matter profile, then pressure profile, then HOD.  Profile legs only:
+        `fn` (_trispec_call).  One or two legs of one HOD: fn + '_tracers' with hmv_power's tracer records."""
+        kinds = []
+        for n in names:
+            if n in self.uk_profiles:
+                kinds.append(_KIND_MATTER)
+            elif n in self.pk_profiles:
+                kinds.append(_KIND_PRESSURE)
+            elif n in self.hods:
+                kinds.append(_KIND_HOD)
+            else:
+                raise ValueError("no matter or pressure profile or HOD named %r" % (n,))
+        hods = [n for n, k in zip(names, kinds) if k == _KIND_HOD]
+        if not hods:
+            return self._trispec_call(fn, names, q1, q2, extra, out_shape)
+        if len(hods) > 2:
+            raise ValueError("%d HOD legs: the 1-halo trispectrum needs occupation moments of order %d, which the HOD "
+                             "does not define" % (len(hods), len(hods)))
+        if len(set(hods)) > 1:
+            raise ValueError("HOD legs %r and %r: the 1-halo trispectrum of two HODs needs their joint occupation, "
+                             "which is not defined" % tuple(hods))
+        if not np.all(np.diff(self._ks64) > 0):
+            raise ValueError("the model's ks must be strictly increasing for the 1-halo trispectrum's interpolation")
+        legs = (capi.Tracer * 4)(*[self._tracer(n, k)[0] for n, k in zip(names, kinds)])
+        nz, nm = self._nz, self._nm
+        fn = fn + '_tracers'
+        ws = self._workspace('trispec', getattr(capi.lib, fn + '_ws_doubles')(nz, nm, q1.size, q2.size, legs))
+        out = self._empty(*out_shape)
+        q1_d, q2_d = self._dev(q1), self._dev(q2)
+        capi.check(getattr(capi.lib, fn)(nz, nm, self._nk, self._ldk, capi.ptr(self._ks_d), capi.ptr(self._ms_d),
+                                         capi.ptr(self._nzm_d), self._rho_m0, legs, q1.size, capi.ptr(q1_d), q2.size,
+                                         capi.ptr(q2_d), *[capi.ptr(e) for e in extra], capi.ptr(ws), capi.ptr(out),
+                                         capi.stream()), fn)
+        res = self._host(out)
+        self._check_hods()
+        return res
+
     def get_trispectrum_1halo(self, ks1, ks2=None, name="nfw", name2=None, name3=None, name4=None):
         """1-halo trispectrum T^{ABCD}(k1, k2; z) = sum_M w_M n(z,M) t_A(k1) t_B(k1) t_C(k2) t_D(k2), [nz, nk1, nk2].
 
@@ -958,15 +996,19 @@ class HaloModel(Cosmology):
         for a matter profile and u(k|M,z) for a pressure profile, the weights of get_power_1halo; w_M is the trapezoid
         weight on ms.  u is interpolated linearly in k on `ks`, and k outside [ks[0], ks[-1]] is clamped to the edge.
         No 1-halo damping factor (1 - exp(-(k/k*)^2)) is applied.  Names resolve as matter profile, then pressure
-        profile; HODs raise ValueError.  Defaults: name2 = name, name3 = name, name4 = name3, ks2 = ks1.  ks1 and ks2
-        need not be sorted."""
+        profile, then HOD.  A galaxy leg is t_g = (Nc u_c + Ns u_s)/ngal, get_power's (u_c = 1 without a central
+        profile).  Two galaxy legs in one halo take the pair moment without self-pairs, as get_power_1halo("g", "g"):
+        t_g(k) t_g(k') is replaced by [NsNsm1 u_s(k) u_s(k') + NcNs (u_c(k) u_s(k') + u_s(k) u_c(k'))] / ngal^2, on one
+        side (k = k') or across the two (k = k1, k' = k2).  Three or four galaxy legs, which need occupation moments
+        the HOD does not define, and galaxy legs of two different HODs raise ValueError.  Defaults: name2 = name,
+        name3 = name, name4 = name3, ks2 = ks1.  ks1 and ks2 need not be sorted."""
         name2 = name if name2 is None else name2
         name3 = name if name3 is None else name3
         name4 = name3 if name4 is None else name4
         k1 = self._positive(ks1, "ks1")
         k2 = k1 if ks2 is None else self._positive(ks2, "ks2")
-        return self._trispec_call('hmv_trispec_1h', (name, name2, name3, name4), k1, k2, (),
-                                  (self._nz, k1.size, k2.size))
+        return self._trispec1h_call('hmv_trispec_1h', (name, name2, name3, name4), k1, k2, (),
+                                    (self._nz, k1.size, k2.size))
 
     def get_cl_cov_1halo(self, ells, name="nfw", name2=None, name3=None, name4=None, windows=(1., 1., 1., 1.), fsky=1.,
                          ells2=None):
@@ -975,9 +1017,10 @@ class HaloModel(Cosmology):
             1/(4 pi fsky) sum_z zeta_z H^3 W_A W_B W_C W_D / chi^6 T^{ABCD}((l+1/2)/chi, (l'+1/2)/chi; z)
 
         with the window convention of limber_integral (C = int dz H W1 W2/chi^2 P), zeta_z the trapezoid weight on
-        self.zs (1 for a single redshift) and T as in get_trispectrum_1halo (no 1-halo damping).  Each window is a
-        scalar or an [nz] array on self.zs: lensing_window(zs, lzs) for kappa, 1 for Compton-y (1/H is inside the y
-        profile).  Defaults: name2 = name, name3 = name, name4 = name3, ells2 = ells; multipoles need not be sorted.
+        self.zs (1 for a single redshift) and T as in get_trispectrum_1halo (no 1-halo damping; galaxy legs of one
+        HOD, at most two).  Each window is a scalar or an [nz] array on self.zs: lensing_window(zs, lzs) for kappa, 1
+        for Compton-y (1/H is inside the y profile), the normalised dN/dz on self.zs for galaxies (as C_kg and C_gg
+        take it).  Defaults: name2 = name, name3 = name, name4 = name3, ells2 = ells; multipoles need not be sorted.
         Not available on a z-sharded model (the z sum would need a cross-rank reduction)."""
         if self._zcomm is not None:
             raise NotImplementedError("get_cl_cov_1halo on a z-sharded model: the z sum spans the ranks")
@@ -992,7 +1035,7 @@ class HaloModel(Cosmology):
         H = np.asarray(self.h_of_z(self.zs), dtype=np.float64).reshape(-1)
         pref = H ** 3 * W / chis ** 6 / (4.0 * np.pi * fsky)
         extra = (self._zs_d, self._dev(chis), self._dev(pref))
-        return self._trispec_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
+        return self._trispec1h_call('hmv_cl_cov_1h', (name, name2, name3, name4), l1, l2, extra, (l1.size, l2.size))
 
     # ------------------------------------------------------------------ 2-halo trispectrum and C_l covariance
     # Workspace budget of one 2-halo call, in doubles (8 GiB): the largest number of redshifts per pass that fits

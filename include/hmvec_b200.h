@@ -319,6 +319,27 @@ int hmv_cl_cov_1h(int nz, int nm, int nk, int ldk, const double* ks_d, const dou
                   const double* ells2_d, const double* zs_d, const double* chis_d, const double* pref_d, double* ws_d,
                   double* out_d, void* stream);
 
+/* The same with galaxy (HOD) legs (DESIGN.md §4.8).  legs_h: HOST array of four hmv_tracer (A, B at k1; C, D at k2)
+ * in place of u_h / kind_h; the other arguments as in hmv_trispec_1h / hmv_cl_cov_1h.  Kind 0 and 2 legs are the
+ * profile legs above (us_d the cube; uc_d and the occupation arrays are not read); a kind-1 leg is the HOD leg of
+ * hmv_power, t_g = (Nc UC + Ns US)/ngal with UC = 1 when uc_d is NULL.  Two galaxy legs take the pair moment without
+ * self-pairs, <g g>(k,k') = [NsNsm1 US(k) US(k') + NcNs (UC(k) US(k') + US(k) UC(k'))]/ngal^2, in place of t_g t_g:
+ * on one side (A, B or C, D) it is formed per column; one on each side runs the contraction over two segments of mass
+ * rows per redshift, K = nz * 2 * nm (even-padded) <= 2^30.  HMV_E_ARG before any launch for: a kind-1 leg with a
+ * NULL occupation array, three or four kind-1 legs (moments the HOD does not define), kind-1 legs that differ in any
+ * cube or occupation pointer (two HODs: no joint occupation), a non-NULL bias_d, and the checks of hmv_trispec_1h.
+ * Profile legs only give hmv_trispec_1h / hmv_cl_cov_1h's result to the bit.  The workspace functions take the legs
+ * (the segment count depends on them) and return 0 on invalid sizes or NULL legs_h. */
+long long hmv_trispec_1h_tracers_ws_doubles(int nz, int nm, int nk1, int nk2, const hmv_tracer* legs_h);
+int hmv_trispec_1h_tracers(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                           const double* nzm_d, double rho_m0, const hmv_tracer* legs_h, int nk1, const double* k1_d,
+                           int nk2, const double* k2_d, double* ws_d, double* out_d, void* stream);
+long long hmv_cl_cov_1h_tracers_ws_doubles(int nz, int nm, int nl1, int nl2, const hmv_tracer* legs_h);
+int hmv_cl_cov_1h_tracers(int nz, int nm, int nk, int ldk, const double* ks_d, const double* ms_d,
+                          const double* nzm_d, double rho_m0, const hmv_tracer* legs_h, int nl1,
+                          const double* ells1_d, int nl2, const double* ells2_d, const double* zs_d,
+                          const double* chis_d, const double* pref_d, double* ws_d, double* out_d, void* stream);
+
 /* ---- 2-halo trispectrum and its non-Gaussian Limber covariance of C_l (DESIGN.md §4.6) ----------------------------
  * No counterpart in the reference.  Cooray & Hu 2001, ApJ 554, 56; Cooray & Sheth 2002, Phys. Rep. 372, 1, §6.2.  Legs,
  * kinds, ks and the projection as in hmv_trispec_1h / hmv_cl_cov_1h; w^ = w_m n(z,m) b(z,m) (bh_d [nz][nm]).  For

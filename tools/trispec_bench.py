@@ -1,5 +1,5 @@
-"""Time the non-Gaussian C_l covariances on the LARGE grid: the 1-halo term (hmv_cl_cov_1h, also on a 25-redshift slab)
-and the 2-halo term (hmv_cl_cov_2h).
+"""Time the non-Gaussian C_l covariances on the LARGE grid: the 1-halo term (hmv_cl_cov_1h, also on a 25-redshift slab),
+its galaxy (HOD) legs (hmv_cl_cov_1h_tracers) and the 2-halo term (hmv_cl_cov_2h).
 
 Cases: C_kk x C_kk (NFW, lensing window of a source at z = 2.5) and C_yy x C_yy (Battaglia pressure) at
 ells = geomspace(10, 1e4, nl) on zs = linspace(0.01, 3, nz), ms = geomspace(2e10, 1e17, nm), ks = geomspace(1e-4, 100,
@@ -13,9 +13,12 @@ nk) (bench.py's grid), and C_kk on the slab zs[:25].  For each case it reports, 
 with the card's name and power limit read in the same run.  2-halo cases: C_kk and C_yy autos (3 contracted blocks)
 and the C_ky x C_ky cross (NFW, y, NFW, y: 8 blocks), zchunk as HaloModel.get_cl_cov_2halo picks it; flop = 2 nz nm
 n1 n2 per block; the split into prep, panel, contraction and assembly kernels; a seeded sample of entries against a
-float64 host evaluation (long-double Pbar prefix).  Prints one JSON document (and writes it to --out).
+float64 host evaluation (long-double Pbar prefix).  HOD cases: C_kg x C_kg (NFW and an HOD with ngal from 2e-3 to
+5e-5 over z, NFW satellites, no central profile: one galaxy leg on each side, two segments of mass rows per redshift)
+and C_kk x C_gg (both galaxy legs on one side: one segment), galaxy window a normalised Gaussian dN/dz; flop = 2 n1 n2
+nz nm per segment.  Prints one JSON document (and writes it to --out).
 
-    python tools/trispec_bench.py [--nz 200 --nm 2000 --nk 10000 --nl 1000 --reps 10 --out FILE]
+    python tools/trispec_bench.py [--nz 200 --nm 2000 --nk 10000 --nl 1000 --reps 10 --cases TAG,... --out FILE]
 """
 import argparse
 import ctypes as C
@@ -99,6 +102,72 @@ class Case(object):
             c = (zw * self.pref)[:, None] * wm[None, :] * nzm
             want = np.sum(c * ti ** 2 * tj ** 2)
             bound = np.sum(np.abs(c) * ti ** 2 * tj ** 2)
+            worst = max(worst, abs(got[i, j] - want) / bound if bound > 0 else abs(got[i, j] - want))
+        return worst
+
+
+class CaseHod(object):
+    """The ABI call of one 1-halo covariance with galaxy legs (hmv_cl_cov_1h_tracers), inputs resident on the device."""
+
+    def __init__(self, h, names, windows, ells):
+        from hmvec_b200 import _capi as capi
+        self.capi, self.h, self.names, self.ells = capi, h, names, ells
+        self.kinds = [0 if n in h.uk_profiles else 1 for n in names]
+        self.legs = (capi.Tracer * 4)(*[h._tracer(n, k)[0] for n, k in zip(names, self.kinds)])
+        zs = h.zs
+        self.chis = np.asarray(h.comoving_radial_distance(zs), dtype=np.float64)
+        H = np.asarray(h.h_of_z(zs), dtype=np.float64)
+        W = np.prod([np.broadcast_to(np.asarray(w, dtype=np.float64), zs.shape) for w in windows], axis=0)
+        self.pref = H ** 3 * W / self.chis ** 6 / (4 * np.pi)
+        self.d = {k: h._dev(v) for k, v in dict(ells=ells, chis=self.chis, pref=self.pref).items()}
+        n = ells.size
+        self.ws = h._empty(int(capi.lib.hmv_cl_cov_1h_tracers_ws_doubles(h._nz, h._nm, n, n, self.legs)))
+        self.out = h._empty(n, n)
+        self.nseg = 2 if 1 in self.kinds[:2] and 1 in self.kinds[2:] else 1
+
+    def launch(self):
+        h, p, d, n = self.h, self.capi.ptr, self.d, self.ells.size
+        self.capi.check(self.capi.lib.hmv_cl_cov_1h_tracers(h._nz, h._nm, h._nk, h._ldk, p(h._ks_d), p(h._ms_d),
+                                                            p(h._nzm_d), h._rho_m0, self.legs, n, p(d["ells"]), n,
+                                                            p(d["ells"]), p(h._zs_d), p(d["chis"]), p(d["pref"]),
+                                                            p(self.ws), p(self.out), self.capi.stream()),
+                        "hmv_cl_cov_1h_tracers")
+
+    def check_sample(self, rng, npairs=8):
+        """Max |got - want| / sum|terms| over seeded (l, l') entries: u_s of the NFW cube gathered on the device at the
+        columns the entries need, t and <g g> formed on the host in float64 (u_c = 1)."""
+        import torch
+        h = self.h
+        got = self.out.cpu().numpy()
+        ks, ms, nzm, zs = h._ks64, h.ms, h.nzm, h.zs
+        hod = h.hods[next(n for n, k in zip(self.names, self.kinds) if k == 1)]
+        Nc, Ns, NcNs, NsNsm1, ig = hod["Nc"], hod["Ns"], hod["NcNs"], hod["NsNsm1"], 1.0 / hod["ngal"][:, None]
+        wm = 0.5 * (ms[np.minimum(np.arange(ms.size) + 1, ms.size - 1)] - ms[np.maximum(np.arange(ms.size) - 1, 0)])
+        zw = 0.5 * (zs[np.minimum(np.arange(zs.size) + 1, zs.size - 1)] - zs[np.maximum(np.arange(zs.size) - 1, 0)])
+        cube = h.uk_profiles.device("nfw")
+        zi = torch.arange(zs.size, device=cube.device)
+
+        def us(ell):                       # u_s(z, m) at k = (l + 1/2)/chi_z, linear in k, clamped
+            k = np.clip((ell + 0.5) / self.chis, ks[0], ks[-1])
+            j = np.clip(np.searchsorted(ks, k, side="right") - 1, 0, ks.size - 2)
+            f = (k - ks[j]) / (ks[j + 1] - ks[j])
+            jd = torch.as_tensor(j, device=cube.device)
+            u0, u1 = cube[zi, :, jd].cpu().numpy(), cube[zi, :, jd + 1].cpu().numpy()
+            return u0 + f[:, None] * (u1 - u0)
+
+        c = (zw * self.pref)[:, None] * wm[None, :] * nzm
+        worst = 0.0
+        for _ in range(npairs):
+            i, j = rng.integers(0, self.ells.size, 2)
+            u1, u2 = us(self.ells[i]), us(self.ells[j])
+            tk1, tk2 = ms[None, :] / h._rho_m0 * u1, ms[None, :] / h._rho_m0 * u2
+            if self.nseg == 2:             # kappa g x kappa g: t_k(k1) t_k(k2) <g g>(k1, k2)
+                terms = [NsNsm1 * u1 * u2, NcNs * u2, NcNs * u1]
+                terms = [tk1 * tk2 * ig ** 2 * t for t in terms]
+            else:                          # kappa kappa x g g: t_k(k1)^2 <g g>(k2, k2)
+                terms = [tk1 ** 2 * ig ** 2 * t for t in (NsNsm1 * u2 ** 2, 2 * NcNs * u2)]
+            want = sum(np.sum(c * t) for t in terms)
+            bound = sum(np.sum(np.abs(c * t)) for t in terms)
             worst = max(worst, abs(got[i, j] - want) / bound if bound > 0 else abs(got[i, j] - want))
         return worst
 
@@ -222,6 +291,7 @@ def time_case(case, reps, dmma_tflops):
         torch.cuda.synchronize()
     per = {}
     names = (("trispec2h_prep_kernel", "prep"), ("trispec2h_panel_kernel", "panel"), ("trispec_panel_kernel", "panel"),
+             ("trispec_tracer_panel_kernel", "panel"),
              ("sigma2_gemm_kernel", "contraction"), ("trispec_reduce_kernel", "reduce"),
              ("trispec2h_assemble_kernel", "assemble"))
     for ev in prof.key_averages():
@@ -232,12 +302,12 @@ def time_case(case, reps, dmma_tflops):
                 t = ev.cuda_time_total
             per[key] = per.get(key, 0.0) + t / 1e3 / nprof
     h, n = case.h, case.ells.size
-    blocks = getattr(case, "blocks", 1)
-    flop = 2.0 * n * n * h._nz * h._nm * blocks
-    K, ld = h._nz * (h._nm + h._nm % 2), n + n % 2
+    blocks, nseg = getattr(case, "blocks", 1), getattr(case, "nseg", 1)
+    flop = 2.0 * n * n * h._nz * h._nm * blocks * nseg
+    K, ld = h._nz * nseg * (h._nm + h._nm % 2), n + n % 2
     res = {"nz": h._nz, "nm": h._nm, "nk": h._nk, "nl": n, "call_ms": total_ms, "reps": reps,
            "panel_ms": per.get("panel"), "contraction_ms": per.get("contraction"), "reduce_ms": per.get("reduce"),
-           "flop": flop, "blocks": blocks}
+           "flop": flop, "blocks": blocks, "segments": nseg}
     if blocks == 1:
         res["panel_bytes_written"] = 2.0 * K * ld * 8
     else:
@@ -260,8 +330,11 @@ def main():
     ap.add_argument("--nl", type=int, default=1000)
     ap.add_argument("--slab", type=int, default=25)
     ap.add_argument("--reps", type=int, default=10)
+    ap.add_argument("--cases", default=None, help="comma-separated result tags to run (default: all)")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
+    want = None if a.cases is None else set(a.cases.split(","))
+    run = lambda tag: want is None or tag in want
     import torch
     if not torch.cuda.is_available():
         sys.exit("trispec_bench needs a CUDA device")
@@ -279,17 +352,34 @@ def main():
     t = time.perf_counter()
     h = hm.HaloModel(zs, ks, ms=ms, accuracy='low')
     h.add_battaglia_pres_profile("y", family="pres", xmax=20, nxs=5000)
+    h.add_hod("g", ngal=np.geomspace(2e-3, 5e-5, a.nz))
     Wk = h.lensing_window(zs, 2.5)
+    dndz = np.exp(-0.5 * ((zs - 0.8) / 0.5) ** 2)
+    Wg = dndz / np.sum(0.5 * (np.r_[zs[1:], zs[-1]] - np.r_[zs[0], zs[:-1]]) * dndz)
     torch.cuda.synchronize()
     info["model_setup_s"] = time.perf_counter() - t
     for tag, name, kind, win in (("large_kk", "nfw", 0, (Wk,) * 4), ("large_yy", "y", 2, (1.,) * 4)):
+        if not run(tag):
+            continue
         c = Case(h, name, kind, win, ells)
         results[tag] = time_case(c, a.reps, dmma)
         results[tag]["sample_max_err_over_bound"] = c.check_sample(rng)
         del c
         torch.cuda.empty_cache()
+    for tag, names, win in (("large_kg_kg", ("nfw", "g", "nfw", "g"), (Wk, Wg, Wk, Wg)),
+                            ("large_kk_gg", ("nfw", "nfw", "g", "g"), (Wk, Wk, Wg, Wg))):
+        if not run(tag):
+            continue
+        c = CaseHod(h, names, win, ells)
+        results[tag] = time_case(c, a.reps, dmma)
+        results[tag]["names"] = list(names)
+        results[tag]["sample_max_err_over_bound"] = c.check_sample(rng)
+        del c
+        torch.cuda.empty_cache()
     for tag, names, win in (("large_kk_2h", ("nfw",) * 4, (Wk,) * 4), ("large_yy_2h", ("y",) * 4, (1.,) * 4),
                             ("large_ky_ky_2h", ("nfw", "y", "nfw", "y"), (Wk, 1., Wk, 1.))):
+        if not run(tag):
+            continue
         c = Case2h(h, names, win, ells)
         results[tag] = time_case(c, a.reps, dmma)
         results[tag]["sample_max_err_over_bound"] = c.check_sample(rng)
@@ -298,10 +388,11 @@ def main():
         torch.cuda.empty_cache()
     del h
     torch.cuda.empty_cache()
-    hs = hm.HaloModel(zs[:a.slab], ks, ms=ms, accuracy='low')
-    c = Case(hs, "nfw", 0, (hs.lensing_window(zs[:a.slab], 2.5),) * 4, ells)
-    results["slab_kk"] = time_case(c, a.reps, dmma)
-    results["slab_kk"]["sample_max_err_over_bound"] = c.check_sample(rng)
+    if run("slab_kk"):
+        hs = hm.HaloModel(zs[:a.slab], ks, ms=ms, accuracy='low')
+        c = Case(hs, "nfw", 0, (hs.lensing_window(zs[:a.slab], 2.5),) * 4, ells)
+        results["slab_kk"] = time_case(c, a.reps, dmma)
+        results["slab_kk"]["sample_max_err_over_bound"] = c.check_sample(rng)
     info["dmma_tflops_after"] = capi.lib.hmv_bench_dmma(20000, capi.stream())
     info["results"] = results
     txt = json.dumps(info, indent=1, sort_keys=True)
